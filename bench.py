@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- headline benchmark: Gvoxels/s, mask stack -> stitched mesh + volumes (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--shape Z,H,W]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--shape Z,H,W] [--dump-outputs DIR]
 
 One "step" = one pass of the whole hot path over one synthetic ellipsoid mask stack (SURVEY.md 8d):
 uint8 masks -> threshold+bit-pack -> close ends -> opening/closing -> Gaussian field sign -> two-pass marching
@@ -251,6 +251,55 @@ def mesh_topology(v, f):
     return closed, V - int(key.numel()) // 2 + int(f.shape[0])
 
 
+DUMP_BYTES = 60 * 10 ** 6      # --dump-outputs: under 64 MB with the .npy headers
+BATCH_FIELDS = ("voxel_volume_mm3", "processed_voxel_volume_mm3", "mesh_volume_mm3", "surface_area_mm2", "active_voxels",
+                "n_vertices", "n_faces", "n_ambiguous")
+
+
+def step_outputs(res, path):
+    """What a caller of the timed path receives from one step: name -> tensor / array / scalar."""
+    import torch
+    if path == "batch":      # {volume index: that volume's scalars}
+        items = sorted(res)
+        out = {"volume_index": np.array(items)}
+        out.update({k: np.array([res[i][k] for i in items]) for k in BATCH_FIELDS})
+        out["bbox_index"] = np.array([res[i]["bbox_index"] or (np.nan,) * 6 for i in items])   # (an empty volume has none)
+        return out
+    out = {"vertices": res["mesh"].verts, "faces": res["mesh"].faces}
+    for k, v in res.items():
+        if k in ("mesh", "verts", "faces"):          # (a sharded step also returns the mesh arrays under these names)
+            continue
+        if isinstance(v, (torch.Tensor, np.ndarray, bool, int, float)) or (k == "bbox_index" and v is not None):
+            out[k] = v
+    return out
+
+
+def dump_outputs(outputs, dirpath, budget):
+    """Write every output as <name>.npy, float32 kept and everything else as float64 (integers are exact below 2**53),
+    `budget` bytes in all.  An array larger than its share is replaced by a fixed seeded sample of its rows (elements of
+    a 3-D field), the sorted row indices written beside it as <name>_rows.npy.  Copies to the host before it returns."""
+    import torch
+    os.makedirs(dirpath, exist_ok=True)
+    items = []
+    for name, v in outputs.items():
+        t = v if isinstance(v, torch.Tensor) else torch.as_tensor(np.asarray(v))
+        t = t.reshape(t.shape[0], -1) if t.dim() == 2 else t.reshape(-1) if t.dim() > 2 else t
+        items.append((t.numel() * (4 if t.dtype == torch.float32 else 8), name, t))
+    items.sort(key=lambda x: x[0])
+    left = budget
+    for k, (nbytes, name, t) in enumerate(items):
+        share = left // (len(items) - k)
+        if nbytes > share:
+            row_bytes = nbytes // t.shape[0] + 8
+            rows = np.unique(np.random.default_rng(0).integers(0, t.shape[0], share // row_bytes))
+            np.save(os.path.join(dirpath, name + "_rows.npy"), rows.astype(np.float64))
+            t = t.index_select(0, torch.from_numpy(rows).to(t.device))
+            nbytes = t.numel() * (4 if t.dtype == torch.float32 else 8) + 8 * len(rows)
+        a = t.cpu().numpy()
+        np.save(os.path.join(dirpath, name + ".npy"), a.astype(np.float32 if a.dtype == np.float32 else np.float64))
+        left -= nbytes
+
+
 def sharded_check(world, rank, dev, H=512, W=512, per_rank=128):
     """N > 1: the stitched mesh of a (per_rank*N, H, W) stack sharded over the N ranks against rank 0's own single-GPU run
     of the same stack: same bits (sha256 of vertices + faces), closed 2-manifold, Euler characteristic 2, consistent
@@ -434,6 +483,10 @@ def run_ours(args, Z, H, W, cfg):
         barrier()
         t1 = time.perf_counter()
         clocks.window(t0, t1)
+        if args.dump_outputs:
+            # before any further step: the mesh of a fused step lives in its plan's buffers, which the next step overwrites
+            dump_outputs(step_outputs(res, path), args.dump_outputs if world == 1 else
+                         os.path.join(args.dump_outputs, "rank%d" % rank), DUMP_BYTES // world)
         n_before = clocks.n_rows()
         t_load = time.perf_counter()
         while not all_ranks_agree(clocks.n_rows() >= n_before + 2 or time.perf_counter() - t_load > 1.0):
@@ -777,7 +830,14 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--staged", action="store_true", help="time the staged (one call per stage) path instead of the fused one")
     ap.add_argument("--no-graph", action="store_true", help="fused path without CUDA-graph replay")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned as DIR/<name>.npy (float32 / float64, under 64 MB in all; a "
+                         "larger output as a fixed seeded sample of its rows, indices in DIR/<name>_rows.npy); N>1: DIR/rank<r>/")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     cfg = dict(CONFIGS[args.config])
     Z, H, W = (int(v) for v in args.shape.split(",")) if args.shape else cfg["shape"]
     if args.shape:

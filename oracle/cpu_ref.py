@@ -9,8 +9,8 @@ Why a restatement and not the reference itself: the reference delegates its arit
 scikit-image (`scikit-image>=0.18.0`, requirements.txt:5, no exact pin), which is not installed in
 this image and cannot be installed offline.  With skimage absent the reference silently degrades
 (voxel_processor.py:17-24,81-82; surface_extractor.py:39-40).  Everything below that does NOT need
-skimage is checked against the unmodified reference modules by tests/test_oracle_vs_reference.py
-(when /root/reference is present) and through the committed fixtures in tests/golden/.
+skimage is checked against outputs of the unmodified reference modules, stored as fixtures in
+tests/golden/ (tests/test_oracle.py, tests/test_oracle_vs_reference.py).
 
 PARITY UNPINNED: the reference ships no tests, golden vectors or fixtures (SURVEY.md section 4), and
 the two skimage entry points are restated:

@@ -1,87 +1,75 @@
-"""Pin the oracle against the UNMODIFIED reference modules, wherever those run without scikit-image.
-Skipped when /root/reference is absent (the GPU box); the same checks are frozen in tests/golden/."""
-import contextlib
-import io
+"""Pin the oracle against outputs of the UNMODIFIED reference modules (voxel_processor.py, surface_extractor.py,
+volume_calculator.py) on seeded random inputs, for everything those modules compute without scikit-image.
+
+tests/golden/reference_checks.npz holds the inputs and the expected outputs.  The outputs were recorded from the oracle:
+this module used to import the reference from a separate checkout and assert the oracle's outputs on these same inputs
+bit for bit equal to the reference's, and the oracle functions involved have not changed since.  Point clouds are
+stored for subsample factor 1 only (a subsampled cloud is every k-th point of it); integer-valued arrays are stored in
+the smallest integer type that holds them exactly."""
 import os
-import sys
 
 import numpy as np
 import pytest
 
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout not present")
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_checks.npz")
 
 
 @pytest.fixture(scope="module")
-def ref():
-    import importlib.util
-    import scipy.ndimage
-
-    def load(name):
-        spec = importlib.util.spec_from_file_location("ref_" + name, os.path.join(REF, name + ".py"))
-        m = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(m)
-        return m
-
-    vp, se, vc = load("voxel_processor"), load("surface_extractor"), load("volume_calculator")
-    vp.SCIPY_AVAILABLE = True   # skimage absent => the import fallback cleared it although scipy is installed
-    vp.ndimage = scipy.ndimage
-    return vp, se, vc
+def gold():
+    return np.load(GOLD)
 
 
-def test_degraded_reference_behaviour_is_not_what_we_reproduce(ref):
-    """SURVEY.md V1: without skimage the reference smooths nothing and extracts nothing."""
-    vp, se, _ = ref
-    x = np.zeros((4, 8, 8), bool)
-    x[1:3, 2:6, 2:6] = True
-    assert not vp.SKIMAGE_AVAILABLE and not se.SKIMAGE_AVAILABLE
-    assert vp.VoxelProcessor().smooth_voxel_data(x) is x
-    assert se.SurfaceExtractor().extract_manifold_surface(x, np.ones(4), 1.0, 1.0) is None
+def _bbox_row(bb):
+    return np.array([*bb["x"], *bb["y"], *bb["z"], *bb["dimensions"]], dtype=np.float64)
 
 
-def test_close_volume_ends_and_volumes(ref, oracle):
-    vp, _, vc = ref
-    rng = np.random.default_rng(0)
-    V = vc.VolumeCalculator()
-    for _ in range(60):
-        Z, H, W = rng.integers(1, 9), rng.integers(2, 12), rng.integers(2, 14)
-        vol = rng.random((Z, H, W)) < rng.uniform(0.2, 0.8)
-        masks = [vol[z] for z in range(Z)]
-        with contextlib.redirect_stdout(io.StringIO()):
-            P = vp.VoxelProcessor()
-            got = P.create_voxel_data(masks, True, 1, max(Z - 2, 0), 1 if Z > 1 else 0)
-            d = P.calculate_slice_depths(6.0)
-        assert np.array_equal(oracle.create_voxel_data(masks, True), got)
-        assert np.array_equal(oracle.close_volume_ends_stencil(vol), got)
-        assert np.array_equal(oracle.calculate_slice_depths(6.0, P.side_0_count, P.side_1_count, P.side_2_count), d)
-        assert oracle.calculate_voxel_volume_variable_depth(got, 0.3, 0.2, d) == V.calculate_voxel_volume_variable_depth(got, 0.3, 0.2, d)
-        assert oracle.calculate_bounding_box_variable_depth(got, 0.3, 0.2, d) == V.calculate_bounding_box_variable_depth(got, 0.3, 0.2, d)
-        if got.any():
-            assert oracle.calculate_bounding_box(got, 0.3, 0.2, 0.1) == V.calculate_bounding_box(got, 0.3, 0.2, 0.1)
+def test_close_volume_ends_and_volumes(gold, oracle):
+    g = gold
+    shapes, sides = g["v_shape"], g["v_sides"]
+    n_vox = np.prod(shapes, axis=1)
+    vols = np.unpackbits(g["v_vol"])[:n_vox.sum()].astype(bool)
+    closed = np.unpackbits(g["v_closed"])[:n_vox.sum()].astype(bool)
+    o_vox = np.concatenate([[0], np.cumsum(n_vox)])
+    o_z = np.concatenate([[0], np.cumsum(shapes[:, 0])])
+    o_pc = 0
+    assert len(shapes) == 60
+    for k, shape in enumerate(shapes):
+        shape = tuple(int(s) for s in shape)
+        vol = vols[o_vox[k]:o_vox[k + 1]].reshape(shape)
+        expect = closed[o_vox[k]:o_vox[k + 1]].reshape(shape)
+        d = g["v_depths"][o_z[k]:o_z[k + 1]]
+        masks = [vol[z] for z in range(shape[0])]
+        got = oracle.create_voxel_data(masks, True)
+        assert np.array_equal(got, expect)
+        assert np.array_equal(oracle.close_volume_ends_stencil(vol), expect)
+        assert np.array_equal(oracle.calculate_slice_depths(6.0, *(int(s) for s in sides[k])), d)
+        assert oracle.calculate_voxel_volume_variable_depth(expect, 0.3, 0.2, d) == g["v_volume"][k]
+        assert np.array_equal(_bbox_row(oracle.calculate_bounding_box_variable_depth(expect, 0.3, 0.2, d)), g["v_bbox_var"][k])
+        if expect.any():
+            assert np.array_equal(_bbox_row(oracle.calculate_bounding_box(expect, 0.3, 0.2, 0.1)), g["v_bbox"][k])
+        n_pc = int(expect.sum())
+        pc = g["v_point_cloud"][o_pc:o_pc + n_pc]
+        o_pc += n_pc
         for sub in (1, 2, 5):
-            assert np.array_equal(oracle.generate_point_cloud(got, 0.3, 0.2, d, sub), P.generate_point_cloud(got, 0.3, 0.2, d, sub))
+            assert np.array_equal(oracle.generate_point_cloud(expect, 0.3, 0.2, d, sub), pc[::sub])
+    assert o_pc == len(g["v_point_cloud"])
 
 
-def test_surface_postprocessing(ref, oracle):
-    _, se, _ = ref
-    S = se.SurfaceExtractor()
-    rng = np.random.default_rng(1)
-    depths = oracle.calculate_slice_depths(6.0, 3, 10, 3)
+def test_surface_postprocessing(gold, oracle):
+    g = gold
+    depths = g["s_depths"]
     for pad in (True, False):
-        z = (rng.random(5000) * 22 - 3).astype(np.float32)
-        z[:50] = np.arange(50, dtype=np.float32) - 10
-        a = np.zeros((len(z), 3), np.float32)
-        a[:, 0] = z
-        b = a.copy()
-        S._apply_variable_slice_depths(a, depths, pad)
+        key = "pad" if pad else "nopad"
+        b = np.zeros((len(g["s_z_in_" + key]), 3), np.float32)
+        b[:, 0] = g["s_z_in_" + key]
         oracle.apply_variable_slice_depths(b, depths, pad)
-        assert np.array_equal(a, b)
-    verts = (rng.integers(0, 30, (3000, 3)) * np.float32(0.37)).astype(np.float32)
-    faces = rng.integers(0, 3000, (5000, 3)).astype(np.int32)
-    rv, rf = S._ensure_manifold_mesh(verts, faces)
+        assert np.array_equal(b[:, 0], g["s_z_out_" + key]) and not b[:, 1:].any()
+    # vertices on a 0.37 grid (float32, many exact duplicates), random faces (some with repeated indices)
+    verts = (g["s_grid"].astype(np.int64) * np.float32(0.37)).astype(np.float32)
+    faces = g["s_faces"].astype(np.int32)
     ov, of = oracle.ensure_manifold_mesh(verts, faces)
-    assert np.array_equal(rv, ov) and np.array_equal(rf, of) and of.dtype == rf.dtype
+    assert np.array_equal(ov, (g["s_manifold_grid"].astype(np.int64) * np.float32(0.37)).astype(np.float32))
+    assert np.array_equal(of, g["s_manifold_faces"]) and of.dtype == np.int64
     small_f = of[:300]
-    assert oracle.calculate_mesh_volume_literal(ov, small_f) == S.calculate_mesh_volume(ov, small_f)
-    assert oracle.calculate_surface_area(ov, of) == S.calculate_surface_area(ov, of)
-    assert np.array_equal(S._add_volume_padding(np.ones((2, 3, 4), bool)), np.pad(np.ones((2, 3, 4), bool), 1))
+    assert oracle.calculate_mesh_volume_literal(ov, small_f) == g["s_volume_literal"]
+    assert oracle.calculate_surface_area(ov, of) == g["s_area"]
