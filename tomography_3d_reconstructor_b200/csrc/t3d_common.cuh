@@ -175,6 +175,3 @@ int t3d_pack_gap_launch(const void* masks_u8, int Z, int H, int W, int threshold
 int t3d_bbox_t_planes_launch(const uint32_t* bits, int n_planes, int H, int W, int z_bias, unsigned int* bbox_t, cudaStream_t st);
 int t3d_close_ends_fixup_launch(const void* masks_u8, int Z, int H, int W, int threshold, const void* filled0, const void* filledT,
                                 void* out, unsigned long long* counts, cudaStream_t st);
-
-// rows each thread of the y-marching stencil kernels walks (tunable through the environment for experiments)
-int t3d_rows_per_thread(const char* env_name, int dflt);

@@ -688,8 +688,6 @@ static int64_t sdf_stack_bytes(int n, int64_t n_lines) { return a256((int64_t)n 
 
 static int sdf_bulk_ok(const void* a, const void* b, int64_t n_lines, int64_t inner, int64_t outer_stride, int64_t stride)
 {
-    static const bool off = getenv("T3D_SDF_NO_BULK") != nullptr;
-    if (off) return 0;
     // every 128-line tile must be one contiguous row segment whose start and length are multiples of 16 bytes
     if (((uintptr_t)a & 15) || ((uintptr_t)b & 15) || (stride & 7) || (outer_stride & 7)) return 0;
     if (inner % SDF_THREADS) {                       // tiles may only straddle an `inner` boundary when lines are contiguous anyway

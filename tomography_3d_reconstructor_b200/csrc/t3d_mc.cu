@@ -720,9 +720,8 @@ extern "C" int t3d_mc_flags(const void* sign_bits, int Zs, int Hs, int Ws, int z
     if (t3d_zero_async(ballots_u32, sizeof(uint32_t) * (size_t)g.n_rows * g.ncr, st)) return 1;
     const int nws4 = g.nws / 4, lanes_x = nws4 < 256 ? nws4 : 256, pzb = 256 / lanes_x;
     const int nz = (g.z_end < Zs ? g.z_end + 1 : Zs) - g.z_begin;
-    static const int gy = t3d_rows_per_thread("T3D_FLAGS_ROWS", GY);
-    dim3 grid((nws4 + lanes_x - 1) / lanes_x, (Hs + gy - 1) / gy, (nz + pzb - 1) / pzb);
-    k_mc_flags<<<grid, 256, 0, st>>>(g, (uint32_t*)ballots_u32, lanes_x, pzb, gy);
+    dim3 grid((nws4 + lanes_x - 1) / lanes_x, (Hs + GY - 1) / GY, (nz + pzb - 1) / pzb);
+    k_mc_flags<<<grid, 256, 0, st>>>(g, (uint32_t*)ballots_u32, lanes_x, pzb, GY);
     T3D_CHECK_LAUNCH("t3d_mc_flags");
     t3d_count_launches(1);
     return 0;

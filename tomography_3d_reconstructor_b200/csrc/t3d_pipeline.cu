@@ -47,8 +47,7 @@ static inline int64_t al(int64_t x) { return (x + 255) & ~(int64_t)255; }
 // word 4 -- no separate field-sign pass, no separately stored smoothed volume.
 static bool fast_surface(int n_stages, unsigned erode_mask, int pad, int Zx, int H, int W)
 {
-    static const bool off = getenv("T3D_NO_FAST_SIGN") != nullptr;
-    return !off && pad == 1 && n_stages == 4 && (erode_mask & 15u) == 9u && Zx >= 2 && H >= 2 && W >= 2;
+    return pad == 1 && n_stages == 4 && (erode_mask & 15u) == 9u && Zx >= 2 && H >= 2 && W >= 2;
 }
 
 struct Layout {
@@ -547,8 +546,7 @@ __global__ void k_merge_pre_stats(unsigned long long* __restrict__ r, const unsi
 
 extern "C" int t3d_slab_pack_gap_ok(const void* masks_u8, int n_own, int H, int W, int threshold)
 {
-    static const bool off = getenv("T3D_NO_SLAB_PACK_GAP") != nullptr;
-    if (off || n_own < 2 * SLAB_RAW || H <= 0 || W <= 0) return 0;
+    if (n_own < 2 * SLAB_RAW || H <= 0 || W <= 0) return 0;
     const uint8_t* sub = (const uint8_t*)masks_u8 + (int64_t)(SLAB_EDGE - 2) * H * W;
     return t3d_pack_gap_supported(sub, n_own - 2 * SLAB_EDGE + 4, H, W, threshold) ? 1 : 0;
 }

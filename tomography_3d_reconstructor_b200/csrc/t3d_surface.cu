@@ -303,9 +303,8 @@ extern "C" int t3d_field_sign(const void* occ_bits, int Z, int H, int W, int pad
     const int nwp = t3d_wpr(v.Wp);
     T3D_CUDA(cudaMemsetAsync(n_exact_u64, 0, 8, st));
     const int nwp4 = nwp / 4, lanes_x = nwp4 < 256 ? nwp4 : 256, pzb = 256 / lanes_x;
-    static const int fy = t3d_rows_per_thread("T3D_SIGN_ROWS", FY);
-    dim3 grid((nwp4 + lanes_x - 1) / lanes_x, (v.Hp + fy - 1) / fy, (v.Zp + pzb - 1) / pzb);
-    k_field_sign<false><<<grid, 256, 0, st>>>(v, (uint32_t*)sign_bits, nwp, lanes_x, pzb, fy, (unsigned long long*)n_exact_u64, nullptr, 0,
+    dim3 grid((nwp4 + lanes_x - 1) / lanes_x, (v.Hp + FY - 1) / FY, (v.Zp + pzb - 1) / pzb);
+    k_field_sign<false><<<grid, 256, 0, st>>>(v, (uint32_t*)sign_bits, nwp, lanes_x, pzb, FY, (unsigned long long*)n_exact_u64, nullptr, 0,
                                               nullptr);
     T3D_CHECK_LAUNCH("t3d_field_sign");
     t3d_count_launches(1);
@@ -324,9 +323,8 @@ extern "C" int t3d_field_sign_lean(const void* occ_bits, int Z, int H, int W, in
     const int nwp = t3d_wpr(v.Wp);
     if (t3d_zero_async(n_exact_u64, 8, st) || t3d_zero_async(exc_count_u64, 8, st)) return 1;
     const int nwp4 = nwp / 4, lanes_x = nwp4 < 256 ? nwp4 : 256, pzb = 256 / lanes_x;
-    static const int fy = t3d_rows_per_thread("T3D_SIGN_ROWS", FY);
-    dim3 grid((nwp4 + lanes_x - 1) / lanes_x, (v.Hp + fy - 1) / fy, (v.Zp + pzb - 1) / pzb);
-    k_field_sign<true><<<grid, 256, 0, st>>>(v, (uint32_t*)sign_bits, nwp, lanes_x, pzb, fy, (unsigned long long*)n_exact_u64,
+    dim3 grid((nwp4 + lanes_x - 1) / lanes_x, (v.Hp + FY - 1) / FY, (v.Zp + pzb - 1) / pzb);
+    k_field_sign<true><<<grid, 256, 0, st>>>(v, (uint32_t*)sign_bits, nwp, lanes_x, pzb, FY, (unsigned long long*)n_exact_u64,
                                              (unsigned long long*)exc_list_u64, exc_cap, (unsigned long long*)exc_count_u64);
     k_field_sign_fix<<<T3D_NUM_SMS, 128, 0, st>>>(v, (uint32_t*)sign_bits, nwp, (const unsigned long long*)exc_list_u64, exc_cap,
                                                   (const unsigned long long*)exc_count_u64);
@@ -817,14 +815,10 @@ static int canonical_tail(const float* vin, const uint32_t* perm, int64_t V, con
         const int64_t nb = (V + UQ_TILE - 1) / UQ_TILE;
         const size_t desc_bytes = (size_t)nb * 8;
         if (t3d_zero_async(scan_ws, desc_bytes + 64, st)) return 1;
-        static const bool optimistic = getenv("T3D_NO_OPTIMISTIC_UNIQUE") == nullptr;
-        unsigned long long* dup = nullptr;
-        if (optimistic) {
-            dup = totals + 8;
-            if (t3d_zero_async(dup, 8, st)) return 1;
-            k_unique_optimistic<<<(unsigned)((V + 255) / 256), 256, 0, st>>>(vin, perm, V, V_dev, (float*)verts_out, newid, counts + 2, counts, dup);
-            t3d_count_launches(1);
-        }
+        unsigned long long* dup = totals + 8;
+        if (t3d_zero_async(dup, 8, st)) return 1;
+        k_unique_optimistic<<<(unsigned)((V + 255) / 256), 256, 0, st>>>(vin, perm, V, V_dev, (float*)verts_out, newid, counts + 2, counts, dup);
+        t3d_count_launches(1);
         k_unique_fused<<<(unsigned)nb, SC_THREADS, 0, st>>>(vin, perm, V, V_dev, (float*)verts_out, newid, (unsigned long long*)scan_ws,
                                                            (int)nb, (unsigned int*)((char*)scan_ws + desc_bytes), counts + 2, counts, dup);
     }
@@ -911,7 +905,7 @@ extern "C" int t3d_mesh_canonicalize_fast_dev(const void* verts_in, int64_t V_ca
 // coordinate transform is monotone, which fixes almost everything without sorting:
 //   * x-edge vertices are already in canonical order among themselves;
 //   * y-edge vertices only need ordering inside their (plane, row gap) segment (a handful of vertices): ranked by counting;
-//   * z-edge vertices need ONE stable radix sort by (layer, z float) -- a third of the vertices, 42-bit keys;
+//   * z-edge vertices need ONE stable sort by (layer, z float) -- a third of the vertices, one segment per layer (below);
 //   * the final position of a vertex = its rank in its own block + how many vertices of the other two blocks precede it;
 //     those counts are per-row / per-plane prefix counts, read from the scanned per-active-word counts of the emit pass.
 // Exception G0: with the z map's clamp (surface_extractor.py:100-103) every vertex at or below un-padded plane 0 gets
@@ -984,34 +978,6 @@ __device__ __forceinline__ float plane_z(const CanonS& c, int k)
     return fz;
 }
 
-__global__ void __launch_bounds__(256) k_canon_zkeys(CanonS c)
-{
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= c.cap_z) return;
-    const uint32_t nx = (uint32_t)c.sizes[1], ny = (uint32_t)c.sizes[2], nz = (uint32_t)c.sizes[3];
-    unsigned long long key = 0xffffffffffffffffull;
-    if ((unsigned long long)nx + ny + nz <= c.cap_verts && i < nz) {
-        uint32_t gX, gY, gZ;
-        g0_sizes(c, gX, gY, gZ);
-        const uint32_t raw = nx + ny + i;
-        if (i < gZ) key = 0ull;
-        else {
-            const int k = (int)(c.vkeys[raw] >> 42);
-            uint32_t zk = float_key(c.verts[3 * (int64_t)raw]);
-            if (c.zkey_bits < 32) {
-                // relative to the layer's lower plane; anything outside the promised span saturates (and fails the check)
-                const uint32_t base = float_key(plane_z(c, k));
-                zk = zk >= base ? zk - base : 0u;
-                const uint32_t lim = (1u << c.zkey_bits) - 1u;
-                zk = zk > lim ? lim : zk;
-            }
-            key = ((unsigned long long)(k + 1) << c.zkey_bits) | zk;
-        }
-    }
-    c.zkeys[i] = key;
-    c.zval[i] = i;
-}
-
 // ------------------------------------------------------------------------------------------------
 // Ordering of the z-edge vertices without a library sort.  They are emitted in raster order of their owning grid point,
 // so the vertices of one cube layer are contiguous: the (layer, z float) order is a SEGMENTED sort, one independent
@@ -1030,7 +996,7 @@ __global__ void __launch_bounds__(256) k_canon_zkeys(CanonS c)
 
 __device__ __forceinline__ uint32_t canon_zkey(const CanonS& c, uint32_t i, uint32_t nx, uint32_t ny, uint32_t gZ)
 {
-    if (i < gZ) return 0u;     // clamp group: ordered elsewhere (k_canon_gkeys); keep raster order here
+    if (i < gZ) return 0u;     // clamp group: ordered elsewhere (k_gsort); keep raster order here
     const uint32_t raw = nx + ny + i;
     const int k = (int)(c.vkeys[raw] >> 42);
     uint32_t zk = float_key(c.verts[3 * (int64_t)raw]);
@@ -1185,26 +1151,6 @@ __global__ void __launch_bounds__(ZS_THREADS) k_gsort(CanonS c, unsigned long lo
     }, raw_of, keyA, keyB, idxA, idxB, gperm);
 }
 
-__global__ void __launch_bounds__(256) k_canon_gkeys(CanonS c)
-{
-    const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= c.cap_g0) return;
-    const uint32_t nx = (uint32_t)c.sizes[1], ny = (uint32_t)c.sizes[2], nz = (uint32_t)c.sizes[3];
-    unsigned long long key = 0xffffffffffffffffull;
-    uint32_t raw = 0;
-    if ((unsigned long long)nx + ny + nz <= c.cap_verts) {
-        uint32_t gX, gY, gZ;
-        g0_sizes(c, gX, gY, gZ);
-        if (t < gX + gY + gZ) {
-            raw = t < gX ? t : t < gX + gY ? nx + (t - gX) : nx + ny + (t - gX - gY);
-            const float* v = c.verts + 3 * (int64_t)raw;
-            key = ((unsigned long long)float_key(v[1]) << 32) | float_key(v[2]);
-        }
-    }
-    c.gkeys[t] = key;
-    c.gval[t] = raw;
-}
-
 __global__ void __launch_bounds__(256) k_canon_positions(CanonS c)
 {
     __shared__ uint32_t s_g[3];
@@ -1249,10 +1195,6 @@ __global__ void __launch_bounds__(256) k_canon_positions(CanonS c)
     }
 }
 
-static int bits_for(unsigned v) { int b = 0; while ((1u << b) <= v) ++b; return b; }   // bits needed to hold values 0..v
-
-static size_t sort64_temp_bytes(int64_t V);
-
 extern "C" int64_t t3d_canonicalize_structured_workspace_bytes(int64_t V, int64_t F, uint32_t cap_z, uint32_t cap_g0, int Zs)
 {
     const int64_t n = V > F ? V : F;
@@ -1262,10 +1204,7 @@ extern "C" int64_t t3d_canonicalize_structured_workspace_bytes(int64_t V, int64_
     b += align256(4 * V);                                                          // perm
     b += 2 * align256(4 * n);                                                      // flags, positions
     b += align256(4 * V);                                                          // newid
-    const int64_t tz = (int64_t)sort64_temp_bytes(cap_z > 0 ? cap_z : 1);
-    int64_t tg = (int64_t)sort64_temp_bytes(cap_g0 > 0 ? cap_g0 : 1);
-    if (tg < 4 * (int64_t)cap_g0 + 256) tg = 4 * (int64_t)cap_g0 + 256;     // k_gsort's second value buffer
-    b += align256(tz > tg ? tz : tg);
+    b += align256(4 * (int64_t)cap_g0 + 256);                                      // k_gsort's second value buffer
     b += 2 * align256(t3d_scan_workspace_bytes(n, 1)) + 256;   // zero tail: unique descriptors, face-scan workspace, totals
     return b;
 }
@@ -1327,10 +1266,7 @@ extern "C" int t3d_mesh_canonicalize_structured_dev(const void* verts_in, const 
     uint32_t* flags = (uint32_t*)ws; ws += align256(4 * n);
     uint32_t* pos = (uint32_t*)ws; ws += align256(4 * n);
     uint32_t* newid = (uint32_t*)ws; ws += align256(4 * V);
-    const size_t tz = sort64_temp_bytes(cap_z);
-    size_t tg = sort64_temp_bytes(cap_g0 > 0 ? cap_g0 : 1);
-    if (tg < 4 * (size_t)cap_g0 + 256) tg = 4 * (size_t)cap_g0 + 256;       // k_gsort's second value buffer
-    void* temp = ws; ws += align256((int64_t)(tz > tg ? tz : tg));
+    void* temp = ws; ws += align256(4 * (int64_t)cap_g0 + 256);             // k_gsort's second value buffer
     void* scan_ws = ws; ws += align256(t3d_scan_workspace_bytes(n, 1));
     void* scan_ws_f = ws; ws += align256(t3d_scan_workspace_bytes(n, 1));
     unsigned long long* totals = (unsigned long long*)ws;
@@ -1338,40 +1274,20 @@ extern "C" int t3d_mesh_canonicalize_structured_dev(const void* verts_in, const 
     c.zperm = zperm; c.gperm = gperm;
     c.n_g0_out = (unsigned long long*)n_g0_u64;
     if (phases & 1) {
-        static const bool lib_sort = getenv("T3D_ZSORT_LIBRARY") != nullptr;     // A/B switch: the previous library radix sort
-        if (lib_sort) {
-            k_canon_zkeys<<<(cap_z + 255) / 256, 256, 0, st>>>(c);
-            size_t tb = tz;
-            T3D_CUDA(cub::DeviceRadixSort::SortPairs(temp, tb, (const unsigned long long*)c.zkeys, zkeys_b, (const uint32_t*)c.zval, zperm,
-                                                     (int)cap_z, 0, zkey_bits + bits_for((unsigned)Zs + 1), st));
-            t3d_count_launches(2);
-        } else {
-            // one CTA per cube layer: segmented stable radix sort of the layer's z-edge vertices (no library)
-            uint32_t* keyA = (uint32_t*)c.zkeys;
-            uint32_t* keyB = keyA + cap_z;
-            uint32_t* idxA = (uint32_t*)zkeys_b;
-            uint32_t* idxB = idxA + cap_z;
-            static const int force_u = getenv("T3D_ZSORT_U") ? atoi(getenv("T3D_ZSORT_U")) : 0;      // A/B switch: 1 or 8
-            const bool batched = force_u ? force_u == 8 : (int64_t)cap_z >= 4096 * (int64_t)Zs;
-            if (batched) k_zsort_layers<8><<<Zs, ZS_THREADS, 0, st>>>(c, keyA, keyB, idxA, idxB, zperm);
-            else k_zsort_layers<1><<<Zs, ZS_THREADS, 0, st>>>(c, keyA, keyB, idxA, idxB, zperm);
-            t3d_count_launches(1);
-        }
+        // one CTA per cube layer: segmented stable radix sort of the layer's z-edge vertices (no library)
+        uint32_t* keyA = (uint32_t*)c.zkeys;
+        uint32_t* keyB = keyA + cap_z;
+        uint32_t* idxA = (uint32_t*)zkeys_b;
+        uint32_t* idxB = idxA + cap_z;
+        if ((int64_t)cap_z >= 4096 * (int64_t)Zs) k_zsort_layers<8><<<Zs, ZS_THREADS, 0, st>>>(c, keyA, keyB, idxA, idxB, zperm);
+        else k_zsort_layers<1><<<Zs, ZS_THREADS, 0, st>>>(c, keyA, keyB, idxA, idxB, zperm);
+        t3d_count_launches(1);
     }
     if (phases & 2) {
         if (t3d_zero_async(counts + 2, 8, st)) return 1;
         if (cap_g0 > 0) {
-            static const bool lib_sort = getenv("T3D_ZSORT_LIBRARY") != nullptr;
-            if (lib_sort) {
-                // (shares the radix sort's temporary storage with the z sort: phase 2 must be ordered after phase 1)
-                k_canon_gkeys<<<(cap_g0 + 255) / 256, 256, 0, st>>>(c);
-                size_t tb = tg;
-                T3D_CUDA(cub::DeviceRadixSort::SortPairs(temp, tb, (const unsigned long long*)c.gkeys, gkeys_b, (const uint32_t*)c.gval, gperm,
-                                                         (int)cap_g0, 0, 64, st));
-            } else {
-                // one CTA: stable radix sort of the clamp group by (y, x); gval / `temp` serve as the second value / key buffers
-                k_gsort<<<1, ZS_THREADS, 0, st>>>(c, c.gkeys, gkeys_b, c.gval, (uint32_t*)temp, gperm);
-            }
+            // one CTA: stable radix sort of the clamp group by (y, x); gval / `temp` serve as the second value / key buffers
+            k_gsort<<<1, ZS_THREADS, 0, st>>>(c, c.gkeys, gkeys_b, c.gval, (uint32_t*)temp, gperm);
         }
         k_canon_positions<<<(unsigned)((V + 255) / 256), 256, 0, st>>>(c);
         if (canonical_tail(c.verts, c.perm, V, (const unsigned long long*)V_dev_u64, faces_in, F, (const unsigned long long*)F_dev_u64,

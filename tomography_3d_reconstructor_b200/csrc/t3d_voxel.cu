@@ -70,13 +70,6 @@ bool t3d_first_use_on_device(int slot)
     return first;
 }
 
-int t3d_rows_per_thread(const char* env_name, int dflt)
-{
-    const char* e = getenv(env_name);
-    if (!e) return dflt;
-    const int v = atoi(e);
-    return (v >= 1 && v <= 4096) ? v : dflt;
-}
 extern "C" int t3d_version(void) { return 100; }
 extern "C" int64_t t3d_words_per_row(int W) { return t3d_wpr(W); }
 
@@ -675,8 +668,7 @@ __global__ void __launch_bounds__(256) k_close_ends_fixup(EndsFixArgs a)
 
 bool t3d_pack_gap_supported(const void* masks_u8, int Z, int H, int W, int threshold)
 {
-    static const bool off = getenv("T3D_NO_PACK_GAP") != nullptr;
-    return !off && Z >= 3 && H > 0 && (W & 127) == 0 && ((uintptr_t)masks_u8 & 15) == 0 && threshold >= 1 && threshold <= 255;
+    return Z >= 3 && H > 0 && (W & 127) == 0 && ((uintptr_t)masks_u8 & 15) == 0 && threshold >= 1 && threshold <= 255;
 }
 
 // masks -> gap-filled grid `out` (end planes still raw), per-slice counts (zeroed by the caller; planes 0, 1, Z-2, Z-1
@@ -692,12 +684,10 @@ int t3d_pack_gap_launch(const void* masks_u8, int Z, int H, int W, int threshold
     a.thr4 = 0x01010101u * (uint32_t)threshold;
     const long long n_spans = (a.plane_bytes + 1023) / 1024;
     // about one wave of resident warps (64 per SM); chunks of 16..PG_ZC planes (each chunk re-reads two halo planes)
-    static const int zc_env = t3d_rows_per_thread("T3D_PACK_ZC", 0);
     long long chunks = ((long long)T3D_NUM_SMS * 64 + n_spans - 1) / n_spans;
     if (chunks < 1) chunks = 1;
     int zc = (int)((Z + chunks - 1) / chunks);
     if (zc < 16) zc = 16;
-    if (zc_env > 0) zc = zc_env;
     if (zc > PG_ZC) zc = PG_ZC;
     a.zc = zc;
     a.skip_ends = skip_ends;
@@ -883,8 +873,7 @@ int t3d_morph_stage(const uint32_t* in, uint32_t* out, int Z, int H, int W, int 
     const int nw4 = a.nw / 4;
     a.lanes_x = nw4 < 256 ? nw4 : 256;
     a.pz_per_block = 256 / a.lanes_x;
-    static const int my_env = t3d_rows_per_thread("T3D_MORPH_ROWS", MY);
-    a.my = my_env;
+    a.my = MY;
     a.ring_tail = ring_tail;
     a.counts = counts;
     dim3 grid((nw4 + a.lanes_x - 1) / a.lanes_x, (H + a.my - 1) / a.my, (nz + a.pz_per_block - 1) / a.pz_per_block);
@@ -1106,13 +1095,10 @@ __global__ void __launch_bounds__(512, 1) k_morph4(Morph4Args a)
     }
 }
 
-static int m4_env(const char* name, int dflt) { const char* e = getenv(name); return e && atoi(e) > 0 ? atoi(e) : dflt; }
-
 // can the one-pass kernel take this volume?  (else the four-launch chain runs)
 bool t3d_morph4_eligible(int Z, int H, int W)
 {
-    static const bool off = getenv("T3D_NO_MORPH4") != nullptr;
-    if (off || (W & 127) || W > 4096 || W < 512) return false;
+    if ((W & 127) || W > 4096 || W < 512) return false;
     const int nw4 = W / 128;
     return (32 % nw4) == 0 && Z >= 1 && H >= 1;
 }
@@ -1136,12 +1122,10 @@ int t3d_morph4_launch(const uint32_t* in, uint32_t* out, int Z, int H, int W, in
     if (rows_max > by_smem) rows_max = by_smem;
     rows_max -= rows_max % warp_rows;
     if (rows_max < 9 || rows_max < warp_rows) { t3d_set_error("t3d_morph4: tile does not fit"); return 2; }
-    static const int ty_env = m4_env("T3D_MORPH4_TY", 0), zc_env = m4_env("T3D_MORPH4_ZC", 0);
     const int sms = T3D_NUM_SMS;
     int rows = 0, zc = 0;
     double best = 1e300;
     for (int rr = rows_max; rr >= 16 && rr >= warp_rows; rr -= warp_rows) {
-        if (ty_env && rr != ((ty_env + 8 + warp_rows - 1) / warp_rows) * warp_rows && rr != rows_max) continue;
         const int ty = rr - 8, bands = (H + ty - 1) / ty, thr = rr / M4_R * a.nw4;
         int per_sm = 512 / thr;
         const int smem_fit = (int)((220 * 1024) / ((size_t)(M4_PF + 6) * rr * nw * 4));
@@ -1149,7 +1133,7 @@ int t3d_morph4_launch(const uint32_t* in, uint32_t* out, int Z, int H, int W, in
         if (per_sm < 1) continue;
         static const int zcs[] = {16, 24, 32, 48, 64, 96, 128};
         for (int zi = 0; zi < 7; ++zi) {
-            const int c = zc_env ? zc_env : zcs[zi];
+            const int c = zcs[zi];
             if (c > M4_ZC_MAX) continue;
             const long long ctas = (long long)bands * ((nz + c - 1) / c);
             const double load = (double)((ctas + sms - 1) / sms) * rr;                                   // tile rows per SM per step
@@ -1158,7 +1142,6 @@ int t3d_morph4_launch(const uint32_t* in, uint32_t* out, int Z, int H, int W, in
             if (cost < best) { best = cost; rows = rr; zc = c; }
         }
     }
-    if (ty_env) { rows = ((ty_env + 8 + warp_rows - 1) / warp_rows) * warp_rows; if (rows > rows_max) rows = rows_max; }
     if (rows == 0) { t3d_set_error("t3d_morph4: no tile configuration"); return 2; }
     a.ty = rows - 8;
     const int bands = (H + a.ty - 1) / a.ty;

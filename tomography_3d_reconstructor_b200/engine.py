@@ -878,9 +878,6 @@ def canonicalize_structured(verts, vkeys, faces_i32, sizes, sign_dims, chunkbase
     sync=True: returns (verts, int64 faces) or None when the structured order could not be verified (the caller then sorts
     generically); the clamp group (vertices under slice 0) is provisioned on a second attempt when the first one reports it.
     sync=False: one attempt, returns capacity-sized (verts, faces, device counts (V', F', unverified flag))."""
-    import os
-    if os.environ.get("T3D_NO_STRUCTURED"):
-        return None
     L = _L()
     n_active, nX, nY, nZ, nT = (int(v) for v in sizes)
     V = nX + nY + nZ
