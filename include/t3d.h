@@ -322,6 +322,40 @@ int t3d_mc_vertices_f32(const void* field_f32, int Z, int H, int W, double level
 int t3d_vertex_normals(const void* verts_f32, int64_t V, const void* faces, int64_t F, int faces_are_i64, void* normals_f32,
                        void* stream);
 
+/* Field-gradient vertex normals (DESIGN.md §2): n = -(Gz/dz, Gy/mm_y, Gx/mm_x) / |.|, float32 (V', 3) [z, y, x], G = the
+ * np.gradient of the marched field at the two end nodes of the vertex's grid edge blended with the vertex kernel's weight t,
+ * dz = slope of the variable-depth z map at the vertex (1 without one).  Outward: from field > level to field < level.
+ * Field source as t3d_mc_vertices (occ_bits, pad, gaussian; level 0.5) or, if field_f32 != NULL, that dense (Z,H,W) field at
+ * `level` (t3d_mc_vertices_f32).  vkeys / block sizes / unpad_shift / z_offset / adj (n_cum = the z map's cum length, 0 = none)
+ * as for the vertex kernel.  newid_u32 (NULL: raw order) scatters row i to its canonical slot; perm_u32 (NULL: no vertices
+ * were merged) is the canonicalisation's sorted order and selects the tie rule: a slot that several raw vertices merged into
+ * takes the normal of the one with the smallest edge key (z, y, x, axis).  dup_u64 (optional): the unique pass's "equal pair
+ * seen" flag -- the tie pass returns at once while it reads 0.  winner_u32: scratch of V' entries (tie pass).  The map, the
+ * order, the flag and a dead scratch range of each canonicalisation's workspace are found with t3d_canonical_map_offsets. */
+int t3d_mc_normals(const void* occ_bits, int Z, int H, int W, int pad, int gaussian, const double* weights3_host,
+                   const void* field_f32, double level, const void* vkeys_u64, uint32_t n_x, uint32_t n_y, uint32_t n_z,
+                   int unpad_shift, int z_offset, const void* adj_f64, int n_cum, double mm_per_pixel_y, double mm_per_pixel_x,
+                   const void* newid_u32, const void* perm_u32, const void* dup_u64, void* winner_u32, void* normals_f32,
+                   void* stream);
+/* the same with the block sizes in device memory (sizes_u64 = {n_active, n_x, n_y, n_z, ...}; nothing runs when the raw
+ * vertex count exceeds cap_verts) */
+int t3d_mc_normals_dev(const void* occ_bits, int Z, int H, int W, int pad, int gaussian, const double* weights3_host,
+                       const void* field_f32, double level, const void* vkeys_u64, const void* sizes_u64, uint32_t cap_verts,
+                       int unpad_shift, int z_offset, const void* adj_f64, int n_cum, double mm_per_pixel_y, double mm_per_pixel_x,
+                       const void* newid_u32, const void* perm_u32, const void* dup_u64, void* winner_u32, void* normals_f32,
+                       void* stream);
+/* byte offsets in a canonicalisation's workspace, out4 = {newid (raw -> slot, u32), perm (sorted position -> raw id, u32),
+ * a u32 scratch of >= V entries dead after the call, "equal pair seen" flag (u64; -1 = none)}; valid once the call finished.
+ * kind 0: t3d_mesh_canonicalize (V, F); 1: t3d_mesh_canonicalize_fast[_dev] (V, F); 2: the structured variant with the same
+ * (V, F, cap_z, cap_g0, Zs) it was sized with. */
+int t3d_canonical_map_offsets(int kind, int64_t V, int64_t F, uint32_t cap_z, uint32_t cap_g0, int Zs, int64_t* out4);
+/* Post-step of t3d_reconstruct (same stream, same geometry, capacities and workspace, enqueued after it): field-gradient
+ * normals of the step's canonical mesh into normals_out_f32 (cap_verts, 3), rows [0, V') valid.  Writes nothing else. */
+int t3d_reconstruct_normals(int Z, int H, int W, int n_stages, unsigned erode_mask, int add_padding, const double* weights3_host,
+                            const void* adj_f64, int n_cum, double mm_per_pixel_y, double mm_per_pixel_x, uint32_t cap_active,
+                            uint32_t cap_verts, uint32_t cap_faces, uint32_t cap_zverts, uint32_t cap_g0, const void* results_u64,
+                            void* workspace, void* normals_out_f32, void* stream);
+
 /* ---- device-side mesh consumers: the step right after the path (SURVEY.md 8f-3) ----------------------------- */
 
 /* glb_exporter.py:52-91 create_layer_colors: rgba_u8 (V,4) = grey (200,200,200,255); red where first_start <= z <=

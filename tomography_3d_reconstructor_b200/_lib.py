@@ -97,6 +97,13 @@ SIGNATURES = {
     "t3d_obj_measure": (_i, [_vp, _i64, _vp, _i64, _i, _vp, _vp, _vp]),
     "t3d_obj_emit": (_i, [_vp, _i64, _vp, _i64, _i, _vp, _vp, _vp, _vp]),
     "t3d_vertex_normals": (_i, [_vp, _i64, _vp, _i64, _i, _vp, _vp]),
+    "t3d_mc_normals": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _dbl, _vp, _u32, _u32, _u32, _i, _i, _vp, _i, _dbl, _dbl, _vp, _vp,
+                            _vp, _vp, _vp, _vp]),
+    "t3d_mc_normals_dev": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _dbl, _vp, _vp, _u32, _i, _i, _vp, _i, _dbl, _dbl, _vp, _vp,
+                                _vp, _vp, _vp, _vp]),
+    "t3d_canonical_map_offsets": (_i, [_i, _i64, _i64, _u32, _u32, _i, _vp]),
+    "t3d_reconstruct_normals": (_i, [_i, _i, _i, _i, _c.c_uint, _i, _vp, _vp, _i, _dbl, _dbl, _u32, _u32, _u32, _u32, _u32, _vp, _vp,
+                                     _vp, _vp]),
 }
 
 

@@ -523,6 +523,52 @@ extern "C" int t3d_reconstruct(const void* masks_u8, int Z, int H, int W, int th
     return 0;
 }
 
+// t3d_normals.cu: normals kernel on a strided view (same x_off convention as t3d_mc_vertices_view_dev)
+int t3d_mc_normals_view_dev(const OccView& view, int x_off, const void* vkeys_u64, const void* sizes_u64, uint32_t cap_verts, int unpad_shift,
+                            int z_offset, const void* adj_f64, int n_cum, double mm_per_pixel_y, double mm_per_pixel_x,
+                            const void* newid_u32, const void* perm_u32, const void* dup_u64, void* winner_u32, void* normals_f32,
+                            void* stream);
+
+// Post-step of t3d_reconstruct: field-gradient normals of the step's canonical mesh, enqueued after it on the same stream with
+// the same geometry, capacities and workspace.  Everything it reads is still intact when the step ends: the vertex keys, the
+// sizes in the result block, the raw -> canonical map of the canonicalisation and the field the vertex kernel evaluated (the
+// smoothed occupancy: the padded sign volume on the fast path, bitsC otherwise; neither is written after the vertex kernel).
+// The face flags of the canonicalisation's workspace serve as the tie pass's scratch.  normals_out_f32: (cap_verts, 3), rows
+// [0, V') valid (V' = results[R_VCANON]); nothing runs when the step overflowed.
+extern "C" int t3d_reconstruct_normals(int Z, int H, int W, int n_stages, unsigned erode_mask, int add_padding, const double* weights3_host,
+                                       const void* adj_f64, int n_cum, double mm_per_pixel_y, double mm_per_pixel_x, uint32_t cap_active,
+                                       uint32_t cap_verts, uint32_t cap_faces, uint32_t cap_zverts, uint32_t cap_g0, const void* results_u64,
+                                       void* workspace, void* normals_out_f32, void* stream)
+{
+    if (Z <= 0 || H <= 0 || W <= 0) { t3d_set_error("t3d_reconstruct_normals: empty volume"); return 2; }
+    if (cap_active == 0 || cap_verts == 0 || cap_faces == 0) { t3d_set_error("t3d_reconstruct_normals: zero capacity"); return 2; }
+    const int pad = add_padding ? 1 : 0;
+    const bool fast = fast_surface(n_stages, erode_mask, pad, Z, H, W);
+    const Layout L = make_layout(Z, Z, H, W, pad, cap_active, cap_verts, cap_faces, cap_zverts, cap_g0, n_stages, true, fast);
+    char* ws = (char*)workspace;
+    const unsigned long long* R = (const unsigned long long*)results_u64;
+    const int Zp = Z + 2 * pad, Hp = H + 2 * pad, Wp = fast ? W + S_XPAD + 1 : W + 2 * pad;
+    OccView view;
+    int x_off = 0;
+    if (fast) {
+        const int nws = (int)t3d_words_per_row(Wp);
+        const long long s_ps = (long long)Hp * nws;
+        const uint32_t* S_origin = (const uint32_t*)(ws + L.sign) + s_ps + nws + S_XPAD / 32;
+        view = t3d_make_view_strided(S_origin, Z, H, W, nws, s_ps, 1, 1, weights3_host);
+        x_off = S_XPAD - 1;
+    } else {
+        const void* smoothed = n_stages > 0 ? ws + L.bitsC : ws + L.bitsB;
+        view = t3d_make_view(smoothed, Z, H, W, pad, 1, weights3_host);
+    }
+    int64_t off[4];
+    RUN(t3d_canonical_map_offsets(cap_zverts ? 2 : 1, cap_verts, cap_faces, cap_zverts, cap_g0, Zp, off));
+    char* canon = ws + L.canon;
+    (void)Hp;
+    return t3d_mc_normals_view_dev(view, x_off, ws + L.vkeys, R + R_NACTIVE, cap_verts, 1, 0, adj_f64, n_cum, mm_per_pixel_y,
+                                   mm_per_pixel_x, canon + off[0], canon + off[1], canon + off[3], canon + off[2], normals_out_f32,
+                                   stream);
+}
+
 // ---- z-slab packing: own slices -> planes [halo_lo, halo_lo + n_own) of ext_bits.  The global end slices (fill_first /
 // fill_last) are packed first and hole-filled on the side stream while the other slices are packed; t3d_reconstruct_slab
 // joins the side stream (join_fill), so the halo exchange in between does not wait for the fill.  (The filled slice is

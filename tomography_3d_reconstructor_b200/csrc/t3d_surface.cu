@@ -1209,6 +1209,45 @@ extern "C" int64_t t3d_canonicalize_structured_workspace_bytes(int64_t V, int64_
     return b;
 }
 
+// Where the raw -> canonical map of a canonicalisation lives in its workspace, for consumers enqueued after it (vertex normals):
+// out4 = byte offsets of {newid (u32 per raw vertex: canonical slot), perm (u32 per sorted position: raw id), a u32 scratch of
+// at least V entries that is dead once the call has finished (the face flags), the unique pass's "equal pair seen" flag
+// (u64; -1: the generic path has none, every sorted run may merge)}.
+// kind: 0 = t3d_mesh_canonicalize (V, F), 1 = the fast variants (V, F), 2 = the structured variant (V, F, cap_z, cap_g0, Zs).
+extern "C" int t3d_canonical_map_offsets(int kind, int64_t V, int64_t F, uint32_t cap_z, uint32_t cap_g0, int Zs, int64_t* out4)
+{
+    if (V <= 0 || F < 0 || !out4 || kind < 0 || kind > 2) { t3d_set_error("t3d_canonical_map_offsets: bad arguments"); return 2; }
+    const int64_t n = V > F ? V : F;
+    int64_t o = 0;
+    if (kind == 0) {
+        out4[1] = 2 * align256(4 * V);                           // perm_a: the order after the three passes
+        o = 4 * align256(4 * V);
+        out4[2] = o; o += 2 * align256(4 * n);
+        out4[0] = o;
+        out4[3] = -1;
+        return 0;
+    }
+    if (kind == 1) {
+        o = 2 * align256(8 * V) + align256(4 * V);
+        out4[1] = o; o += align256(4 * V);
+        out4[2] = o; o += 2 * align256(4 * n);
+        out4[0] = o; o += align256(4 * V);
+        o += align256((int64_t)sort64_temp_bytes(V));
+        o += align256(t3d_scan_workspace_bytes(n, 1));
+    } else {
+        o = 2 * align256(8 * (int64_t)cap_z) + 2 * align256(4 * (int64_t)cap_z) + 2 * align256(8 * (int64_t)cap_g0) +
+            2 * align256(4 * (int64_t)cap_g0);
+        out4[1] = o; o += align256(4 * V);
+        out4[2] = o; o += 2 * align256(4 * n);
+        out4[0] = o; o += align256(4 * V);
+        o += align256(4 * (int64_t)cap_g0 + 256);
+        o += 2 * align256(t3d_scan_workspace_bytes(n, 1));
+    }
+    out4[3] = o + 8 * 8;                                         // canonical_tail: dup = totals + 8
+    (void)Zs;
+    return 0;
+}
+
 // the part of the workspace the call needs zeroed on entry (it does so itself unless the range was zeroed up front and
 // registered, see t3d_zero_async): [offset, offset + size) from the start of the workspace
 void t3d_canonicalize_structured_zero_range(int64_t V, int64_t F, uint32_t cap_z, uint32_t cap_g0, int Zs, int64_t* offset,

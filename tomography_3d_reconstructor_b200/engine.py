@@ -154,7 +154,7 @@ class DeviceMesh:
     live in `counts_dev` until resolve() (one D2H copy) or set_sizes() trims them."""
 
     __slots__ = ("_verts", "_faces", "counts_dev", "n_ambiguous", "n_exact", "_measures", "raw", "n_active", "n_raw", "n_z",
-                 "__weakref__")
+                 "normal_src", "canon_map", "_normals", "__weakref__")
 
     def __init__(self, verts: torch.Tensor, faces: torch.Tensor, n_ambiguous: int = 0, n_exact: int = 0,
                  counts_dev: Optional[torch.Tensor] = None):
@@ -165,12 +165,20 @@ class DeviceMesh:
         self.raw = None  # (raw verts, raw faces) of an asynchronous canonicalisation, until the sizes are known
         self.n_active = 0        # active 32-voxel words / raw (vertices, faces): capacity hints for the fused path
         self.n_raw = (0, 0)
+        # field-gradient normals (extract_surface(normals=True)): what the kernel reads -- field source, vertex keys, z map --
+        # and the raw -> canonical map of the canonicalisation (canonical_map(); None: raw vertex order)
+        self.normal_src = None
+        self.canon_map = None
+        self._normals = None
 
     def set_sizes(self, n_verts: int, n_faces: int, unverified: int = 0) -> None:
         """Trim the capacity-sized arrays.  unverified != 0: the fast ordering failed its device-side check, redo the
         canonicalisation with the general three-key sort (degenerate inputs only)."""
         if unverified and self.raw is not None:
-            self._verts, self._faces = canonicalize(self.raw[0], self.raw[1], self._faces.dtype == torch.int64, True, False)
+            keep = {} if self.normal_src is not None else None
+            self._verts, self._faces = canonicalize(self.raw[0], self.raw[1], self._faces.dtype == torch.int64, True, False, keep=keep)
+            if keep is not None:
+                self.canon_map = keep["map"]
         else:
             self._verts, self._faces = self._verts[:n_verts], self._faces[:n_faces]
         self.counts_dev = None
@@ -189,6 +197,14 @@ class DeviceMesh:
     @property
     def faces(self) -> torch.Tensor:
         return self.resolve()._faces
+
+    @property
+    def normals(self) -> Optional[torch.Tensor]:
+        """Field-gradient unit normals, device float32 (V', 3) [z, y, x], row i for vertex i (DESIGN.md §2); None unless the
+        mesh was extracted with normals=True."""
+        if self._normals is None and self.normal_src is not None:
+            self._normals = mesh_normals(self)
+        return self._normals
 
     def measures(self) -> Tuple[float, float]:
         """(signed volume, area), float64 accumulation on the device."""
@@ -727,11 +743,13 @@ def exclusive_scan_u32(x: torch.Tensor, n: int, n_arrays: int, out_u64: bool = F
 def extract_surface(dv: DeviceVolume, slice_depths, mm_per_pixel_y, mm_per_pixel_x, manifold: bool = True,
                     add_padding: bool = True, canonical: Optional[bool] = None, mark=None,
                     z_begin: int = 0, z_end: int = -1, z_offset: int = 0, field: Optional[torch.Tensor] = None,
-                    level: float = 0.5) -> DeviceMesh:
+                    level: float = 0.5, normals: bool = False) -> DeviceMesh:
     """surface_extractor.py:43-68 on the device.  Raises RuntimeError/ValueError where skimage would.
 
     z_begin / z_end / z_offset: z-slab sharding (sharded.py): owned planes of the local sign volume and the global
-    padded plane index of local padded plane 0."""
+    padded plane index of local padded plane 0.
+    normals=True: the mesh keeps what the normals kernel reads, and `mesh.normals` is the device float32 (V', 3) array of
+    field-gradient normals (computed on first access, DESIGN.md §2)."""
     L = _L()
     mark = mark or (lambda _n: None)
     if field is not None:     # march a dense float32 field (SDF path): dv is ignored
@@ -815,40 +833,82 @@ def extract_surface(dv: DeviceVolume, slice_depths, mm_per_pixel_y, mm_per_pixel
                                 z_offset, _p(cum_d), _p(adj_d), n_cum, float(mm_per_pixel_y), float(mm_per_pixel_x),
                                 1 if strong else 0, _p(verts), _stream()), "t3d_mc_vertices")
     mark("mc_vertices")
+    src = None
+    if normals:
+        src = {"occ": None if field is not None else dv.bits, "field": field, "dims": (Z, H, W), "pad": pad, "gaussian": gaussian,
+               "level": float(level) if field is not None else 0.5, "vkeys": vkeys, "blocks": (nX, nY, nZ),
+               "unpad": 1 if manifold else 0, "z_offset": z_offset, "adj": adj_d, "n_cum": n_cum,
+               "mm": (float(mm_per_pixel_y), float(mm_per_pixel_x))}
+    keep = {} if normals else None
     if canonical is None:
         canonical = manifold or field is not None
     if not canonical:
-        return DeviceMesh(verts, faces, n_ambiguous, n_exact)
+        m = DeviceMesh(verts, faces, n_ambiguous, n_exact)
+        m.normal_src = src
+        return m
     if canonical == "async":
         unpad = 1 if (manifold and field is None) else 0
         res = canonicalize_structured(verts, vkeys, faces, (n_active, nX, nY, nZ, nT), (Zs, Hs, Ws), chunkbase, aw_base, n_active,
                                       z_offset, unpad, cum_d, adj_d, n_cum, zkey_bits(slice_depths, add_padding, Zs, z_offset, unpad),
-                                      sync=False)
-        v2, f2, counts = res if res is not None else canonicalize(verts, faces, sync=False, fast=True)
+                                      sync=False, keep=keep)
+        v2, f2, counts = res if res is not None else canonicalize(verts, faces, sync=False, fast=True, keep=keep)
         mark("canonicalize")
         m = DeviceMesh(v2, f2, n_ambiguous, n_exact, counts_dev=counts)
         m.raw = (verts, faces)
         m.n_active, m.n_raw, m.n_z = n_active, (V, nT), nZ
+        if normals:
+            m.normal_src, m.canon_map = src, keep["map"]
         return m
     # structured ordering (no global sort: x-edge vertices are in place, y-edge vertices ranked per row gap, z-edge vertices
     # ordered per cube layer); the generic sort-based path only if its device-side order check fails
     unpad = 1 if (manifold and field is None) else 0
     res = canonicalize_structured(verts, vkeys, faces, (n_active, nX, nY, nZ, nT), (Zs, Hs, Ws), chunkbase, aw_base, n_active,
-                                  z_offset, unpad, cum_d, adj_d, n_cum, zkey_bits(slice_depths, add_padding, Zs, z_offset, unpad))
-    v2, f2 = res if res is not None else canonicalize(verts, faces, fast=True)
+                                  z_offset, unpad, cum_d, adj_d, n_cum, zkey_bits(slice_depths, add_padding, Zs, z_offset, unpad),
+                                  keep=keep)
+    v2, f2 = res if res is not None else canonicalize(verts, faces, fast=True, keep=keep)
     mark("canonicalize")
     m = DeviceMesh(v2, f2, n_ambiguous, n_exact)
     m.n_active, m.n_raw, m.n_z = n_active, (V, nT), nZ
+    if normals:
+        m.normal_src, m.canon_map = src, keep["map"]
     return m
 
 
+def canonical_map(ws: torch.Tensor, kind: int, V: int, F: int, cap_z: int = 0, cap_g0: int = 0, Zs: int = 0):
+    """(newid, perm, scratch, dup flag or None, workspace) of a finished canonicalisation: device addresses of its raw ->
+    canonical map inside workspace `ws` (t3d_canonical_map_offsets; kind 0 generic, 1 fast, 2 structured).  The tuple
+    keeps the workspace alive."""
+    off = (ctypes.c_int64 * 4)()
+    check(_L().t3d_canonical_map_offsets(int(kind), int(V), int(F), int(cap_z), int(cap_g0), int(Zs), off), "t3d_canonical_map_offsets")
+    base = ws.data_ptr()
+    return (base + off[0], base + off[1], base + off[2], base + off[3] if off[3] >= 0 else None, ws)
+
+
+def mesh_normals(mesh: DeviceMesh) -> torch.Tensor:
+    """Field-gradient normals of a mesh from extract_surface(normals=True): one launch of t3d_mc_normals (plus its tie pass
+    when the canonicalisation may have merged vertices), rows in the mesh's vertex order."""
+    src = mesh.normal_src
+    n_rows = int(mesh.verts.shape[0])          # (resolves an asynchronous canonicalisation and its map first)
+    out = torch.empty((n_rows, 3), dtype=torch.float32, device=src["vkeys"].device)
+    newid = perm = dup = scratch = None
+    if mesh.canon_map is not None:
+        newid, perm, scratch, dup = (None if a is None else ctypes.c_void_p(a) for a in mesh.canon_map[:4])
+    Z, H, W = src["dims"]
+    nX, nY, nZ = src["blocks"]
+    check(_L().t3d_mc_normals(_p(src["occ"]), Z, H, W, src["pad"], src["gaussian"], _W3_C, _p(src["field"]), src["level"],
+                              _p(src["vkeys"]), nX, nY, nZ, src["unpad"], src["z_offset"], _p(src["adj"]), src["n_cum"],
+                              src["mm"][0], src["mm"][1], newid, perm, dup, scratch, _p(out), _stream()), "t3d_mc_normals")
+    return out
+
+
 def canonicalize(verts: torch.Tensor, faces_i32: torch.Tensor, faces_i64: bool = True, sync: bool = True,
-                 fast: bool = False):
+                 fast: bool = False, keep: Optional[dict] = None):
     """_ensure_manifold_mesh (surface_extractor.py:115-126) on the device.
 
     fast=True (meshes in t3d_mc_emit's vertex order only): one stable 64-bit (z,y)-key sort, verified on the device;
     if the verification fails the general three-key path runs instead (sync=True) or the caller must do so
-    (sync=False: returns capacity-sized arrays and the device tensor (V', F', unverified-flag))."""
+    (sync=False: returns capacity-sized arrays and the device tensor (V', F', unverified-flag)).
+    keep (a dict): receives keep["map"] = canonical_map(...) of the canonicalisation that produced the result."""
     L = _L()
     V, F = int(verts.shape[0]), int(faces_i32.shape[0])
     dev = verts.device
@@ -864,20 +924,23 @@ def canonicalize(verts: torch.Tensor, faces_i32: torch.Tensor, faces_i64: bool =
         ws = torch.empty(int(L.t3d_canonicalize_workspace_bytes(V, F)) // 8 + 1, dtype=torch.int64, device=dev)
         check(L.t3d_mesh_canonicalize(_p(verts), V, _p(faces_i32), F, _p(vout), f64, f32, _p(counts), _p(ws), _stream()),
               "t3d_mesh_canonicalize")
+    if keep is not None:
+        keep["map"] = canonical_map(ws, 1 if fast else 0, V, F)
     if not sync:
         return vout, fout, counts
     v2, f2, bad = (int(c) for c in counts.cpu().tolist())
     if bad:
-        return canonicalize(verts, faces_i32, faces_i64, True, False)
+        return canonicalize(verts, faces_i32, faces_i64, True, False, keep=keep)
     return vout[:v2], fout[:f2]
 
 
 def canonicalize_structured(verts, vkeys, faces_i32, sizes, sign_dims, chunkbase, aw_base, aw_stride, z_offset, unpad_shift, cum_d,
-                            adj_d, n_cum, zkey_bits_, sync: bool = True):
+                            adj_d, n_cum, zkey_bits_, sync: bool = True, keep: Optional[dict] = None):
     """_ensure_manifold_mesh for a mesh straight out of t3d_mc_emit (t3d_mesh_canonicalize_structured_dev).
     sync=True: returns (verts, int64 faces) or None when the structured order could not be verified (the caller then sorts
     generically); the clamp group (vertices under slice 0) is provisioned on a second attempt when the first one reports it.
-    sync=False: one attempt, returns capacity-sized (verts, faces, device counts (V', F', unverified flag))."""
+    sync=False: one attempt, returns capacity-sized (verts, faces, device counts (V', F', unverified flag)).
+    keep (a dict): receives keep["map"] = canonical_map(...) of the last attempt."""
     L = _L()
     n_active, nX, nY, nZ, nT = (int(v) for v in sizes)
     V = nX + nY + nZ
@@ -894,6 +957,8 @@ def canonicalize_structured(verts, vkeys, faces_i32, sizes, sign_dims, chunkbase
             _p(verts), _p(vkeys), V, _p(sizes_d), _p(sizes_d[5:]), Zs, Hs, Ws, _p(chunkbase), _p(aw_base), int(aw_stride), int(z_offset),
             int(unpad_shift), _p(cum_d), _p(adj_d), int(n_cum), int(zkey_bits_), cap_z, cap_g0, _p(faces_i32), nT, _p(sizes_d[4:]),
             _p(vout), _p(fout), None, _p(counts), _p(counts[3:]), _p(ws), 3, _stream()), "t3d_mesh_canonicalize_structured_dev")
+        if keep is not None:
+            keep["map"] = canonical_map(ws, 2, V, nT, cap_z, cap_g0, Zs)
         if not sync:
             return vout, fout, counts[:3]
         v2, f2, bad, n_g0 = (int(c) for c in counts.cpu().tolist())

@@ -19,13 +19,14 @@ class GLBExporter:
         pass
 
     def export_to_glb(self, vertices: np.ndarray, faces: np.ndarray, filename: str = "tomography_model.glb",
-                      vertex_colors: Optional[np.ndarray] = None) -> bool:
+                      vertex_colors: Optional[np.ndarray] = None, vertex_normals: Optional[np.ndarray] = None) -> bool:
         """glb_exporter.py:26-50.  The reference hands the mesh to trimesh (Trimesh(...), fix_normals(), export 'glb');
         here the binary glTF 2.0 file is written directly: the binary chunk (uint32 indices, float32 positions, uint8
         RGBA COLOR_0) is assembled on the device from the mesh that is already there and downloaded once, the JSON
-        chunk describes it.  Same prints and return values as the reference."""
+        chunk describes it.  Same prints and return values as the reference.  vertex_normals (float32 (V,3), e.g. from
+        SurfaceExtractor.extract_manifold_surface_ex): written as the NORMAL attribute, for smooth shading."""
         try:
-            write_glb(filename, vertices, faces, vertex_colors)
+            write_glb(filename, vertices, faces, vertex_colors, vertex_normals)
             print(f"Model exported: {filename}")
             return True
         except engine.T3DUnavailable:
@@ -59,8 +60,12 @@ class GLBExporter:
         return engine.download(out)
 
 
-def glb_bytes(vertices: np.ndarray, faces: np.ndarray, vertex_colors: Optional[np.ndarray] = None) -> bytes:
-    """The GLB file as bytes: 12-byte header, JSON chunk, BIN chunk (glTF 2.0 binary container)."""
+def glb_bytes(vertices: np.ndarray, faces: np.ndarray, vertex_colors: Optional[np.ndarray] = None,
+              vertex_normals: Optional[np.ndarray] = None) -> bytes:
+    """The GLB file as bytes: 12-byte header, JSON chunk, BIN chunk (glTF 2.0 binary container).  vertex_normals: float32
+    (V,3) [z,y,x] like the vertices, appended after the rest of the binary chunk as a NORMAL accessor; the normals point
+    out of the object by definition, so the winding fix below leaves them as they are.  Without them the file is what it
+    was before normals existed, byte for byte."""
     import json
     import struct
     L = engine._L()
@@ -76,6 +81,12 @@ def glb_bytes(vertices: np.ndarray, faces: np.ndarray, vertex_colors: Optional[n
         if c.shape != (V, 4) or c.dtype != np.uint8:
             raise ValueError("vertex_colors must be (V, 4) uint8 RGBA")
         colors = torch.from_numpy(c).to(dev)
+    normals = None
+    if vertex_normals is not None:
+        n = np.ascontiguousarray(vertex_normals)
+        if n.shape != (V, 3) or n.dtype != np.float32:
+            raise ValueError("vertex_normals must be (V, 3) float32")
+        normals = torch.from_numpy(n).to(dev)
     # trimesh.fix_normals(): a closed, consistently wound mesh is turned inside out when its signed volume is negative
     signed_volume, _area = mesh.measures() if hasattr(mesh, "measures") else engine.mesh_measure(verts, fcs)
     flip = 1 if signed_volume < 0 else 0
@@ -85,6 +96,8 @@ def glb_bytes(vertices: np.ndarray, faces: np.ndarray, vertex_colors: Optional[n
     check(L.t3d_glb_pack(engine._p(verts), V, engine._p(fcs), F, 1 if fcs.dtype == torch.int64 else 0, engine._p(colors), flip,
                          engine._p(payload), engine._p(minmax), engine._stream()), "t3d_glb_pack")
     mm = minmax.cpu().tolist()
+    if normals is not None:
+        payload = torch.cat([payload, normals.view(-1).view(torch.uint8)])
     blob = engine.download(payload)
     views = [{"buffer": 0, "byteOffset": 0, "byteLength": 12 * F, "target": 34963},
              {"buffer": 0, "byteOffset": 12 * F, "byteLength": 12 * V, "target": 34962}]
@@ -95,6 +108,11 @@ def glb_bytes(vertices: np.ndarray, faces: np.ndarray, vertex_colors: Optional[n
         views.append({"buffer": 0, "byteOffset": 12 * F + 12 * V, "byteLength": 4 * V, "target": 34962})
         accessors.append({"bufferView": 2, "componentType": 5121, "normalized": True, "count": V, "type": "VEC4"})
         attributes["COLOR_0"] = 2
+    if normals is not None:
+        views.append({"buffer": 0, "byteOffset": nbytes, "byteLength": 12 * V, "target": 34962})
+        accessors.append({"bufferView": len(views) - 1, "componentType": 5126, "count": V, "type": "VEC3"})
+        attributes["NORMAL"] = len(accessors) - 1
+        nbytes += 12 * V
     doc = {"asset": {"version": "2.0", "generator": "tomography_3d_reconstructor_b200"},
            "scene": 0, "scenes": [{"nodes": [0]}], "nodes": [{"name": "tomography_model", "mesh": 0}],
            "meshes": [{"name": "tomography_model", "primitives": [{"attributes": attributes, "indices": 0, "mode": 4}]}],
@@ -107,15 +125,17 @@ def glb_bytes(vertices: np.ndarray, faces: np.ndarray, vertex_colors: Optional[n
                      struct.pack("<I4s", nbytes + pad, b"BIN\x00"), blob.tobytes(), b"\x00" * pad])
 
 
-def write_glb(filename: str, vertices: np.ndarray, faces: np.ndarray, vertex_colors: Optional[np.ndarray] = None) -> None:
-    data = glb_bytes(vertices, faces, vertex_colors)
+def write_glb(filename: str, vertices: np.ndarray, faces: np.ndarray, vertex_colors: Optional[np.ndarray] = None,
+              vertex_normals: Optional[np.ndarray] = None) -> None:
+    data = glb_bytes(vertices, faces, vertex_colors, vertex_normals)
     with open(filename, "wb") as f:
         f.write(data)
 
 
-def parse_glb(data: bytes):
+def parse_glb(data: bytes, with_normals: bool = False):
     """Minimal reader of what write_glb produces (used by the tests and tools/run_orchestrator.py to re-parse the file):
-    returns (positions (V,3) f32, indices (F,3) u32, colours (V,4) u8 or None, json document)."""
+    returns (positions (V,3) f32, indices (F,3) u32, colours (V,4) u8 or None, json document); with_normals=True:
+    (positions, indices, colours, normals (V,3) f32 or None, json document)."""
     import json
     import struct
     magic, version, total = struct.unpack_from("<4sII", data, 0)
@@ -138,4 +158,7 @@ def parse_glb(data: bytes):
     pos = read(prim["attributes"]["POSITION"], np.float32, 3)
     idx = read(prim["indices"], np.uint32, 1).reshape(-1, 3)
     col = read(prim["attributes"]["COLOR_0"], np.uint8, 4) if "COLOR_0" in prim["attributes"] else None
+    if with_normals:
+        nrm = read(prim["attributes"]["NORMAL"], np.float32, 3) if "NORMAL" in prim["attributes"] else None
+        return pos, idx, col, nrm, doc
     return pos, idx, col, doc

@@ -49,10 +49,11 @@ def variable_depth_volume(counts: np.ndarray, mm_x: float, mm_y: float, depths: 
 
 def reconstruct(masks_u8: torch.Tensor, threshold: int, side_counts, total_depth_mm: float, x_length_mm: float,
                 y_length_mm: float, iterations: int = 3, close_ends: bool = True, add_padding: bool = True,
-                mark: Optional[Callable[[str], None]] = None) -> Dict:
+                mark: Optional[Callable[[str], None]] = None, normals: bool = False) -> Dict:
     """masks_u8: CUDA uint8 (Z,H,W).  Returns the device mesh and the host scalars of analyze_object_properties.
 
-    `mark(name)` is called after each stage has been enqueued (bench.py records CUDA events there)."""
+    `mark(name)` is called after each stage has been enqueued (bench.py records CUDA events there).
+    normals=True: also "normals", the device float32 (V', 3) field-gradient normals of the mesh (DESIGN.md §2)."""
     mark = mark or (lambda _n: None)
     Z, H, W = (int(s) for s in masks_u8.shape)
     mm_x, mm_y = x_length_mm / W, y_length_mm / H
@@ -72,7 +73,7 @@ def reconstruct(masks_u8: torch.Tensor, threshold: int, side_counts, total_depth
         bbox_done.record(side)
     sm = engine.smooth(dv, iterations, True)
     mark("smooth")
-    mesh = engine.extract_surface(sm, depths, mm_y, mm_x, True, add_padding, canonical="async", mark=mark)
+    mesh = engine.extract_surface(sm, depths, mm_y, mm_x, True, add_padding, canonical="async", mark=mark, normals=normals)
     # measures on the emitted (pre-canonical) mesh: merging exact duplicates and dropping zero-area faces changes
     # neither the signed volume nor the area, and it removes a dependency on the canonical sizes
     raw_verts, raw_faces = mesh.raw
@@ -93,7 +94,7 @@ def reconstruct(masks_u8: torch.Tensor, threshold: int, side_counts, total_depth
     dv.set_host_stats(raw_counts, bb)
     sm.set_host_stats(sm_counts, None)
     bbox = dv.bbox()
-    return {
+    out = {
         "mesh": mesh,
         "voxel_volume_mm3": variable_depth_volume(raw_counts, mm_x, mm_y, depths),
         "processed_voxel_volume_mm3": variable_depth_volume(sm_counts, mm_x, mm_y, depths),
@@ -103,6 +104,9 @@ def reconstruct(masks_u8: torch.Tensor, threshold: int, side_counts, total_depth
         "active_voxels": int(raw_counts.sum()),
         "slice_depths": depths,
     }
+    if normals:
+        out["normals"] = mesh.normals
+    return out
 
 
 def sdf_sampling(depths: np.ndarray, mm_y: float, mm_x: float):
@@ -147,10 +151,11 @@ R_NAMBIGUOUS, R_NEXACT, R_VOLUME, R_AREA, R_BBOX, R_VRAW, R_NG0, R_COUNTS = 9, 1
 class FusedPlan:
     """Buffers + (optionally) a captured CUDA graph for one problem shape.  Data-dependent sizes stay on the device;
     buffers are capacity-sized from hints (a previous run of the same input) and the result block reports overflow.
-    The mesh returned by run() lives in the plan's output buffers: valid until the next run()."""
+    The mesh returned by run() lives in the plan's output buffers: valid until the next run().
+    normals=True: every step is followed by t3d_reconstruct_normals (in the same graph), into `self.normals`."""
 
     def __init__(self, shape, threshold, side_counts, total_depth_mm, x_length_mm, y_length_mm, iterations, close_ends,
-                 add_padding, caps, device):
+                 add_padding, caps, device, normals: bool = False):
         L = engine._L()
         self.shape = Z, H, W = tuple(int(v) for v in shape)
         self.threshold, self.close_ends, self.add_padding = int(threshold), bool(close_ends), bool(add_padding)
@@ -172,6 +177,7 @@ class FusedPlan:
         self.ws = torch.empty(nbytes // 8 + 1, dtype=torch.int64, device=device)
         self.verts = torch.empty((self.caps[1], 3), dtype=torch.float32, device=device)
         self.faces = torch.empty((self.caps[2], 3), dtype=torch.int64, device=device)
+        self.normals = torch.empty((self.caps[1], 3), dtype=torch.float32, device=device) if normals else None
         self.n_res = int(L.t3d_reconstruct_results_len(Z))
         self.res = torch.zeros(self.n_res, dtype=torch.int64, device=device)
         self.res_host = torch.zeros(self.n_res, dtype=torch.int64, pin_memory=True)
@@ -187,6 +193,11 @@ class FusedPlan:
             1 if self.add_padding else 0, engine._W3_C, p(self.cum_d), p(self.adj_d), self.n_cum, float(self.mm_y),
             float(self.mm_x), 0, self.caps[0], self.caps[1], self.caps[2], self.caps[3], self.caps[4], self.zkey_bits, p(self.verts),
             p(self.faces), p(self.res), p(self.ws), engine._stream()), "t3d_reconstruct")
+        if self.normals is not None:
+            engine.check(engine._L().t3d_reconstruct_normals(
+                Z, H, W, self.n_stages, self.erode_mask, 1 if self.add_padding else 0, engine._W3_C, p(self.adj_d), self.n_cum,
+                float(self.mm_y), float(self.mm_x), *self.caps, p(self.res), p(self.ws), p(self.normals), engine._stream()),
+                "t3d_reconstruct_normals")
 
     def capture(self, masks_u8: torch.Tensor) -> None:
         """Record the step for this input buffer into a CUDA graph (after one eager warm-up run)."""
@@ -246,21 +257,31 @@ def _caps_from(n_active: int, v_raw: int, f_raw: int, n_z: int, n_g0: int = 0):
     return _grow(n_active), _grow(v_raw), _grow(f_raw), _grow(n_z), (_grow(n_g0) if n_g0 > 0 else 0)
 
 
+def plan_key(masks_u8: torch.Tensor, threshold: int, side_counts, total_depth_mm: float, x_length_mm: float,
+             y_length_mm: float, iterations: int = 3, close_ends: bool = True, add_padding: bool = True, normals: bool = False):
+    """Key of the fused plan / capacity hints of one problem (plans with and without normals are distinct)."""
+    Z, H, W = (int(s) for s in masks_u8.shape)
+    key = (Z, H, W, int(threshold), tuple(side_counts), float(total_depth_mm), float(x_length_mm), float(y_length_mm),
+           int(iterations), bool(close_ends), bool(add_padding), masks_u8.device.index)
+    return key + ("normals",) if normals else key
+
+
 def reconstruct_fused(masks_u8: torch.Tensor, threshold: int, side_counts, total_depth_mm: float, x_length_mm: float,
                       y_length_mm: float, iterations: int = 3, close_ends: bool = True, add_padding: bool = True,
-                      use_graph: bool = True) -> Dict:
+                      use_graph: bool = True, normals: bool = False) -> Dict:
     """Same contract as reconstruct(), executed as one graph launch + one device->host copy.
 
     The first call for a given (shape, parameters) runs the staged path to learn the mesh size; later calls reuse a
     FusedPlan.  If the input changes so much that a capacity overflows (or the fast vertex ordering cannot be
-    verified) the staged path runs instead and the hints are refreshed."""
+    verified) the staged path runs instead and the hints are refreshed.
+    normals=True: out["normals"] is the device float32 (V', 3) array of field-gradient normals (DESIGN.md §2)."""
     Z, H, W = (int(s) for s in masks_u8.shape)
-    key = (Z, H, W, int(threshold), tuple(side_counts), float(total_depth_mm), float(x_length_mm), float(y_length_mm),
-           int(iterations), bool(close_ends), bool(add_padding), masks_u8.device.index)
+    key = plan_key(masks_u8, threshold, side_counts, total_depth_mm, x_length_mm, y_length_mm, iterations, close_ends, add_padding,
+                   normals)
 
     def staged():
         out = reconstruct(masks_u8, threshold, side_counts, total_depth_mm, x_length_mm, y_length_mm, iterations, close_ends,
-                          add_padding)
+                          add_padding, normals=normals)
         m = out["mesh"]
         _hints[key] = _caps_from(m.n_active, *m.n_raw, m.n_z)
         return out
@@ -271,7 +292,7 @@ def reconstruct_fused(masks_u8: torch.Tensor, threshold: int, side_counts, total
     plan = _plans.get(key)
     if plan is None or any(c < h for c, h in zip(plan.caps, caps)) or (plan.caps[3] == 0) != (caps[3] == 0):
         plan = FusedPlan((Z, H, W), threshold, side_counts, total_depth_mm, x_length_mm, y_length_mm, iterations,
-                         close_ends, add_padding, caps, masks_u8.device)
+                         close_ends, add_padding, caps, masks_u8.device, normals)
         _plans[key] = plan
     if use_graph and plan.graph_ptr != masks_u8.data_ptr():
         plan.capture(masks_u8)
@@ -281,7 +302,7 @@ def reconstruct_fused(masks_u8: torch.Tensor, threshold: int, side_counts, total
     if h[R_UNVERIFIED] and not h[R_OVERFLOW] and plan.caps[3] and _retune(key, h[R_NG0], plan.caps[4]):
         _plans.pop(key, None)
         return reconstruct_fused(masks_u8, threshold, side_counts, total_depth_mm, x_length_mm, y_length_mm, iterations,
-                                 close_ends, add_padding, use_graph)
+                                 close_ends, add_padding, use_graph, normals)
     if h[R_OVERFLOW] or h[R_UNVERIFIED] or h[R_NT] == 0:
         _plans.pop(key, None)
         _hints.pop(key, None)
@@ -313,7 +334,7 @@ def _result_from_block(plan: "FusedPlan", r: np.ndarray, h: list, hints_key=None
     n = min(Z, len(plan.depths))
     vols = np.cumsum(counts2[:, :n].astype(np.float64) * plan.vol_weights[:n], axis=1)[:, -1].tolist() if n else [0.0, 0.0]
     bb = r[R_BBOX:R_BBOX + 3].view(np.int32).tolist()
-    return {
+    out = {
         "mesh": mesh,
         "voxel_volume_mm3": vols[0],
         "processed_voxel_volume_mm3": vols[1],
@@ -323,17 +344,22 @@ def _result_from_block(plan: "FusedPlan", r: np.ndarray, h: list, hints_key=None
         "active_voxels": int(counts2[0].sum()),
         "slice_depths": plan.depths,
     }
+    if plan.normals is not None:
+        out["normals"] = plan.normals[:canon[0]]
+    return out
 
 
 _device_inputs: Dict = {}
 
 
 def reconstruct_host(mask_images, threshold: int, side_counts, total_depth_mm: float, x_length_mm: float, y_length_mm: float,
-                     iterations: int = 3, close_ends: bool = True, add_padding: bool = True, use_graph: bool = True) -> Dict:
+                     iterations: int = 3, close_ends: bool = True, add_padding: bool = True, use_graph: bool = True,
+                     normals: bool = False) -> Dict:
     """The whole path on HOST data, as one call: a list of (H,W) bool / uint8 masks (what ImageLoader returns,
     image_loader.py:97-109) or a (Z,H,W) array -> one host->device copy -> reconstruct_fused -> the mesh as numpy arrays
     (out["vertices"] f32 (V,3) [z,y,x] mm, out["faces"] int64 (F,3)) + the scalars of reconstruct().  bool masks:
-    pass threshold=1.  The intermediate voxel grids stay on the device (the class API has to return them as arrays)."""
+    pass threshold=1.  The intermediate voxel grids stay on the device (the class API has to return them as arrays).
+    normals=True: also out["normals"], float32 (V,3) field-gradient unit normals, row i for vertex i (DESIGN.md §2)."""
     _src, Z, H, W, _pinned = engine.mask_source(mask_images)
     dev = engine._require_cuda()
     key = ((Z, H, W), torch.cuda.current_device())
@@ -343,12 +369,18 @@ def reconstruct_host(mask_images, threshold: int, side_counts, total_depth_mm: f
     # one async copy from a pinned stack; a list of pageable masks is gathered through the pinned staging ring
     engine.upload_masks(mask_images, buf)
     out = reconstruct_fused(buf, threshold, side_counts, total_depth_mm, x_length_mm, y_length_mm, iterations, close_ends,
-                            add_padding, use_graph)
+                            add_padding, use_graph, normals)
     v, f = out["mesh"].verts.contiguous(), out["mesh"].faces.contiguous()
     hv = torch.empty(v.shape, dtype=v.dtype, pin_memory=True)
     hf = torch.empty(f.shape, dtype=f.dtype, pin_memory=True)
     hv.copy_(v, non_blocking=True)
     hf.copy_(f, non_blocking=True)
+    if normals:
+        n = out["normals"].contiguous()
+        hn = torch.empty(n.shape, dtype=n.dtype, pin_memory=True)
+        hn.copy_(n, non_blocking=True)
     torch.cuda.current_stream().synchronize()
     out["vertices"], out["faces"] = hv.numpy(), hf.numpy()
+    if normals:
+        out["normals"] = hn.numpy()
     return out
