@@ -84,10 +84,12 @@ int t3d_point_cloud_emit(const void* bits, int Z, int H, int W, const void* row_
                          const void* z_centre_mm_f64, double mm_per_pixel_y, double mm_per_pixel_x, void* out_f64,
                          void* stream);
 
-/* generic exclusive scan of n_arrays uint32 arrays of length n (array k at in + k*n) */
+/* generic exclusive scan of n_arrays uint32 arrays of n_cap elements, `stride` elements apart (array k at in + k*stride),
+ * into uint32 (out_is_u64 = 0) or uint64 (1) arrays of the same layout; popcount_input = 1 scans popcount(in[i]).
+ * totals_u64: n_arrays uint64.  n_dev_u64: the true length in device memory (at most n_cap); NULL = the capacity is the size. */
 int64_t t3d_scan_workspace_bytes(int64_t n, int n_arrays);
-int t3d_exclusive_scan_u32(const void* in, void* out, int64_t n, int n_arrays, int out_is_u64, int popcount_input,
-                           void* totals_u64, void* workspace, void* stream);
+int t3d_exclusive_scan_u32_dev(const void* in, void* out, int64_t n_cap, int64_t stride, int n_arrays, int out_is_u64,
+                               int popcount_input, const void* n_dev_u64, void* totals_u64, void* workspace, void* stream);
 
 /* ---- SurfaceExtractor.extract_manifold_surface  (surface_extractor.py:34-75) ---------------------------- */
 
@@ -104,25 +106,28 @@ int t3d_field_sign_lean(const void* occ_bits, int Z, int H, int W, int pad, cons
                         void* n_exact_u64, void* exc_list_u64, uint32_t exc_cap, void* exc_count_u64, void* stream);
 
 /* Two-pass marching cubes on a sign volume (Zs,Hs,Ws) = skimage.measure.marching_cubes(volume, 0.5), sparse after the
- * first dense pass (see csrc/t3d_mc.cu):
- *   t3d_mc_flags    -> ballots_u32[t3d_mc_num_chunks]: bit l of word c set iff sign word 32c+l owns a cut edge or an
- *                      active cube origin
- *   (caller) exclusive scan of popcount(ballots) -> chunkbase_u32, n_active
- *   t3d_mc_words    -> aw_idx_u32[n_active] (flat word index) and aw_cnt_u32[4][n_active] (owned x/y/z cut edges,
- *                      triangles); n_ambiguous_u64: cubes tiled through Lewiner's face / interior tests (mc_field)
- *   (caller) exclusive scan of aw_cnt -> aw_base_u32, totals n_x, n_y, n_z, n_t
- *   t3d_mc_emit     -> vkeys_u64[n_x+n_y+n_z] (edge key per vertex) and faces_i32 (n_t,3): reference cube order,
- *                      reversed winding (gradient_direction='descent')
- *   t3d_mc_vertices -> verts_f32 (V,3) [z,y,x]: skimage's interpolation on the exact float64 field, then un-pad,
- *                      variable-depth z map and mm scaling (surface_extractor.py:57-65, 82-113).
+ * first dense pass (see csrc/t3d_mc.cu).  The data-dependent sizes stay in device memory, in the block
+ * sizes_u64 = {n_active, n_x, n_y, n_z, n_t} that the two scans write their totals into; arrays are capacity-sized
+ * (cap_active, cap_verts, cap_faces) and nothing is written beyond a capacity, so the whole sequence needs no host round
+ * trip and can be graph-captured.  A caller that has read the sizes back passes capacities equal to them.
+ *   t3d_mc_flags        -> ballots_u32[t3d_mc_num_chunks]: bit l of word c set iff sign word 32c+l owns a cut edge or an
+ *                          active cube origin
+ *   (caller) t3d_exclusive_scan_u32_dev of popcount(ballots) -> chunkbase_u32, total n_active -> sizes_u64[0]
+ *   t3d_mc_words_dev    -> aw_idx_u32[n_active] (flat word index) and aw_cnt_u32[4][cap_active] (owned x/y/z cut edges,
+ *                          triangles); n_ambiguous_u64: cubes tiled through Lewiner's face / interior tests (mc_field)
+ *   (caller) t3d_exclusive_scan_u32_dev of aw_cnt -> aw_base_u32, totals n_x, n_y, n_z, n_t -> sizes_u64[1..4]
+ *   t3d_mc_emit_dev     -> vkeys_u64[n_x+n_y+n_z] (edge key per vertex) and faces_i32 (n_t,3): reference cube order,
+ *                          reversed winding (gradient_direction='descent')
+ *   t3d_mc_vertices_dev -> verts_f32 (V,3) [z,y,x]: skimage's interpolation on the exact float64 field, then un-pad,
+ *                          variable-depth z map and mm scaling (surface_extractor.py:57-65, 82-113).
  * z_begin/z_end: owned planes of the sign volume ([0, Zs) on one device; -1 = Zs).  With z-slab sharding a rank owns
  * [z_begin, z_end) and additionally emits the x/y-edge vertices of ghost plane z_end; z_offset is the global padded
  * plane index of local padded plane 0. */
-/* The marched field as the ambiguity tests of t3d_mc_words / t3d_mc_emit see it.  Cubes whose index has an ambiguous face
- * (Lewiner's cases 3, 6, 7, 10, 12, 13) or is case 4 are tiled by the row that Lewiner's face test (asymptotic decider) and
+/* The marched field as the ambiguity tests of t3d_mc_words_dev / t3d_mc_emit_dev see it.  Cubes whose index has an ambiguous
+ * face (Lewiner's cases 3, 6, 7, 10, 12, 13) or is case 4 are tiled by the row that Lewiner's face test (asymptotic decider) and
  * interior test select (csrc/mc33_tables.h; oracle/mc_ref.c restates the same decisions); both need the corner VALUES:
  *   field_f32 != NULL: dense float32 field of the sign volume's own shape (Z,H,W), marched at `level`;
- *   else occ_bits != NULL: Gaussian(0.5) (gaussian = 1) of the occupancy (Z,H,W) padded by `pad`, as for t3d_mc_vertices;
+ *   else occ_bits != NULL: Gaussian(0.5) (gaussian = 1) of the occupancy (Z,H,W) padded by `pad`, as for t3d_mc_vertices_dev;
  *   NULL struct: only the signs are known (values level +- 0.5: every face test is a tie -> positive corners joined). */
 typedef struct t3d_mc_field {
     const void* occ_bits;
@@ -134,19 +139,22 @@ typedef struct t3d_mc_field {
 
 int64_t t3d_mc_num_chunks(int Zs, int Hs, int Ws);
 int t3d_mc_flags(const void* sign_bits, int Zs, int Hs, int Ws, int z_begin, int z_end, void* ballots_u32, void* stream);
-int t3d_mc_words(const void* sign_bits, int Zs, int Hs, int Ws, int z_begin, int z_end, const void* ballots_u32,
-                 const void* chunkbase_u32,
-                 uint32_t n_active, void* aw_idx_u32, void* aw_cnt_u32, void* n_ambiguous_u64, const t3d_mc_field* mc_field,
-                 void* stream);
-int t3d_mc_emit(const void* sign_bits, int Zs, int Hs, int Ws, int z_begin, int z_end, const void* ballots_u32,
-                const void* chunkbase_u32,
-                const void* aw_idx_u32, const void* aw_base_u32, uint32_t n_active, uint32_t n_x, uint32_t n_y,
-                void* vkeys_u64, void* faces_i32, const t3d_mc_field* mc_field, void* stream);
-int t3d_mc_vertices(const void* occ_bits, int Z, int H, int W, int pad, int gaussian, const double* weights3_host,
-                    const void* vkeys_u64, uint32_t n_x, uint32_t n_y, uint32_t n_z, int unpad_shift, int z_offset,
-                    const void* cum_f64,
-                    const void* adj_f64, int n_cum, double mm_per_pixel_y, double mm_per_pixel_x, int scale_in_f64,
-                    void* verts_f32, void* stream);
+int t3d_mc_words_dev(const void* sign_bits, int Zs, int Hs, int Ws, int z_begin, int z_end, const void* ballots_u32,
+                     const void* chunkbase_u32, uint32_t cap_active, const void* sizes_u64, void* aw_idx_u32, void* aw_cnt_u32,
+                     void* n_ambiguous_u64, const t3d_mc_field* mc_field, void* stream);
+/* parts 1: vertex keys; 2: faces (the words without an ambiguous cube, then the others: two launches); 3: both in one launch */
+int t3d_mc_emit_dev(const void* sign_bits, int Zs, int Hs, int Ws, int z_begin, int z_end, const void* ballots_u32,
+                    const void* chunkbase_u32, const void* aw_idx_u32, const void* aw_base_u32, uint32_t cap_active,
+                    const void* sizes_u64, uint32_t cap_verts, uint32_t cap_faces, void* vkeys_u64, void* faces_i32,
+                    int parts, const t3d_mc_field* mc_field, void* stream);
+/* Field: occ_bits as t3d_field_sign had it (pad / gaussian; gaussian = 0: the sign volume IS the occupancy and pad must be 0,
+ * level 0.5), or field_f32 != NULL: the dense (Z,H,W) field the sign volume was taken from (t3d_sign_from_f32), at `level`.
+ * cum/adj: device float64 arrays of the variable-slice-depth z map (n_cum = 0 disables it). */
+int t3d_mc_vertices_dev(const void* occ_bits, int Z, int H, int W, int pad, int gaussian, const double* weights3_host,
+                        const void* field_f32, double level, const void* vkeys_u64, const void* sizes_u64, uint32_t cap_verts,
+                        int unpad_shift, int z_offset, const void* cum_f64, const void* adj_f64, int n_cum, double mm_per_pixel_y,
+                        double mm_per_pixel_x, int scale_in_f64, int which_blocks /* 1: x-edge, 2: y-edge, 4: z-edge vertices */,
+                        void* verts_f32, void* stream);
 
 /* test aids: the float32 field itself and the uint8 cube-case volume */
 int t3d_field_dense(const void* occ_bits, int Z, int H, int W, int pad, int gaussian, const double* weights3_host,
@@ -159,44 +167,21 @@ int64_t t3d_canonicalize_workspace_bytes(int64_t V, int64_t F);
 int t3d_mesh_canonicalize(const void* verts_in, int64_t V, const void* faces_in, int64_t F, void* verts_out,
                           void* faces_out_i64, void* faces_out_i32, void* counts_u64, void* workspace, void* stream);
 
-/* Same outputs for meshes in t3d_mc_emit's vertex order ([x|y|z]-edge blocks, raster order inside each): ONE stable
- * 64-bit (z,y)-key sort; counts_u64 has 3 entries, [2] != 0 = ordering not verified, call t3d_mesh_canonicalize. */
+/* Same outputs for meshes in t3d_mc_emit_dev's vertex order ([x|y|z]-edge blocks, raster order inside each): ONE stable
+ * 64-bit (z,y)-key sort; counts_u64 has 3 entries, [2] != 0 = ordering not verified, call t3d_mesh_canonicalize.
+ * V_dev_u64 / F_dev_u64: the true vertex / face counts in device memory (at most the capacities); NULL = the capacity is
+ * the size. */
 int64_t t3d_canonicalize_fast_workspace_bytes(int64_t V, int64_t F);
-int t3d_mesh_canonicalize_fast(const void* verts_in, int64_t V, const void* faces_in, int64_t F, void* verts_out,
-                               void* faces_out_i64, void* faces_out_i32, void* counts_u64, void* workspace, void* stream);
-
-/* calculate_mesh_volume / calculate_surface_area (surface_extractor.py:128-148): out_f64 = {signed volume, area} */
-int64_t t3d_mesh_measure_workspace_bytes(void);
-int t3d_mesh_measure(const void* verts_f32, int64_t V, const void* faces, int64_t F, int faces_are_i64, void* out_f64,
-                     void* workspace, void* stream);
-
-/* ---- device-resident sizes: the whole path as one enqueue --------------------------------------------------
- * Variants whose data-dependent sizes stay in device memory (sizes_u64 = {n_active, n_x, n_y, n_z, n_t}, or a single
- * uint64): arrays are capacity-sized, nothing is written beyond a capacity, no host round trip => graph-capturable. */
-int t3d_exclusive_scan_u32_dev(const void* in, void* out, int64_t n_cap, int64_t stride, int n_arrays, int out_is_u64,
-                               int popcount_input, const void* n_dev_u64, void* totals_u64, void* workspace, void* stream);
-int t3d_mc_words_dev(const void* sign_bits, int Zs, int Hs, int Ws, int z_begin, int z_end, const void* ballots_u32,
-                     const void* chunkbase_u32, uint32_t cap_active, const void* sizes_u64, void* aw_idx_u32, void* aw_cnt_u32,
-                     void* n_ambiguous_u64, const t3d_mc_field* mc_field, void* stream);
-int t3d_mc_emit_dev(const void* sign_bits, int Zs, int Hs, int Ws, int z_begin, int z_end, const void* ballots_u32,
-                    const void* chunkbase_u32, const void* aw_idx_u32, const void* aw_base_u32, uint32_t cap_active,
-                    const void* sizes_u64, uint32_t cap_verts, uint32_t cap_faces, void* vkeys_u64, void* faces_i32,
-                    int parts /* 1: vertex keys, 2: faces, 3: both */, const t3d_mc_field* mc_field, void* stream);
-int t3d_mc_vertices_dev(const void* occ_bits, int Z, int H, int W, int pad, int gaussian, const double* weights3_host,
-                        const void* vkeys_u64, const void* sizes_u64, uint32_t cap_verts, int unpad_shift, int z_offset,
-                        const void* cum_f64, const void* adj_f64, int n_cum, double mm_per_pixel_y, double mm_per_pixel_x,
-                        int scale_in_f64, int which_blocks /* 1: x-edge, 2: y-edge, 4: z-edge vertices */, void* verts_f32,
-                        void* stream);
 int t3d_mesh_canonicalize_fast_dev(const void* verts_in, int64_t V_cap, const void* V_dev_u64, const void* faces_in, int64_t F_cap,
                                    const void* F_dev_u64, void* verts_out, void* faces_out_i64, void* faces_out_i32,
                                    void* counts_u64, void* workspace, void* stream);
 /* Structured canonical order (same outputs as t3d_mesh_canonicalize_fast_dev, a third of the sorting work): uses the
- * vertex keys of t3d_mc_emit.  x-edge vertices are already in order, y-edge vertices are ranked inside their (plane, row
+ * vertex keys of t3d_mc_emit_dev.  x-edge vertices are already in order, y-edge vertices are ranked inside their (plane, row
  * gap) segment, z-edge vertices get one stable radix sort by (layer, z) over cap_z entries, final positions come from
  * the per-row prefix counts of the emit pass (chunkbase_u32 / aw_base_u32 with array stride aw_stride, as passed to
  * t3d_mc_emit_dev; Zs,Hs,Ws = the marched sign volume).  The vertices the z map clamps onto z = 0 (surface_extractor.py:100-103;
  * non-empty only when the object touches slice 0) are ordered by a generic (y,x) sort over cap_g0 entries (0 = not
- * provisioned).  sizes_u64 = {n_active, n_x, n_y, n_z, n_t}; Zs / z_offset / unpad_shift / n_cum as for t3d_mc_vertices.
+ * provisioned).  sizes_u64 = {n_active, n_x, n_y, n_z, n_t}; Zs / z_offset / unpad_shift / n_cum as for t3d_mc_vertices_dev.
  * counts_u64[2] != 0: order not verified (level model broken by rounding, cap_z or cap_g0 too small) -> fall back.
  * zkey_bits (0 = 32): the z keys are sorted as (layer, key(z) - key(z of the layer's lower plane)) truncated to that many
  * bits -- the caller bounds the span of one layer from the z map (fewer radix passes); a wrong bound only fails the
@@ -210,6 +195,10 @@ int t3d_mesh_canonicalize_structured_dev(const void* verts_in, const void* vkeys
                                          uint32_t cap_g0, const void* faces_in, int64_t F_cap, const void* F_dev_u64,
                                          void* verts_out, void* faces_out_i64, void* faces_out_i32, void* counts_u64,
                                          void* n_g0_u64, void* workspace, int phases, void* stream);
+
+/* calculate_mesh_volume / calculate_surface_area (surface_extractor.py:128-148): out_f64 = {signed volume, area}.  F_dev_u64:
+ * the true face count in device memory (at most F_cap); NULL = the capacity is the size. */
+int64_t t3d_mesh_measure_workspace_bytes(void);
 int t3d_mesh_measure_dev(const void* verts_f32, const void* faces, int64_t F_cap, const void* F_dev_u64, int faces_are_i64,
                          void* out_f64, void* workspace, void* stream);
 
@@ -241,7 +230,7 @@ int t3d_reconstruct(const void* masks_u8, int Z, int H, int W, int threshold, in
  * halo_lo + n_own + halo_hi bit-planes: the rank's own packed slices (global end slices already hole-filled) between the
  * planes received from its z-neighbours.  Gap fill and morphology are recomputed on the halo; the surface is marched on
  * min(3, halo) planes either side with z_begin/z_end (owned planes of the local padded sign volume, as t3d_mc_flags) and
- * z_offset (global plane index of local surface plane 0, as t3d_mc_vertices).  The result block is t3d_reconstruct's with
+ * z_offset (global plane index of local surface plane 0, as t3d_mc_vertices_dev).  The result block is t3d_reconstruct's with
  * Zx = halo_lo + n_own + halo_hi per-plane counts twice from slot 32 (bbox is over the own planes, local z), plus
  *   [18] ghost tail: canonical vertices with z == z_ghost (the next rank's first plane), if want_ghost
  *   [19] lead: canonical vertices with z == z_lead (this rank's first plane), if want_lead.
@@ -311,12 +300,9 @@ int t3d_sdf_z(const void* dy_i16, const void* dx_i16, int Z, int H, int W, const
 int64_t t3d_sdf_workspace_bytes(int Z, int H, int W);
 int t3d_sdf(const void* occ_bits, int Z, int H, int W, const double* sampling_host, void* sdf_f32, void* workspace, void* stream);
 
-/* Marching a dense float32 field directly (e.g. the SDF): sign bits = (field > level) packed like an occupancy volume,
- * then t3d_mc_flags/words/emit on them, and vertices interpolated on the field itself. */
+/* Marching a dense float32 field directly (e.g. the SDF): sign bits = (field > level) packed like an occupancy volume, then
+ * the marching-cubes entry points above on them with the field passed as field_f32 (mc_field, t3d_mc_vertices_dev). */
 int t3d_sign_from_f32(const void* field_f32, int Z, int H, int W, double level, void* sign_bits, void* stream);
-int t3d_mc_vertices_f32(const void* field_f32, int Z, int H, int W, double level, const void* vkeys_u64, uint32_t n_x, uint32_t n_y,
-                        uint32_t n_z, int unpad_shift, int z_offset, const void* cum_f64, const void* adj_f64, int n_cum,
-                        double mm_per_pixel_y, double mm_per_pixel_x, int scale_in_f64, void* verts_f32, void* stream);
 
 /* area-weighted unit vertex normals (the reference discards skimage's normals, surface_extractor.py:55 vs :72) */
 int t3d_vertex_normals(const void* verts_f32, int64_t V, const void* faces, int64_t F, int faces_are_i64, void* normals_f32,
@@ -325,20 +311,14 @@ int t3d_vertex_normals(const void* verts_f32, int64_t V, const void* faces, int6
 /* Field-gradient vertex normals (DESIGN.md §2): n = -(Gz/dz, Gy/mm_y, Gx/mm_x) / |.|, float32 (V', 3) [z, y, x], G = the
  * np.gradient of the marched field at the two end nodes of the vertex's grid edge blended with the vertex kernel's weight t,
  * dz = slope of the variable-depth z map at the vertex (1 without one).  Outward: from field > level to field < level.
- * Field source as t3d_mc_vertices (occ_bits, pad, gaussian; level 0.5) or, if field_f32 != NULL, that dense (Z,H,W) field at
- * `level` (t3d_mc_vertices_f32).  vkeys / block sizes / unpad_shift / z_offset / adj (n_cum = the z map's cum length, 0 = none)
- * as for the vertex kernel.  newid_u32 (NULL: raw order) scatters row i to its canonical slot; perm_u32 (NULL: no vertices
- * were merged) is the canonicalisation's sorted order and selects the tie rule: a slot that several raw vertices merged into
- * takes the normal of the one with the smallest edge key (z, y, x, axis).  dup_u64 (optional): the unique pass's "equal pair
- * seen" flag -- the tie pass returns at once while it reads 0.  winner_u32: scratch of V' entries (tie pass).  The map, the
- * order, the flag and a dead scratch range of each canonicalisation's workspace are found with t3d_canonical_map_offsets. */
-int t3d_mc_normals(const void* occ_bits, int Z, int H, int W, int pad, int gaussian, const double* weights3_host,
-                   const void* field_f32, double level, const void* vkeys_u64, uint32_t n_x, uint32_t n_y, uint32_t n_z,
-                   int unpad_shift, int z_offset, const void* adj_f64, int n_cum, double mm_per_pixel_y, double mm_per_pixel_x,
-                   const void* newid_u32, const void* perm_u32, const void* dup_u64, void* winner_u32, void* normals_f32,
-                   void* stream);
-/* the same with the block sizes in device memory (sizes_u64 = {n_active, n_x, n_y, n_z, ...}; nothing runs when the raw
- * vertex count exceeds cap_verts) */
+ * Field source as t3d_mc_vertices_dev (occ_bits, pad, gaussian; level 0.5) or, if field_f32 != NULL, that dense (Z,H,W) field
+ * at `level`.  vkeys / sizes_u64 / unpad_shift / z_offset / adj (n_cum = the z map's cum length, 0 = none) as for the vertex
+ * kernel; nothing runs when the raw vertex count n_x + n_y + n_z exceeds cap_verts.  newid_u32 (NULL: raw order) scatters row i
+ * to its canonical slot; perm_u32 (NULL: no vertices were merged) is the canonicalisation's sorted order and selects the tie
+ * rule: a slot that several raw vertices merged into takes the normal of the one with the smallest edge key (z, y, x, axis).
+ * dup_u64 (optional): the unique pass's "equal pair seen" flag -- the tie pass returns at once while it reads 0.  winner_u32:
+ * scratch of V' entries (tie pass).  The map, the order, the flag and a dead scratch range of each canonicalisation's
+ * workspace are found with t3d_canonical_map_offsets. */
 int t3d_mc_normals_dev(const void* occ_bits, int Z, int H, int W, int pad, int gaussian, const double* weights3_host,
                        const void* field_f32, double level, const void* vkeys_u64, const void* sizes_u64, uint32_t cap_verts,
                        int unpad_shift, int z_offset, const void* adj_f64, int n_cum, double mm_per_pixel_y, double mm_per_pixel_x,
@@ -346,7 +326,7 @@ int t3d_mc_normals_dev(const void* occ_bits, int Z, int H, int W, int pad, int g
                        void* stream);
 /* byte offsets in a canonicalisation's workspace, out4 = {newid (raw -> slot, u32), perm (sorted position -> raw id, u32),
  * a u32 scratch of >= V entries dead after the call, "equal pair seen" flag (u64; -1 = none)}; valid once the call finished.
- * kind 0: t3d_mesh_canonicalize (V, F); 1: t3d_mesh_canonicalize_fast[_dev] (V, F); 2: the structured variant with the same
+ * kind 0: t3d_mesh_canonicalize (V, F); 1: t3d_mesh_canonicalize_fast_dev (V, F); 2: the structured variant with the same
  * (V, F, cap_z, cap_g0, Zs) it was sized with. */
 int t3d_canonical_map_offsets(int kind, int64_t V, int64_t F, uint32_t cap_z, uint32_t cap_g0, int Zs, int64_t* out4);
 /* Post-step of t3d_reconstruct (same stream, same geometry, capacities and workspace, enqueued after it): field-gradient

@@ -39,27 +39,21 @@ SIGNATURES = {
     "t3d_row_popcounts": (_i, [_vp, _i, _i, _i, _vp, _vp]),
     "t3d_point_cloud_emit": (_i, [_vp, _i, _i, _i, _vp, _i, _vp, _dbl, _dbl, _vp, _vp]),
     "t3d_scan_workspace_bytes": (_i64, [_i64, _i]),
-    "t3d_exclusive_scan_u32": (_i, [_vp, _vp, _i64, _i, _i, _i, _vp, _vp, _vp]),
     "t3d_field_sign": (_i, [_vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp]),
     "t3d_field_sign_lean": (_i, [_vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _u32, _vp, _vp]),
     "t3d_mc_num_chunks": (_i64, [_i, _i, _i]),
     "t3d_mc_flags": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp]),
-    "t3d_mc_words": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _u32, _vp, _vp, _vp, _vp, _vp]),
-    "t3d_mc_emit": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _u32, _u32, _u32, _vp, _vp, _vp, _vp]),
-    "t3d_mc_vertices": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _u32, _u32, _u32, _i, _i, _vp, _vp, _i, _dbl, _dbl, _i,
-                             _vp, _vp]),
     "t3d_field_dense": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _vp]),
     "t3d_cube_cases": (_i, [_vp, _i, _i, _i, _vp, _vp]),
     "t3d_canonicalize_workspace_bytes": (_i64, [_i64, _i64]),
     "t3d_mesh_canonicalize": (_i, [_vp, _i64, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp]),
     "t3d_canonicalize_fast_workspace_bytes": (_i64, [_i64, _i64]),
-    "t3d_mesh_canonicalize_fast": (_i, [_vp, _i64, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp]),
     "t3d_mesh_measure_workspace_bytes": (_i64, []),
-    "t3d_mesh_measure": (_i, [_vp, _i64, _vp, _i64, _i, _vp, _vp, _vp]),
     "t3d_exclusive_scan_u32_dev": (_i, [_vp, _vp, _i64, _i64, _i, _i, _i, _vp, _vp, _vp, _vp]),
     "t3d_mc_words_dev": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _u32, _vp, _vp, _vp, _vp, _vp, _vp]),
     "t3d_mc_emit_dev": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _u32, _vp, _u32, _u32, _vp, _vp, _i, _vp, _vp]),
-    "t3d_mc_vertices_dev": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _u32, _i, _i, _vp, _vp, _i, _dbl, _dbl, _i, _i, _vp, _vp]),
+    "t3d_mc_vertices_dev": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _dbl, _vp, _vp, _u32, _i, _i, _vp, _vp, _i, _dbl, _dbl, _i, _i, _vp,
+                                 _vp]),
     "t3d_mesh_canonicalize_fast_dev": (_i, [_vp, _i64, _vp, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "t3d_mesh_measure_dev": (_i, [_vp, _vp, _i64, _vp, _i, _vp, _vp, _vp]),
     "t3d_canonicalize_structured_workspace_bytes": (_i64, [_i64, _i64, _u32, _u32, _i]),
@@ -89,7 +83,6 @@ SIGNATURES = {
     "t3d_sdf_workspace_bytes": (_i64, [_i, _i, _i]),
     "t3d_sdf": (_i, [_vp, _i, _i, _i, _vp, _vp, _vp, _vp]),
     "t3d_sign_from_f32": (_i, [_vp, _i, _i, _i, _dbl, _vp, _vp]),
-    "t3d_mc_vertices_f32": (_i, [_vp, _i, _i, _i, _dbl, _vp, _u32, _u32, _u32, _i, _i, _vp, _vp, _i, _dbl, _dbl, _i, _vp, _vp]),
     "t3d_layer_colors": (_i, [_vp, _i64, _i, _dbl, _dbl, _i, _dbl, _dbl, _vp, _vp]),
     "t3d_obj_workspace_bytes": (_i64, [_i64, _i64]),
     "t3d_glb_payload_bytes": (_i64, [_i64, _i64, _i]),
@@ -97,8 +90,6 @@ SIGNATURES = {
     "t3d_obj_measure": (_i, [_vp, _i64, _vp, _i64, _i, _vp, _vp, _vp]),
     "t3d_obj_emit": (_i, [_vp, _i64, _vp, _i64, _i, _vp, _vp, _vp, _vp]),
     "t3d_vertex_normals": (_i, [_vp, _i64, _vp, _i64, _i, _vp, _vp]),
-    "t3d_mc_normals": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _dbl, _vp, _u32, _u32, _u32, _i, _i, _vp, _i, _dbl, _dbl, _vp, _vp,
-                            _vp, _vp, _vp, _vp]),
     "t3d_mc_normals_dev": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _dbl, _vp, _vp, _u32, _i, _i, _vp, _i, _dbl, _dbl, _vp, _vp,
                                 _vp, _vp, _vp, _vp]),
     "t3d_canonical_map_offsets": (_i, [_i, _i64, _i64, _u32, _u32, _i, _vp]),

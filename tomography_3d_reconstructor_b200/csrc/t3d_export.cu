@@ -177,7 +177,7 @@ extern "C" int t3d_obj_measure(const void* verts_f32, int64_t V, const void* fac
     else k_obj_lengths<int32_t><<<g, 256, 0, st>>>((const float*)verts_f32, V, (const int32_t*)faces, F, len);
     T3D_CHECK_LAUNCH("t3d_obj_measure");
     t3d_count_launches(1);
-    return t3d_exclusive_scan_u32(len, offs, n, 1, 1, 0, total_len_u64, ws, stream);
+    return t3d_exclusive_scan_u32_dev(len, offs, n, n, 1, 1, 0, nullptr, total_len_u64, ws, stream);
 }
 
 // Phase 2: the body of the OBJ file (everything after the two comment lines and the blank line that follow them):

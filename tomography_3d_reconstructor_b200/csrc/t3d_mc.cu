@@ -7,12 +7,13 @@
 //   1. t3d_mc_flags    dense, one thread per 32-voxel word of the sign volume: does this word own a cut edge or the
 //                      origin of an active cube?  -> one ballot word per warp (1 bit per word).
 //   2. exclusive scan  of the ballot popcounts  -> rank of every active word (order-preserving compaction).
-//   3. t3d_mc_words    active words only: packed counts of owned x/y/z cut edges and triangles -> compact arrays.
-//   4. exclusive scan  of those counts -> vertex / triangle bases per active word.
-//   5. t3d_mc_emit     one thread per active word: edge keys of the owned vertices, faces of its cubes
-//                      (ids of vertices owned by neighbouring words through ballot-rank lookups).
-//   6. t3d_mc_vertices one thread per vertex: exact float64 field at the two end points, skimage's interpolation,
-//                      un-pad, variable-depth z map, mm scaling.
+//   3. t3d_mc_words_dev    active words only: packed counts of owned x/y/z cut edges and triangles -> compact arrays.
+//   4. exclusive scan      of those counts -> vertex / triangle bases per active word.
+//   5. t3d_mc_emit_dev     one thread per active word: edge keys of the owned vertices, faces of its cubes
+//                          (ids of vertices owned by neighbouring words through ballot-rank lookups).
+//   6. t3d_mc_vertices_dev one thread per vertex: exact float64 field at the two end points, skimage's interpolation,
+//                          un-pad, variable-depth z map, mm scaling.
+// Steps 3, 5 and 6 read the data-dependent sizes from a device block {n_active, n_x, n_y, n_z, n_t} (scan totals).
 // Vertex ids: [x-edge vertices | y-edge | z-edge], each in raster order of the owning voxel (edge owned by its lower
 // corner).  Faces come out in the reference's order: cubes z-major, y, x fastest, table order inside a cube,
 // winding reversed (gradient_direction='descent').
@@ -409,11 +410,10 @@ struct EmitArgs {
     const uint32_t* ballots;
     const uint32_t* chunkbase;
     const uint32_t* aw_idx;
-    const uint32_t* aw_base;  // 4 arrays, `n_active` (= capacity) elements apart: X, Y, Z, T (exclusive scans)
-    uint32_t n_active;        // number of active words, or the capacity of the arrays when `sizes` is given
-    uint32_t offY, offZ;      // offX = 0
-    const unsigned long long* sizes;  // optional device block {n_active, n_x, n_y, n_z, n_t}: overrides the three above
-    uint32_t cap_verts, cap_faces;    // with `sizes`: nothing is written beyond these
+    const uint32_t* aw_base;  // 4 arrays, `cap_active` elements apart: X, Y, Z, T (exclusive scans)
+    uint32_t cap_active;      // capacity of the word arrays
+    const unsigned long long* sizes;  // device block {n_active, n_x, n_y, n_z, n_t}
+    uint32_t cap_verts, cap_faces;    // nothing is written beyond these
     unsigned long long* vkeys;  // per vertex: axis | x << 2 | y << 22 | z << 42
     int32_t* faces;
 };
@@ -447,8 +447,8 @@ __global__ void __launch_bounds__(128) k_mc_emit(EmitArgs a)
     __shared__ uint32_t s_next[4][128];   // ids of the y/z-edge vertices at bit 0 of the next word (edges 1, 5, 9, 10 at b = 31)
     if (AMB == 1) {                       // nearly every CTA of this launch finds no flagged word in its share of the list:
         int any = 0;                      // leave before the table copy (the second look at the list comes from L2)
-        uint32_t nw_ = a.n_active;
-        if (a.sizes && a.sizes[0] < nw_) nw_ = (uint32_t)a.sizes[0];
+        uint32_t nw_ = a.cap_active;
+        if (a.sizes[0] < nw_) nw_ = (uint32_t)a.sizes[0];
         for (uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < nw_; k += gridDim.x * blockDim.x) any |= (int)(a.aw_idx[k] >> 31);
         if (!__syncthreads_or(any)) return;
     }
@@ -462,13 +462,10 @@ __global__ void __launch_bounds__(128) k_mc_emit(EmitArgs a)
         __syncthreads();
     }
     const uint32_t tid = threadIdx.x;
-    uint32_t n_words = a.n_active;
-    if (a.sizes) {
-        if (a.sizes[0] < n_words) n_words = (uint32_t)a.sizes[0];
-        a.offY = (uint32_t)a.sizes[1];
-        a.offZ = (uint32_t)(a.sizes[1] + a.sizes[2]);
-        if (a.sizes[1] + a.sizes[2] + a.sizes[3] > a.cap_verts || a.sizes[4] > a.cap_faces) return;  // overflow: flagged by the caller
-    }
+    uint32_t n_words = a.cap_active;
+    if (a.sizes[0] < n_words) n_words = (uint32_t)a.sizes[0];
+    const uint32_t offY = (uint32_t)a.sizes[1], offZ = (uint32_t)(a.sizes[1] + a.sizes[2]);  // offX = 0
+    if (a.sizes[1] + a.sizes[2] + a.sizes[3] > a.cap_verts || a.sizes[4] > a.cap_faces) return;  // overflow: flagged by the caller
     // one active word (the tables above are per thread: a thread may take several words in turn)
     auto emit_word = [&](const uint32_t k, const uint32_t iraw) {
     const uint32_t i = iraw & AW_MASK;
@@ -476,8 +473,8 @@ __global__ void __launch_bounds__(128) k_mc_emit(EmitArgs a)
     const int w = (int)(i - row * (uint32_t)a.g.nws);
     int z, y;
     const WordMasks m = load_masks(a.g, row, w, z, y);
-    const int64_t NA = a.n_active;
-    const uint32_t bX00 = a.aw_base[k], bY0 = a.offY + a.aw_base[NA + k], bZ0 = a.offZ + a.aw_base[2 * NA + k];
+    const int64_t NA = a.cap_active;
+    const uint32_t bX00 = a.aw_base[k], bY0 = offY + a.aw_base[NA + k], bZ0 = offZ + a.aw_base[2 * NA + k];
     uint32_t pT = a.aw_base[3 * NA + k];
     const int x0 = w << 5;
 
@@ -499,22 +496,22 @@ __global__ void __launch_bounds__(128) k_mc_emit(EmitArgs a)
     if (m.X01 | m.Z1) {
         const uint32_t r = active_rank(a, row + 1, w);
         bX01 = a.aw_base[r];
-        bZ1 = a.offZ + a.aw_base[2 * NA + r];
+        bZ1 = offZ + a.aw_base[2 * NA + r];
     }
     if (m.X10 | m.Y1) {
         const uint32_t r = active_rank(a, row + Hs, w);
         bX10 = a.aw_base[r];
-        bY1 = a.offY + a.aw_base[NA + r];
+        bY1 = offY + a.aw_base[NA + r];
     }
     if (m.X11) bX11 = a.aw_base[active_rank(a, row + Hs + 1, w)];
     // y/z edges at x0+32 (bit 0 of the next word) are only used by the cube at bit 31
     uint32_t nY0 = 0, nY1 = 0, nZ0 = 0, nZ1 = 0;
     if ((m.act >> 31) & 1u) {
         const uint32_t v1 = (m.a00 >> 31) & 1u, v2 = (m.a01 >> 31) & 1u, v5 = (m.a10 >> 31) & 1u, v6 = (m.a11 >> 31) & 1u;
-        if (v1 != v2) nY0 = a.offY + a.aw_base[NA + active_rank(a, row, w + 1)];            // edge 1
-        if (v5 != v6) nY1 = a.offY + a.aw_base[NA + active_rank(a, row + Hs, w + 1)];       // edge 5
-        if (v1 != v5) nZ0 = a.offZ + a.aw_base[2 * NA + active_rank(a, row, w + 1)];        // edge 9
-        if (v2 != v6) nZ1 = a.offZ + a.aw_base[2 * NA + active_rank(a, row + 1, w + 1)];    // edge 10
+        if (v1 != v2) nY0 = offY + a.aw_base[NA + active_rank(a, row, w + 1)];            // edge 1
+        if (v5 != v6) nY1 = offY + a.aw_base[NA + active_rank(a, row + Hs, w + 1)];       // edge 5
+        if (v1 != v5) nZ0 = offZ + a.aw_base[2 * NA + active_rank(a, row, w + 1)];        // edge 9
+        if (v2 != v6) nZ1 = offZ + a.aw_base[2 * NA + active_rank(a, row + 1, w + 1)];    // edge 10
     }
     // edge -> (base id of the owning word's block, cut mask of that block)
     s_base[0][tid] = bX00; s_mask[0][tid] = m.X00;
@@ -591,14 +588,13 @@ __global__ void __launch_bounds__(128) k_mc_emit(EmitArgs a)
 }
 
 // ------------------------------------------------------------------------------------------------
-// 6. vertices: one thread per vertex of one axis block
+// 6. vertices: one thread per vertex
 // ------------------------------------------------------------------------------------------------
 struct VertexArgs {
     OccView occ;
     const float* field;       // optional dense float32 field (Z,H,W): marched directly at `level` (SDF path)
     double level;             // iso level (0.5 for the Gaussian occupancy field)
     const unsigned long long* vkeys;
-    uint32_t first, count;    // id range of this axis block
     int x_off;                // the keys' x minus this = x in the (reference-)padded grid (padded-storage layout: 127)
     int z_offset;             // global padded plane of local padded plane 0 (z-slab sharding; 0 on a single device)
     float shift;              // 1 if manifold else 0 (surface_extractor.py:57-60)
@@ -654,18 +650,6 @@ __device__ __forceinline__ void vertex_body(const VertexArgs& p, const ZLut& zlu
     }
     float* o = p.verts + 3 * (int64_t)id;
     o[0] = fz; o[1] = fy; o[2] = fx;
-}
-
-
-template <int AXIS>
-__global__ void __launch_bounds__(128) k_mc_vertices(VertexArgs p)
-{
-    __shared__ ZLut zlut;
-    fill_zlut(p.occ, zlut);
-    __syncthreads();
-    const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= p.count) return;
-    vertex_body<AXIS>(p, zlut, p.first + t);
 }
 
 // axis blocks selected by `which` (1: x-edge, 2: y-edge, 4: z-edge vertices) in one launch, block sizes read from device
@@ -727,99 +711,9 @@ extern "C" int t3d_mc_flags(const void* sign_bits, int Zs, int Hs, int Ws, int z
     return 0;
 }
 
-// chunkbase_u32: exclusive scan of popcount(ballots); aw_idx_u32: n_active; aw_cnt_u32: 4 arrays of n_active
-extern "C" int t3d_mc_words(const void* sign_bits, int Zs, int Hs, int Ws, int z_begin, int z_end, const void* ballots_u32,
-                            const void* chunkbase_u32,
-                            uint32_t n_active, void* aw_idx_u32, void* aw_cnt_u32, void* n_ambiguous_u64, const t3d_mc_field* mc_field,
-                            void* stream)
-{
-    Grid g;
-    if (int rc = make_grid(g, sign_bits, Zs, Hs, Ws, z_begin, z_end, "t3d_mc_words")) return rc;
-    const McField fld = mc_field_from_abi(mc_field);
-    if (ensure_luts()) return 1;
-    cudaStream_t st = (cudaStream_t)stream;
-    if (t3d_zero_async(n_ambiguous_u64, 8, st)) return 1;
-    if (n_active == 0) return 0;
-    const int64_t n_chunks = (int64_t)g.n_rows * g.ncr;
-    k_mc_compact<<<(unsigned)((n_chunks + 255) / 256), 256, 0, st>>>(g, (const uint32_t*)ballots_u32,
-                                                                      (const uint32_t*)chunkbase_u32, n_chunks,
-                                                                      (uint32_t*)aw_idx_u32, n_active);
-    k_mc_words<0><<<(n_active + 127) / 128, 128, 0, st>>>(g, fld, (uint32_t*)aw_idx_u32, n_active, nullptr, (uint32_t*)aw_cnt_u32,
-                                                          (unsigned long long*)n_ambiguous_u64);
-    k_mc_words<1><<<amb_grid(n_active), 128, 0, st>>>(g, fld, (uint32_t*)aw_idx_u32, n_active, nullptr, (uint32_t*)aw_cnt_u32,
-                                                          (unsigned long long*)n_ambiguous_u64);
-    T3D_CHECK_LAUNCH("t3d_mc_words");
-    t3d_count_launches(3);
-    return 0;
-}
-
-// aw_base_u32: exclusive scans of aw_cnt; n_x / n_y: totals of the x- and y-edge counts.
-// vkeys_u64: one key per vertex (n_x + n_y + n_z); faces_i32: (n_t, 3).
-extern "C" int t3d_mc_emit(const void* sign_bits, int Zs, int Hs, int Ws, int z_begin, int z_end, const void* ballots_u32,
-                           const void* chunkbase_u32,
-                           const void* aw_idx_u32, const void* aw_base_u32, uint32_t n_active, uint32_t n_x, uint32_t n_y,
-                           void* vkeys_u64, void* faces_i32, const t3d_mc_field* mc_field, void* stream)
-{
-    EmitArgs a;
-    if (int rc = make_grid(a.g, sign_bits, Zs, Hs, Ws, z_begin, z_end, "t3d_mc_emit")) return rc;
-    a.fld = mc_field_from_abi(mc_field);
-    if (ensure_luts()) return 1;
-    if (n_active == 0) return 0;
-    a.ballots = (const uint32_t*)ballots_u32;
-    a.chunkbase = (const uint32_t*)chunkbase_u32;
-    a.aw_idx = (const uint32_t*)aw_idx_u32;
-    a.aw_base = (const uint32_t*)aw_base_u32;
-    a.n_active = n_active;
-    a.offY = n_x;
-    a.offZ = n_x + n_y;
-    a.vkeys = (unsigned long long*)vkeys_u64;
-    a.faces = (int32_t*)faces_i32;
-    a.sizes = nullptr;
-    a.cap_verts = a.cap_faces = 0xffffffffu;
-    k_mc_emit<3, 2><<<(n_active + 127) / 128, 128, 0, (cudaStream_t)stream>>>(a);
-    T3D_CHECK_LAUNCH("t3d_mc_emit");
-    t3d_count_launches(1);
-    return 0;
-}
-
-// vertices from their keys.  occ_*: the occupancy the sign volume was derived from (pad / gaussian as in
-// t3d_field_sign; gaussian = 0: the sign volume IS the occupancy and pad must be 0).
-// cum/adj: device float64 arrays of the variable-slice-depth z map (n_cum = 0 disables it).
-extern "C" int t3d_mc_vertices(const void* occ_bits, int Z, int H, int W, int pad, int gaussian, const double* weights3_host,
-                               const void* vkeys_u64, uint32_t n_x, uint32_t n_y, uint32_t n_z, int unpad_shift,
-                               int z_offset, const void* cum_f64, const void* adj_f64, int n_cum, double mm_per_pixel_y,
-                               double mm_per_pixel_x, int scale_in_f64, void* verts_f32, void* stream)
-{
-    if (Z <= 0 || H <= 0 || W <= 0) { t3d_set_error("t3d_mc_vertices: empty volume"); return 2; }
-    if (!gaussian && pad) { t3d_set_error("t3d_mc_vertices: pad requires gaussian"); return 2; }
-    cudaStream_t st = (cudaStream_t)stream;
-    VertexArgs p;
-    p.occ = t3d_make_view(occ_bits, Z, H, W, pad, gaussian, weights3_host);
-    p.vkeys = (const unsigned long long*)vkeys_u64;
-    p.field = nullptr;
-    p.level = 0.5;
-    p.x_off = 0;
-    p.shift = unpad_shift ? 1.0f : 0.0f;
-    p.z_offset = z_offset;
-    p.cum = (const double*)cum_f64;
-    p.adj = (const double*)adj_f64;
-    p.n_cum = n_cum;
-    p.mm_y = mm_per_pixel_y;
-    p.mm_x = mm_per_pixel_x;
-    p.scale_f64 = scale_in_f64 ? 1 : 0;
-    p.verts = (float*)verts_f32;
-    int launches = 0;
-    if (n_x) { p.first = 0; p.count = n_x; k_mc_vertices<2><<<(n_x + 127) / 128, 128, 0, st>>>(p); ++launches; }
-    if (n_y) { p.first = n_x; p.count = n_y; k_mc_vertices<1><<<(n_y + 127) / 128, 128, 0, st>>>(p); ++launches; }
-    if (n_z) { p.first = n_x + n_y; p.count = n_z; k_mc_vertices<0><<<(n_z + 127) / 128, 128, 0, st>>>(p); ++launches; }
-    T3D_CHECK_LAUNCH("t3d_mc_vertices");
-    t3d_count_launches(launches);
-    return 0;
-}
-
 // ------------------------------------------------------------------------------------------------
-// device-size variants: every data-dependent size stays in device memory (sizes_u64 = {n_active, n_x, n_y, n_z, n_t}),
-// arrays are capacity-sized, nothing is written beyond the capacities.  No host round trip => graph-capturable.
+// Every data-dependent size stays in device memory (sizes_u64 = {n_active, n_x, n_y, n_z, n_t}), arrays are capacity-sized
+// and nothing is written beyond the capacities.  No host round trip => graph-capturable.
 // ------------------------------------------------------------------------------------------------
 static int mc_words_dev_impl(const McField& fld, const void* sign_bits, int Zs, int Hs, int Ws, int z_begin, int z_end,
                              const void* ballots_u32, const void* chunkbase_u32, uint32_t cap_active, const void* sizes_u64,
@@ -865,8 +759,7 @@ static int mc_emit_dev_impl(const McField& fld, const void* sign_bits, int Zs, i
     a.chunkbase = (const uint32_t*)chunkbase_u32;
     a.aw_idx = (const uint32_t*)aw_idx_u32;
     a.aw_base = (const uint32_t*)aw_base_u32;
-    a.n_active = cap_active;
-    a.offY = a.offZ = 0;
+    a.cap_active = cap_active;
     a.sizes = (const unsigned long long*)sizes_u64;
     a.cap_verts = cap_verts;
     a.cap_faces = cap_faces;
@@ -877,7 +770,7 @@ static int mc_emit_dev_impl(const McField& fld, const void* sign_bits, int Zs, i
     if ((parts & 3) == 1) k_mc_emit<1, 0><<<ge, 128, 0, (cudaStream_t)stream>>>(a);
     else if ((parts & 3) == 2) {        // the common words, then the (rare) words holding ambiguous cubes
         k_mc_emit<2, 0><<<ge, 128, 0, (cudaStream_t)stream>>>(a);
-        k_mc_emit<2, 1><<<amb_grid(a.n_active), 128, 0, (cudaStream_t)stream>>>(a);
+        k_mc_emit<2, 1><<<amb_grid(cap_active), 128, 0, (cudaStream_t)stream>>>(a);
         launches = 2;
     } else k_mc_emit<3, 2><<<ge, 128, 0, (cudaStream_t)stream>>>(a);
     T3D_CHECK_LAUNCH("t3d_mc_emit_dev");
@@ -916,20 +809,20 @@ int t3d_mc_emit_view_dev(const OccView& view, int x_off, const void* sign_bits, 
                             sizes_u64, cap_verts, cap_faces, vkeys_u64, faces_i32, parts, stream);
 }
 
-// vertices of a mesh emitted on a sign volume whose x coordinates are shifted by x_off against `view`'s padded grid
-int t3d_mc_vertices_view_dev(const OccView& view, int x_off, const void* vkeys_u64, const void* sizes_u64, uint32_t cap_verts,
-                             int unpad_shift, int z_offset, const void* cum_f64, const void* adj_f64, int n_cum, double mm_per_pixel_y,
-                             double mm_per_pixel_x, int scale_in_f64, int which_blocks, void* verts_f32, void* stream)
+// vertices of a mesh emitted on a sign volume whose x coordinates are shifted by x_off against `view`'s padded grid; with
+// `field`, the dense float32 field of the view's extents is interpolated at `level` instead
+static int mc_vertices_impl(const OccView& view, const float* field, double level, int x_off, const void* vkeys_u64, const void* sizes_u64,
+                            uint32_t cap_verts, int unpad_shift, int z_offset, const void* cum_f64, const void* adj_f64, int n_cum,
+                            double mm_per_pixel_y, double mm_per_pixel_x, int scale_in_f64, int which_blocks, void* verts_f32, void* stream)
 {
     if ((which_blocks & 7) == 0) return 0;
     if (cap_verts == 0) return 0;
     VertexArgs p;
     p.occ = view;
     p.vkeys = (const unsigned long long*)vkeys_u64;
-    p.field = nullptr;
-    p.level = 0.5;
+    p.field = field;
+    p.level = level;
     p.x_off = x_off;
-    p.first = 0; p.count = cap_verts;
     p.shift = unpad_shift ? 1.0f : 0.0f;
     p.z_offset = z_offset;
     p.cum = (const double*)cum_f64;
@@ -946,19 +839,34 @@ int t3d_mc_vertices_view_dev(const OccView& view, int x_off, const void* vkeys_u
     return 0;
 }
 
+int t3d_mc_vertices_view_dev(const OccView& view, int x_off, const void* vkeys_u64, const void* sizes_u64, uint32_t cap_verts,
+                             int unpad_shift, int z_offset, const void* cum_f64, const void* adj_f64, int n_cum, double mm_per_pixel_y,
+                             double mm_per_pixel_x, int scale_in_f64, int which_blocks, void* verts_f32, void* stream)
+{
+    return mc_vertices_impl(view, nullptr, 0.5, x_off, vkeys_u64, sizes_u64, cap_verts, unpad_shift, z_offset, cum_f64, adj_f64, n_cum,
+                            mm_per_pixel_y, mm_per_pixel_x, scale_in_f64, which_blocks, verts_f32, stream);
+}
+
+// occ_*: the occupancy the sign volume was derived from (pad / gaussian as in t3d_field_sign; gaussian = 0: the sign volume IS
+// the occupancy and pad must be 0), or field_f32: the dense field the sign volume was taken from (t3d_sign_from_f32).
 extern "C" int t3d_mc_vertices_dev(const void* occ_bits, int Z, int H, int W, int pad, int gaussian, const double* weights3_host,
-                                   const void* vkeys_u64, const void* sizes_u64, uint32_t cap_verts, int unpad_shift, int z_offset,
-                                   const void* cum_f64, const void* adj_f64, int n_cum, double mm_per_pixel_y,
-                                   double mm_per_pixel_x, int scale_in_f64, int which_blocks, void* verts_f32, void* stream)
+                                   const void* field_f32, double level, const void* vkeys_u64, const void* sizes_u64, uint32_t cap_verts,
+                                   int unpad_shift, int z_offset, const void* cum_f64, const void* adj_f64, int n_cum,
+                                   double mm_per_pixel_y, double mm_per_pixel_x, int scale_in_f64, int which_blocks, void* verts_f32,
+                                   void* stream)
 {
     if (Z <= 0 || H <= 0 || W <= 0) { t3d_set_error("t3d_mc_vertices_dev: empty volume"); return 2; }
-    return t3d_mc_vertices_view_dev(t3d_make_view(occ_bits, Z, H, W, pad, gaussian, weights3_host), 0, vkeys_u64, sizes_u64, cap_verts,
-                                    unpad_shift, z_offset, cum_f64, adj_f64, n_cum, mm_per_pixel_y, mm_per_pixel_x, scale_in_f64,
-                                    which_blocks, verts_f32, stream);
+    if (!field_f32 && !gaussian && pad) { t3d_set_error("t3d_mc_vertices_dev: pad requires gaussian"); return 2; }
+    const OccView view = field_f32 ? t3d_make_view(nullptr, Z, H, W, 0, 0, nullptr)
+                                   : t3d_make_view(occ_bits, Z, H, W, pad, gaussian, weights3_host);
+    return mc_vertices_impl(view, (const float*)field_f32, field_f32 ? level : 0.5, 0, vkeys_u64, sizes_u64, cap_verts, unpad_shift,
+                            z_offset, cum_f64, adj_f64, n_cum, mm_per_pixel_y, mm_per_pixel_x, scale_in_f64, which_blocks, verts_f32,
+                            stream);
 }
 
 // ------------------------------------------------------------------------------------------------
-// marching a dense float32 field (additive SDF path, SURVEY.md 8a-16 / 8b): sign bits and vertices straight from it
+// marching a dense float32 field (additive SDF path, SURVEY.md 8a-16 / 8b): sign bits straight from it (the vertices come from
+// t3d_mc_vertices_dev with field_f32)
 // ------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) k_sign_from_f32(const float* __restrict__ field, int64_t n_rows, int W, int nw, double level,
                                                        uint32_t* __restrict__ bits)
@@ -984,37 +892,5 @@ extern "C" int t3d_sign_from_f32(const void* field_f32, int Z, int H, int W, dou
                                                                                  (uint32_t*)sign_bits);
     T3D_CHECK_LAUNCH("t3d_sign_from_f32");
     t3d_count_launches(1);
-    return 0;
-}
-
-// vertices of a mesh marched on the float field itself (no padding, no Gaussian): skimage's interpolation at `level`
-extern "C" int t3d_mc_vertices_f32(const void* field_f32, int Z, int H, int W, double level, const void* vkeys_u64, uint32_t n_x,
-                                   uint32_t n_y, uint32_t n_z, int unpad_shift, int z_offset, const void* cum_f64,
-                                   const void* adj_f64, int n_cum, double mm_per_pixel_y, double mm_per_pixel_x, int scale_in_f64,
-                                   void* verts_f32, void* stream)
-{
-    if (Z <= 0 || H <= 0 || W <= 0) { t3d_set_error("t3d_mc_vertices_f32: empty volume"); return 2; }
-    cudaStream_t st = (cudaStream_t)stream;
-    VertexArgs p;
-    p.occ = t3d_make_view(nullptr, Z, H, W, 0, 0, nullptr);
-    p.field = (const float*)field_f32;
-    p.level = level;
-    p.x_off = 0;
-    p.vkeys = (const unsigned long long*)vkeys_u64;
-    p.shift = unpad_shift ? 1.0f : 0.0f;
-    p.z_offset = z_offset;
-    p.cum = (const double*)cum_f64;
-    p.adj = (const double*)adj_f64;
-    p.n_cum = n_cum;
-    p.mm_y = mm_per_pixel_y;
-    p.mm_x = mm_per_pixel_x;
-    p.scale_f64 = scale_in_f64 ? 1 : 0;
-    p.verts = (float*)verts_f32;
-    int launches = 0;
-    if (n_x) { p.first = 0; p.count = n_x; k_mc_vertices<2><<<(n_x + 127) / 128, 128, 0, st>>>(p); ++launches; }
-    if (n_y) { p.first = n_x; p.count = n_y; k_mc_vertices<1><<<(n_y + 127) / 128, 128, 0, st>>>(p); ++launches; }
-    if (n_z) { p.first = n_x + n_y; p.count = n_z; k_mc_vertices<0><<<(n_z + 127) / 128, 128, 0, st>>>(p); ++launches; }
-    T3D_CHECK_LAUNCH("t3d_mc_vertices_f32");
-    t3d_count_launches(launches);
     return 0;
 }

@@ -24,9 +24,8 @@ struct NormalArgs {
     const float* field;        // or: dense float32 field of extents occ.Z x occ.H x occ.W (occ without bits, pad 0)
     double level;
     const unsigned long long* vkeys;
-    const unsigned long long* sizes;   // device {n_active, n_x, n_y, n_z, ...}; null: the host sizes below
-    uint32_t nx, ny, nz;
-    uint32_t cap_verts;        // with `sizes`: nothing runs when n_x + n_y + n_z exceeds it
+    const unsigned long long* sizes;   // device {n_active, n_x, n_y, n_z, ...}
+    uint32_t cap_verts;        // nothing runs when n_x + n_y + n_z exceeds it
     int x_off;                 // key x minus this = x in the padded grid
     int z_offset;
     float shift;               // 1 if the vertices are un-padded
@@ -42,7 +41,6 @@ struct NormalArgs {
 
 __device__ __forceinline__ uint32_t raw_count(const NormalArgs& p)
 {
-    if (!p.sizes) return p.nx + p.ny + p.nz;
     const unsigned long long v = p.sizes[1] + p.sizes[2] + p.sizes[3];
     return v > p.cap_verts ? 0u : (uint32_t)v;
 }
@@ -232,7 +230,7 @@ __global__ void __launch_bounds__(128) k_mc_normals(NormalArgs p)
     __shared__ ZLut zlut;
     fill_zlut(p.occ, zlut);
     __syncthreads();
-    const uint32_t nx = p.sizes ? (uint32_t)p.sizes[1] : p.nx, ny = p.sizes ? (uint32_t)p.sizes[2] : p.ny;
+    const uint32_t nx = (uint32_t)p.sizes[1], ny = (uint32_t)p.sizes[2];
     const uint32_t n = raw_count(p);
     const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= n) return;
@@ -262,8 +260,9 @@ __global__ void __launch_bounds__(256) k_mc_normal_ties(NormalArgs p)
     p.winner[slot] = best;
 }
 
-static int launch_normals(NormalArgs& p, uint32_t grid_verts, cudaStream_t st, const char* who)
+static int launch_normals(NormalArgs& p, cudaStream_t st, const char* who)
 {
+    const uint32_t grid_verts = p.cap_verts;
     if (grid_verts == 0) return 0;
     int launches = 1;
     if (p.perm) {
@@ -278,9 +277,9 @@ static int launch_normals(NormalArgs& p, uint32_t grid_verts, cudaStream_t st, c
 }
 
 static int make_args(NormalArgs& p, const void* occ_bits, int Z, int H, int W, int pad, int gaussian, const double* weights3_host,
-                     const void* field_f32, double level, const void* vkeys_u64, int unpad_shift, int z_offset, const void* adj_f64,
-                     int n_cum, double mm_y, double mm_x, const void* newid_u32, const void* perm_u32, const void* dup_u64,
-                     void* winner_u32, void* normals_f32, const char* who)
+                     const void* field_f32, double level, const void* vkeys_u64, const void* sizes_u64, uint32_t cap_verts,
+                     int unpad_shift, int z_offset, const void* adj_f64, int n_cum, double mm_y, double mm_x, const void* newid_u32,
+                     const void* perm_u32, const void* dup_u64, void* winner_u32, void* normals_f32, const char* who)
 {
     if (Z <= 0 || H <= 0 || W <= 0) { t3d_set_error("%s: empty volume", who); return 2; }
     if (field_f32) {
@@ -293,7 +292,8 @@ static int make_args(NormalArgs& p, const void* occ_bits, int Z, int H, int W, i
     p.field = (const float*)field_f32;
     p.level = field_f32 ? level : 0.5;
     p.vkeys = (const unsigned long long*)vkeys_u64;
-    p.sizes = nullptr; p.nx = p.ny = p.nz = 0; p.cap_verts = 0;
+    p.sizes = (const unsigned long long*)sizes_u64;
+    p.cap_verts = cap_verts;
     p.x_off = 0;
     p.z_offset = z_offset;
     p.shift = unpad_shift ? 1.0f : 0.0f;
@@ -308,20 +308,6 @@ static int make_args(NormalArgs& p, const void* occ_bits, int Z, int H, int W, i
     return 0;
 }
 
-extern "C" int t3d_mc_normals(const void* occ_bits, int Z, int H, int W, int pad, int gaussian, const double* weights3_host,
-                              const void* field_f32, double level, const void* vkeys_u64, uint32_t n_x, uint32_t n_y, uint32_t n_z,
-                              int unpad_shift, int z_offset, const void* adj_f64, int n_cum, double mm_per_pixel_y, double mm_per_pixel_x,
-                              const void* newid_u32, const void* perm_u32, const void* dup_u64, void* winner_u32, void* normals_f32,
-                              void* stream)
-{
-    NormalArgs p;
-    if (int rc = make_args(p, occ_bits, Z, H, W, pad, gaussian, weights3_host, field_f32, level, vkeys_u64, unpad_shift, z_offset, adj_f64,
-                           n_cum, mm_per_pixel_y, mm_per_pixel_x, newid_u32, perm_u32, dup_u64, winner_u32, normals_f32, "t3d_mc_normals"))
-        return rc;
-    p.nx = n_x; p.ny = n_y; p.nz = n_z;
-    return launch_normals(p, n_x + n_y + n_z, (cudaStream_t)stream, "t3d_mc_normals");
-}
-
 extern "C" int t3d_mc_normals_dev(const void* occ_bits, int Z, int H, int W, int pad, int gaussian, const double* weights3_host,
                                   const void* field_f32, double level, const void* vkeys_u64, const void* sizes_u64, uint32_t cap_verts,
                                   int unpad_shift, int z_offset, const void* adj_f64, int n_cum, double mm_per_pixel_y,
@@ -329,13 +315,11 @@ extern "C" int t3d_mc_normals_dev(const void* occ_bits, int Z, int H, int W, int
                                   void* winner_u32, void* normals_f32, void* stream)
 {
     NormalArgs p;
-    if (int rc = make_args(p, occ_bits, Z, H, W, pad, gaussian, weights3_host, field_f32, level, vkeys_u64, unpad_shift, z_offset, adj_f64,
-                           n_cum, mm_per_pixel_y, mm_per_pixel_x, newid_u32, perm_u32, dup_u64, winner_u32, normals_f32,
-                           "t3d_mc_normals_dev"))
+    if (int rc = make_args(p, occ_bits, Z, H, W, pad, gaussian, weights3_host, field_f32, level, vkeys_u64, sizes_u64, cap_verts,
+                           unpad_shift, z_offset, adj_f64, n_cum, mm_per_pixel_y, mm_per_pixel_x, newid_u32, perm_u32, dup_u64,
+                           winner_u32, normals_f32, "t3d_mc_normals_dev"))
         return rc;
-    p.sizes = (const unsigned long long*)sizes_u64;
-    p.cap_verts = cap_verts;
-    return launch_normals(p, cap_verts, (cudaStream_t)stream, "t3d_mc_normals_dev");
+    return launch_normals(p, (cudaStream_t)stream, "t3d_mc_normals_dev");
 }
 
 // the fused step's variant: the field is a strided view whose padded x is the key's x minus x_off (t3d_pipeline.cu)
@@ -345,13 +329,11 @@ int t3d_mc_normals_view_dev(const OccView& view, int x_off, const void* vkeys_u6
                             void* stream)
 {
     NormalArgs p;
-    if (int rc = make_args(p, view.bits, view.Z, view.H, view.W, view.pad, view.gaussian, nullptr, nullptr, 0.5, vkeys_u64, unpad_shift,
-                           z_offset, adj_f64, n_cum, mm_per_pixel_y, mm_per_pixel_x, newid_u32, perm_u32, dup_u64, winner_u32,
-                           normals_f32, "t3d_reconstruct_normals"))
+    if (int rc = make_args(p, view.bits, view.Z, view.H, view.W, view.pad, view.gaussian, nullptr, nullptr, 0.5, vkeys_u64, sizes_u64,
+                           cap_verts, unpad_shift, z_offset, adj_f64, n_cum, mm_per_pixel_y, mm_per_pixel_x, newid_u32, perm_u32, dup_u64,
+                           winner_u32, normals_f32, "t3d_reconstruct_normals"))
         return rc;
     p.occ = view;
     p.x_off = x_off;
-    p.sizes = (const unsigned long long*)sizes_u64;
-    p.cap_verts = cap_verts;
-    return launch_normals(p, cap_verts, (cudaStream_t)stream, "t3d_reconstruct_normals");
+    return launch_normals(p, (cudaStream_t)stream, "t3d_reconstruct_normals");
 }

@@ -389,7 +389,8 @@ static int reconstruct_core(const uint32_t* grid, const SlabGeom& g, int H, int 
     NvtxRange r_mc("t3d:extract_manifold_surface");
     RUN(t3d_mc_flags(ws + L.sign, Zp, Hp, Wp, g.z_begin, g.z_end, ws + L.ballots, st));
     marks.mark("flags", st);
-    RUN(t3d_exclusive_scan_u32(ws + L.ballots, ws + L.chunkbase, n_chunks, 1, 0, 1, R + R_NACTIVE, ws + L.scan1, st));
+    RUN(t3d_exclusive_scan_u32_dev(ws + L.ballots, ws + L.chunkbase, n_chunks, n_chunks, 1, 0, 1, nullptr, R + R_NACTIVE,
+                                   ws + L.scan1, st));
     RUN(t3d_mc_words_view_dev(view, x_off, ws + L.sign, Zp, Hp, Wp, g.z_begin, g.z_end, ws + L.ballots, ws + L.chunkbase, cap_active,
                               R + R_NACTIVE, ws + L.aw_idx, ws + L.aw_cnt, R + R_NAMBIGUOUS, st));
     RUN(t3d_exclusive_scan_u32_dev(ws + L.aw_cnt, ws + L.aw_base, cap_active, cap_active, 4, 0, 0, R + R_NACTIVE, R + R_NX,

@@ -249,10 +249,9 @@ extern "C" int64_t t3d_scan_workspace_bytes(int64_t n, int n_arrays)
     return (nb * n_arrays + 16) * 8 + 256;
 }
 
-// in: n_arrays arrays of n uint32 (array k starts at in + k*n); out: same layout, uint32 (out_is_u64 = 0)
-// or uint64 (1); may alias `in` only for uint32 output.  popcount_input = 1 scans popcount(in[i]) instead of in[i].
-// totals: n_arrays uint64 (device).
-// general form: arrays `stride` elements apart, at most n_cap elements each, true length optionally in device memory
+// in: n_arrays arrays of n_cap uint32, `stride` elements apart; out: same layout, uint32 (out_is_u64 = 0) or uint64 (1); may
+// alias `in` only for uint32 output.  popcount_input = 1 scans popcount(in[i]) instead of in[i].  n_dev_u64 (optional, device):
+// the true length when n_cap is only a capacity.  totals: n_arrays uint64 (device).
 extern "C" int t3d_exclusive_scan_u32_dev(const void* in, void* out, int64_t n_cap, int64_t stride, int n_arrays, int out_is_u64,
                                           int popcount_input, const void* n_dev_u64, void* totals_u64, void* workspace, void* stream)
 {
@@ -261,9 +260,9 @@ extern "C" int t3d_exclusive_scan_u32_dev(const void* in, void* out, int64_t n_c
         if (n_arrays > 0) T3D_CUDA(cudaMemsetAsync(totals_u64, 0, 8 * n_arrays, st));
         return 0;
     }
-    if (n_arrays > 16) { t3d_set_error("t3d_exclusive_scan_u32: at most 16 arrays per call"); return 2; }
+    if (n_arrays > 16) { t3d_set_error("t3d_exclusive_scan_u32_dev: at most 16 arrays per call"); return 2; }
     const int64_t nb = (n_cap + SC_TILE - 1) / SC_TILE;
-    if (nb > 0x7fffffff) { t3d_set_error("t3d_exclusive_scan_u32: too many elements"); return 2; }
+    if (nb > 0x7fffffff) { t3d_set_error("t3d_exclusive_scan_u32_dev: too many elements"); return 2; }
     // workspace: [tile descriptors: nb * n_arrays u64][tickets: 16 u32], zeroed for every scan
     const size_t desc_bytes = (size_t)nb * n_arrays * 8;
     if (t3d_zero_async(workspace, desc_bytes + 64, st)) return 1;
@@ -278,15 +277,9 @@ extern "C" int t3d_exclusive_scan_u32_dev(const void* in, void* out, int64_t n_c
     else
         k_scan_lookback<uint32_t><<<grid, SC_THREADS, 0, st>>>((const uint32_t*)in, (uint32_t*)out, n_cap, stride, desc, (int)nb, tickets,
                                                                popcount_input, nd, (unsigned long long*)totals_u64);
-    T3D_CHECK_LAUNCH("t3d_exclusive_scan_u32");
+    T3D_CHECK_LAUNCH("t3d_exclusive_scan_u32_dev");
     t3d_count_launches(1);
     return 0;
-}
-
-extern "C" int t3d_exclusive_scan_u32(const void* in, void* out, int64_t n, int n_arrays, int out_is_u64, int popcount_input,
-                                      void* totals_u64, void* workspace, void* stream)
-{
-    return t3d_exclusive_scan_u32_dev(in, out, n, n, n_arrays, out_is_u64, popcount_input, nullptr, totals_u64, workspace, stream);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -556,13 +549,13 @@ extern "C" int t3d_mesh_canonicalize(const void* verts_in, int64_t V, const void
     }
     const uint32_t* perm = pin;
     k_unique_heads<<<gv, 256, 0, st>>>(vin, perm, V, flags);
-    if (t3d_exclusive_scan_u32(flags, pos, V, 1, 0, 0, totals, scan_ws, stream)) return 1;
+    if (t3d_exclusive_scan_u32_dev(flags, pos, V, V, 1, 0, 0, nullptr, totals, scan_ws, stream)) return 1;
     T3D_CUDA(cudaMemcpyAsync(counts, totals, 8, cudaMemcpyDeviceToDevice, st));
     k_scatter_unique<<<gv, 256, 0, st>>>(vin, perm, flags, pos, V, (float*)verts_out, newid);
     if (F > 0) {
         const unsigned gf = (unsigned)((F + 255) / 256);
         k_face_valid<<<gf, 256, 0, st>>>((const int32_t*)faces_in, F, newid, flags);
-        if (t3d_exclusive_scan_u32(flags, pos, F, 1, 0, 0, totals, scan_ws, stream)) return 1;
+        if (t3d_exclusive_scan_u32_dev(flags, pos, F, F, 1, 0, 0, nullptr, totals, scan_ws, stream)) return 1;
         T3D_CUDA(cudaMemcpyAsync(counts + 1, totals, 8, cudaMemcpyDeviceToDevice, st));
         k_face_compact<<<gf, 256, 0, st>>>((const int32_t*)faces_in, F, newid, flags, pos, (long long*)faces_out_i64,
                                            (int32_t*)faces_out_i32);
@@ -575,7 +568,7 @@ extern "C" int t3d_mesh_canonicalize(const void* verts_in, int64_t V, const void
 }
 
 // ------------------------------------------------------------------------------------------------
-// fast canonical mesh for meshes emitted by t3d_mc_emit.  The raw vertex order is [x-edge | y-edge | z-edge] blocks,
+// fast canonical mesh for meshes emitted by t3d_mc_emit_dev.  The raw vertex order is [x-edge | y-edge | z-edge] blocks,
 // each in raster order of the owning voxel, so among vertices with equal (z, y) float keys the x keys are already
 // ascending (equal (z,y) keys across blocks would need a vertex coordinate to round onto a grid plane).  One STABLE
 // radix sort on the 64-bit key (z key << 32 | y key) therefore yields np.unique's lexicographic order.  The result is
@@ -844,13 +837,15 @@ static int canonical_tail(const float* vin, const uint32_t* perm, int64_t V, con
 }
 
 // same outputs as t3d_mesh_canonicalize; counts_u64[0] = V', [1] = F', [2] = 0 if the fast ordering was verified.
-// V_dev / F_dev (optional, device uint64): true sizes when V / F are only capacities.
-static int canonicalize_fast_impl(const void* verts_in, int64_t V, const unsigned long long* V_dev, const void* faces_in, int64_t F,
-                                  const unsigned long long* F_dev, void* verts_out, void* faces_out_i64, void* faces_out_i32,
-                                  void* counts_u64, void* workspace, void* stream)
+// V_dev_u64 / F_dev_u64 (optional, device uint64): true sizes when V / F are only capacities.
+extern "C" int t3d_mesh_canonicalize_fast_dev(const void* verts_in, int64_t V, const void* V_dev_u64, const void* faces_in, int64_t F,
+                                              const void* F_dev_u64, void* verts_out, void* faces_out_i64, void* faces_out_i32,
+                                              void* counts_u64, void* workspace, void* stream)
 {
     cudaStream_t st = (cudaStream_t)stream;
-    if (V <= 0 || V > 0x7fffffff || F < 0) { t3d_set_error("t3d_mesh_canonicalize_fast: bad sizes"); return 2; }
+    if (V <= 0 || V > 0x7fffffff || F < 0) { t3d_set_error("t3d_mesh_canonicalize_fast_dev: bad sizes"); return 2; }
+    const unsigned long long* V_dev = (const unsigned long long*)V_dev_u64;
+    const unsigned long long* F_dev = (const unsigned long long*)F_dev_u64;
     const int64_t n = V > F ? V : F;
     char* ws = (char*)workspace;
     unsigned long long* keys_a = (unsigned long long*)ws; ws += align256(8 * V);
@@ -873,31 +868,13 @@ static int canonicalize_fast_impl(const void* verts_in, int64_t V, const unsigne
                                              (int)V, 0, 64, st));
     if (canonical_tail(vin, perm, V, V_dev, faces_in, F, F_dev, verts_out, faces_out_i64, faces_out_i32, counts, flags, pos, newid,
                        scan_ws, scan_ws, totals, st)) return 1;
-    T3D_CHECK_LAUNCH("t3d_mesh_canonicalize_fast");
+    T3D_CHECK_LAUNCH("t3d_mesh_canonicalize_fast_dev");
     t3d_count_launches(F > 0 ? 5 : 3);
     return 0;
 }
 
-extern "C" int t3d_mesh_canonicalize_fast(const void* verts_in, int64_t V, const void* faces_in, int64_t F, void* verts_out,
-                                          void* faces_out_i64, void* faces_out_i32, void* counts_u64, void* workspace,
-                                          void* stream)
-{
-    return canonicalize_fast_impl(verts_in, V, nullptr, faces_in, F, nullptr, verts_out, faces_out_i64, faces_out_i32, counts_u64,
-                                  workspace, stream);
-}
-
-// capacity-sized inputs, true sizes in device memory (graph-capturable)
-extern "C" int t3d_mesh_canonicalize_fast_dev(const void* verts_in, int64_t V_cap, const void* V_dev_u64, const void* faces_in,
-                                              int64_t F_cap, const void* F_dev_u64, void* verts_out, void* faces_out_i64,
-                                              void* faces_out_i32, void* counts_u64, void* workspace, void* stream)
-{
-    return canonicalize_fast_impl(verts_in, V_cap, (const unsigned long long*)V_dev_u64, faces_in, F_cap,
-                                  (const unsigned long long*)F_dev_u64, verts_out, faces_out_i64, faces_out_i32, counts_u64, workspace,
-                                  stream);
-}
-
 // ------------------------------------------------------------------------------------------------
-// structured canonical order for meshes emitted by t3d_mc_emit (vertex keys available).
+// structured canonical order for meshes emitted by t3d_mc_emit_dev (vertex keys available).
 //
 // Raw order = [x-edge | y-edge | z-edge] blocks, each in raster order of the owning grid point (zc, yc, xc).  A vertex
 // has one fractional coordinate; give every coordinate a level (2c on a grid line, 2c+1 strictly inside cell c).
@@ -925,7 +902,7 @@ struct CanonS {
     const uint32_t* aw_base;           // 4 arrays (x, y, z vertices, triangles before each active word), `stride` apart
     uint32_t stride;
     int g_plane;                       // local plane index of un-padded plane 0 (= shift - z_offset); < 0: no clamp group here
-    int z_offset; float shift;         // as in t3d_mc_vertices: global plane of local plane 0, un-pad shift
+    int z_offset; float shift;         // as in t3d_mc_vertices_dev: global plane of local plane 0, un-pad shift
     const double* cum; const double* adj; int n_cum;
     int zkey_bits;                     // 32: absolute z keys; less: key relative to the layer's lower plane, that many bits
     unsigned long long* zkeys;
@@ -1260,7 +1237,7 @@ void t3d_canonicalize_structured_zero_range(int64_t V, int64_t F, uint32_t cap_z
 
 // verts_in / vkeys: capacity V_cap, true block sizes in sizes_u64 = {n_active, n_x, n_y, n_z, n_t} (device); V_dev_u64 = n_x+n_y+n_z
 // and F_dev_u64 = n_t (device).  Zs: planes of the marched (local) sign volume; z_offset / unpad_shift / n_cum as passed to
-// t3d_mc_vertices.  counts_u64: [0] V' [1] F' [2] != 0: order not verified, fall back; n_g0_u64 (optional): size of the
+// t3d_mc_vertices_dev.  counts_u64: [0] V' [1] F' [2] != 0: order not verified, fall back; n_g0_u64 (optional): size of the
 // clamp group (a caller seeing [2] != 0 with *n_g0 > cap_g0 retries with a larger cap_g0).
 extern "C" int t3d_mesh_canonicalize_structured_dev(const void* verts_in, const void* vkeys_u64, int64_t V_cap, const void* sizes_u64,
                                                     const void* V_dev_u64, int Zs, int Hs, int Ws, const void* chunkbase_u32,
@@ -1388,28 +1365,13 @@ __global__ void __launch_bounds__(256) k_reduce_partials(const double* __restric
 
 extern "C" int64_t t3d_mesh_measure_workspace_bytes(void) { return (int64_t)MM_BLOCKS * 2 * 8; }
 
-// out_f64[0] = signed volume, out_f64[1] = area (device)
-static int mesh_measure_impl(const void* verts_f32, const void* faces, int64_t F, const unsigned long long* F_dev, int faces_are_i64,
-                             void* out_f64, void* workspace, void* stream);
-
-extern "C" int t3d_mesh_measure(const void* verts_f32, int64_t V, const void* faces, int64_t F, int faces_are_i64, void* out_f64,
-                                void* workspace, void* stream)
-{
-    (void)V;
-    return mesh_measure_impl(verts_f32, faces, F, nullptr, faces_are_i64, out_f64, workspace, stream);
-}
-
-// F is a capacity, the true face count is read from device memory
-extern "C" int t3d_mesh_measure_dev(const void* verts_f32, const void* faces, int64_t F_cap, const void* F_dev_u64, int faces_are_i64,
+// out_f64[0] = signed volume, out_f64[1] = area (device).  F_dev_u64 (optional, device uint64): the true face count when F is
+// only a capacity.
+extern "C" int t3d_mesh_measure_dev(const void* verts_f32, const void* faces, int64_t F, const void* F_dev_u64, int faces_are_i64,
                                     void* out_f64, void* workspace, void* stream)
 {
-    return mesh_measure_impl(verts_f32, faces, F_cap, (const unsigned long long*)F_dev_u64, faces_are_i64, out_f64, workspace, stream);
-}
-
-static int mesh_measure_impl(const void* verts_f32, const void* faces, int64_t F, const unsigned long long* F_dev, int faces_are_i64,
-                             void* out_f64, void* workspace, void* stream)
-{
     cudaStream_t st = (cudaStream_t)stream;
+    const unsigned long long* F_dev = (const unsigned long long*)F_dev_u64;
     if (F <= 0) { T3D_CUDA(cudaMemsetAsync(out_f64, 0, 16, st)); return 0; }
     int blocks = (int)((F + 255) / 256);
     if (blocks > MM_BLOCKS) blocks = MM_BLOCKS;
@@ -1418,7 +1380,7 @@ static int mesh_measure_impl(const void* verts_f32, const void* faces, int64_t F
     else
         k_mesh_measure<int32_t><<<blocks, 256, 0, st>>>((const float*)verts_f32, (const int32_t*)faces, F, (double*)workspace, F_dev);
     k_reduce_partials<<<1, 256, 0, st>>>((const double*)workspace, blocks, (double*)out_f64);
-    T3D_CHECK_LAUNCH("t3d_mesh_measure");
+    T3D_CHECK_LAUNCH("t3d_mesh_measure_dev");
     t3d_count_launches(2);
     return 0;
 }

@@ -729,14 +729,18 @@ def field_sign(dv: DeviceVolume, pad: int, lean: bool = False):
     return sign, (Zp, Hp, Wp), n_exact, n_exc
 
 
-def exclusive_scan_u32(x: torch.Tensor, n: int, n_arrays: int, out_u64: bool = False, popcount_input: bool = False):
+def exclusive_scan_u32(x: torch.Tensor, n: int, n_arrays: int, out_u64: bool = False, popcount_input: bool = False,
+                       totals: Optional[torch.Tensor] = None):
+    """Exclusive scans of the n_arrays arrays of n elements stored back to back in x -> (scans, device int64 totals).
+    totals: where the n_arrays totals go (a slice of a device sizes block); a new tensor if None."""
     L = _L()
     ws = torch.empty(int(L.t3d_scan_workspace_bytes(n, n_arrays)) // 8 + 1, dtype=torch.int64, device=x.device)
-    totals = torch.empty(n_arrays, dtype=torch.int64, device=x.device)
+    if totals is None:
+        totals = torch.empty(n_arrays, dtype=torch.int64, device=x.device)
     out = torch.empty(n * n_arrays, dtype=torch.int64 if out_u64 else torch.int32, device=x.device)
-    check(L.t3d_exclusive_scan_u32(_p(x), _p(out), n, n_arrays, 1 if out_u64 else 0, 1 if popcount_input else 0,
-                                   _p(totals), _p(ws), _stream()),
-          "t3d_exclusive_scan_u32")
+    check(L.t3d_exclusive_scan_u32_dev(_p(x), _p(out), n, n, n_arrays, 1 if out_u64 else 0, 1 if popcount_input else 0, None,
+                                       _p(totals), _p(ws), _stream()),
+          "t3d_exclusive_scan_u32_dev")
     return out, totals
 
 
@@ -756,8 +760,7 @@ def extract_surface(dv: DeviceVolume, slice_depths, mm_per_pixel_y, mm_per_pixel
         Z, H, W = (int(v) for v in field.shape)
         sbits = torch.empty((Z, H, words_per_row(W)), dtype=torch.int32, device=field.device)
         check(L.t3d_sign_from_f32(_p(field), Z, H, W, float(level), _p(sbits), _stream()), "t3d_sign_from_f32")
-        dv, manifold_shift = DeviceVolume(sbits, Z, H, W), manifold
-        manifold = False
+        dv, manifold = DeviceVolume(sbits, Z, H, W), False
     Z, H, W = dv.shape
     pad = 1 if (manifold and add_padding) else 0
     gaussian = 1 if manifold else 0
@@ -777,21 +780,23 @@ def extract_surface(dv: DeviceVolume, slice_depths, mm_per_pixel_y, mm_per_pixel
     mark("field_sign")
     n_chunks = int(L.t3d_mc_num_chunks(Zs, Hs, Ws))
     ballots = torch.empty(n_chunks, dtype=torch.int32, device=dev)
+    # device sizes block {n_active, n_x, n_y, n_z, n_t} (include/t3d.h): the two scans write their totals into it
+    sizes = torch.empty(5, dtype=torch.int64, device=dev)
 
     def flag_and_rank():
         check(L.t3d_mc_flags(_p(sign), Zs, Hs, Ws, z_begin, z_end, _p(ballots), _stream()), "t3d_mc_flags")
-        return exclusive_scan_u32(ballots, n_chunks, 1, popcount_input=True)
+        return exclusive_scan_u32(ballots, n_chunks, 1, popcount_input=True, totals=sizes[:1])[0]
 
-    chunkbase, n_act_t = flag_and_rank()
+    chunkbase = flag_and_rank()
     mark("mc_flags")
     if n_exc_t is not None:
-        n_active, n_exc = (int(v) for v in torch.cat([n_act_t, n_exc_t]).cpu().tolist())
+        n_active, n_exc = (int(v) for v in torch.cat([sizes[:1], n_exc_t]).cpu().tolist())
         if n_exc > EXC_CAP:  # too many isolated voxels for the exception list: robust single-kernel variant
             sign, _, n_exact_t = field_sign(dv, pad, lean=False)
-            chunkbase, n_act_t = flag_and_rank()
-            n_active = int(n_act_t.cpu().item())
+            chunkbase = flag_and_rank()
+            n_active = int(sizes[0].cpu().item())
     else:
-        n_active = int(n_act_t.cpu().item())
+        n_active = int(sizes[0].cpu().item())
     if n_active == 0:
         # skimage: ValueError (level outside the data range) or RuntimeError (no surface)
         raise RuntimeError("No surface found at the given iso value.")
@@ -805,11 +810,11 @@ def extract_surface(dv: DeviceVolume, slice_depths, mm_per_pixel_y, mm_per_pixel
     else:
         mcf = McField(_p(dv.bits), Z, H, W, pad, gaussian, ctypes.cast(_W3_C, ctypes.c_void_p), None, 0.5)
     mcf_p = ctypes.cast(ctypes.pointer(mcf), ctypes.c_void_p)
-    check(L.t3d_mc_words(_p(sign), Zs, Hs, Ws, z_begin, z_end, _p(ballots), _p(chunkbase), n_active, _p(aw_idx), _p(aw_cnt), _p(n_amb),
-                         mcf_p, _stream()), "t3d_mc_words")
-    aw_base, totals = exclusive_scan_u32(aw_cnt, n_active, 4)
+    check(L.t3d_mc_words_dev(_p(sign), Zs, Hs, Ws, z_begin, z_end, _p(ballots), _p(chunkbase), n_active, _p(sizes), _p(aw_idx),
+                             _p(aw_cnt), _p(n_amb), mcf_p, _stream()), "t3d_mc_words_dev")
+    aw_base, _ = exclusive_scan_u32(aw_cnt, n_active, 4, totals=sizes[1:])
     mark("mc_words")
-    tail = torch.cat([totals, n_amb, n_exact_t if n_exact_t is not None else torch.zeros_like(n_amb)]).cpu().tolist()
+    tail = torch.cat([sizes[1:], n_amb, n_exact_t if n_exact_t is not None else torch.zeros_like(n_amb)]).cpu().tolist()
     nX, nY, nZ, nT, n_ambiguous, n_exact = (int(v) for v in tail)
     V = nX + nY + nZ
     if nT == 0 or V == 0:
@@ -820,24 +825,19 @@ def extract_surface(dv: DeviceVolume, slice_depths, mm_per_pixel_y, mm_per_pixel
     faces = torch.empty((nT, 3), dtype=torch.int32, device=dev)
     vkeys = torch.empty(V, dtype=torch.int64, device=dev)
     strong = isinstance(mm_per_pixel_y, np.floating) or isinstance(mm_per_pixel_x, np.floating)
-    check(L.t3d_mc_emit(_p(sign), Zs, Hs, Ws, z_begin, z_end, _p(ballots), _p(chunkbase), _p(aw_idx), _p(aw_base), n_active,
-                        nX, nY,
-                        _p(vkeys), _p(faces), mcf_p, _stream()), "t3d_mc_emit")
+    check(L.t3d_mc_emit_dev(_p(sign), Zs, Hs, Ws, z_begin, z_end, _p(ballots), _p(chunkbase), _p(aw_idx), _p(aw_base), n_active,
+                            _p(sizes), V, nT, _p(vkeys), _p(faces), 3, mcf_p, _stream()), "t3d_mc_emit_dev")
     mark("mc_emit")
-    if field is not None:
-        check(L.t3d_mc_vertices_f32(_p(field), Z, H, W, float(level), _p(vkeys), nX, nY, nZ, 0, z_offset, _p(cum_d), _p(adj_d),
-                                    n_cum, float(mm_per_pixel_y), float(mm_per_pixel_x), 1 if strong else 0, _p(verts),
-                                    _stream()), "t3d_mc_vertices_f32")
-    else:
-        check(L.t3d_mc_vertices(_p(dv.bits), Z, H, W, pad, gaussian, _W3_C, _p(vkeys), nX, nY, nZ, 1 if manifold else 0,
+    occ = None if field is not None else dv.bits     # the vertex and normal kernels read the dense field if one is given
+    unpad = 1 if manifold else 0
+    check(L.t3d_mc_vertices_dev(_p(occ), Z, H, W, pad, gaussian, _W3_C, _p(field), float(level), _p(vkeys), _p(sizes), V, unpad,
                                 z_offset, _p(cum_d), _p(adj_d), n_cum, float(mm_per_pixel_y), float(mm_per_pixel_x),
-                                1 if strong else 0, _p(verts), _stream()), "t3d_mc_vertices")
+                                1 if strong else 0, 7, _p(verts), _stream()), "t3d_mc_vertices_dev")
     mark("mc_vertices")
     src = None
     if normals:
-        src = {"occ": None if field is not None else dv.bits, "field": field, "dims": (Z, H, W), "pad": pad, "gaussian": gaussian,
-               "level": float(level) if field is not None else 0.5, "vkeys": vkeys, "blocks": (nX, nY, nZ),
-               "unpad": 1 if manifold else 0, "z_offset": z_offset, "adj": adj_d, "n_cum": n_cum,
+        src = {"occ": occ, "field": field, "dims": (Z, H, W), "pad": pad, "gaussian": gaussian, "level": float(level), "vkeys": vkeys,
+               "sizes": sizes, "unpad": unpad, "z_offset": z_offset, "adj": adj_d, "n_cum": n_cum,
                "mm": (float(mm_per_pixel_y), float(mm_per_pixel_x))}
     keep = {} if normals else None
     if canonical is None:
@@ -846,28 +846,18 @@ def extract_surface(dv: DeviceVolume, slice_depths, mm_per_pixel_y, mm_per_pixel
         m = DeviceMesh(verts, faces, n_ambiguous, n_exact)
         m.normal_src = src
         return m
-    if canonical == "async":
-        unpad = 1 if (manifold and field is None) else 0
-        res = canonicalize_structured(verts, vkeys, faces, (n_active, nX, nY, nZ, nT), (Zs, Hs, Ws), chunkbase, aw_base, n_active,
-                                      z_offset, unpad, cum_d, adj_d, n_cum, zkey_bits(slice_depths, add_padding, Zs, z_offset, unpad),
-                                      sync=False, keep=keep)
-        v2, f2, counts = res if res is not None else canonicalize(verts, faces, sync=False, fast=True, keep=keep)
-        mark("canonicalize")
-        m = DeviceMesh(v2, f2, n_ambiguous, n_exact, counts_dev=counts)
-        m.raw = (verts, faces)
-        m.n_active, m.n_raw, m.n_z = n_active, (V, nT), nZ
-        if normals:
-            m.normal_src, m.canon_map = src, keep["map"]
-        return m
     # structured ordering (no global sort: x-edge vertices are in place, y-edge vertices ranked per row gap, z-edge vertices
-    # ordered per cube layer); the generic sort-based path only if its device-side order check fails
-    unpad = 1 if (manifold and field is None) else 0
-    res = canonicalize_structured(verts, vkeys, faces, (n_active, nX, nY, nZ, nT), (Zs, Hs, Ws), chunkbase, aw_base, n_active,
-                                  z_offset, unpad, cum_d, adj_d, n_cum, zkey_bits(slice_depths, add_padding, Zs, z_offset, unpad),
-                                  keep=keep)
-    v2, f2 = res if res is not None else canonicalize(verts, faces, fast=True, keep=keep)
+    # ordered per cube layer); the generic sort-based path only if its device-side order check fails.  "async": capacity-sized
+    # arrays, the sizes stay on the device until the mesh is resolved.
+    sync = canonical != "async"
+    res = canonicalize_structured(verts, vkeys, faces, sizes, nZ, (Zs, Hs, Ws), chunkbase, aw_base, n_active, z_offset, unpad,
+                                  cum_d, adj_d, n_cum, zkey_bits(slice_depths, add_padding, Zs, z_offset, unpad), sync=sync, keep=keep)
+    if res is None:
+        res = canonicalize(verts, faces, sync=sync, fast=True, keep=keep)
     mark("canonicalize")
-    m = DeviceMesh(v2, f2, n_ambiguous, n_exact)
+    m = DeviceMesh(res[0], res[1], n_ambiguous, n_exact, counts_dev=None if sync else res[2])
+    if not sync:
+        m.raw = (verts, faces)
     m.n_active, m.n_raw, m.n_z = n_active, (V, nT), nZ
     if normals:
         m.normal_src, m.canon_map = src, keep["map"]
@@ -885,7 +875,7 @@ def canonical_map(ws: torch.Tensor, kind: int, V: int, F: int, cap_z: int = 0, c
 
 
 def mesh_normals(mesh: DeviceMesh) -> torch.Tensor:
-    """Field-gradient normals of a mesh from extract_surface(normals=True): one launch of t3d_mc_normals (plus its tie pass
+    """Field-gradient normals of a mesh from extract_surface(normals=True): one launch of t3d_mc_normals_dev (plus its tie pass
     when the canonicalisation may have merged vertices), rows in the mesh's vertex order."""
     src = mesh.normal_src
     n_rows = int(mesh.verts.shape[0])          # (resolves an asynchronous canonicalisation and its map first)
@@ -894,10 +884,10 @@ def mesh_normals(mesh: DeviceMesh) -> torch.Tensor:
     if mesh.canon_map is not None:
         newid, perm, scratch, dup = (None if a is None else ctypes.c_void_p(a) for a in mesh.canon_map[:4])
     Z, H, W = src["dims"]
-    nX, nY, nZ = src["blocks"]
-    check(_L().t3d_mc_normals(_p(src["occ"]), Z, H, W, src["pad"], src["gaussian"], _W3_C, _p(src["field"]), src["level"],
-                              _p(src["vkeys"]), nX, nY, nZ, src["unpad"], src["z_offset"], _p(src["adj"]), src["n_cum"],
-                              src["mm"][0], src["mm"][1], newid, perm, dup, scratch, _p(out), _stream()), "t3d_mc_normals")
+    check(_L().t3d_mc_normals_dev(_p(src["occ"]), Z, H, W, src["pad"], src["gaussian"], _W3_C, _p(src["field"]), src["level"],
+                                  _p(src["vkeys"]), _p(src["sizes"]), int(src["vkeys"].shape[0]), src["unpad"], src["z_offset"],
+                                  _p(src["adj"]), src["n_cum"], src["mm"][0], src["mm"][1], newid, perm, dup, scratch, _p(out),
+                                  _stream()), "t3d_mc_normals_dev")
     return out
 
 
@@ -905,7 +895,7 @@ def canonicalize(verts: torch.Tensor, faces_i32: torch.Tensor, faces_i64: bool =
                  fast: bool = False, keep: Optional[dict] = None):
     """_ensure_manifold_mesh (surface_extractor.py:115-126) on the device.
 
-    fast=True (meshes in t3d_mc_emit's vertex order only): one stable 64-bit (z,y)-key sort, verified on the device;
+    fast=True (meshes in t3d_mc_emit_dev's vertex order only): one stable 64-bit (z,y)-key sort, verified on the device;
     if the verification fails the general three-key path runs instead (sync=True) or the caller must do so
     (sync=False: returns capacity-sized arrays and the device tensor (V', F', unverified-flag)).
     keep (a dict): receives keep["map"] = canonical_map(...) of the canonicalisation that produced the result."""
@@ -918,8 +908,8 @@ def canonicalize(verts: torch.Tensor, faces_i32: torch.Tensor, faces_i64: bool =
     f64, f32 = (_p(fout), None) if faces_i64 else (None, _p(fout))
     if fast:
         ws = torch.empty(int(L.t3d_canonicalize_fast_workspace_bytes(V, F)) // 8 + 1, dtype=torch.int64, device=dev)
-        check(L.t3d_mesh_canonicalize_fast(_p(verts), V, _p(faces_i32), F, _p(vout), f64, f32, _p(counts), _p(ws), _stream()),
-              "t3d_mesh_canonicalize_fast")
+        check(L.t3d_mesh_canonicalize_fast_dev(_p(verts), V, None, _p(faces_i32), F, None, _p(vout), f64, f32, _p(counts), _p(ws),
+                                               _stream()), "t3d_mesh_canonicalize_fast_dev")
     else:
         ws = torch.empty(int(L.t3d_canonicalize_workspace_bytes(V, F)) // 8 + 1, dtype=torch.int64, device=dev)
         check(L.t3d_mesh_canonicalize(_p(verts), V, _p(faces_i32), F, _p(vout), f64, f32, _p(counts), _p(ws), _stream()),
@@ -934,28 +924,27 @@ def canonicalize(verts: torch.Tensor, faces_i32: torch.Tensor, faces_i64: bool =
     return vout[:v2], fout[:f2]
 
 
-def canonicalize_structured(verts, vkeys, faces_i32, sizes, sign_dims, chunkbase, aw_base, aw_stride, z_offset, unpad_shift, cum_d,
-                            adj_d, n_cum, zkey_bits_, sync: bool = True, keep: Optional[dict] = None):
-    """_ensure_manifold_mesh for a mesh straight out of t3d_mc_emit (t3d_mesh_canonicalize_structured_dev).
+def canonicalize_structured(verts, vkeys, faces_i32, sizes, n_z, sign_dims, chunkbase, aw_base, aw_stride, z_offset, unpad_shift,
+                            cum_d, adj_d, n_cum, zkey_bits_, sync: bool = True, keep: Optional[dict] = None):
+    """_ensure_manifold_mesh for a mesh straight out of t3d_mc_emit_dev (t3d_mesh_canonicalize_structured_dev); `sizes` is the
+    extraction's device sizes block, n_z its z-edge vertex count.
     sync=True: returns (verts, int64 faces) or None when the structured order could not be verified (the caller then sorts
     generically); the clamp group (vertices under slice 0) is provisioned on a second attempt when the first one reports it.
     sync=False: one attempt, returns capacity-sized (verts, faces, device counts (V', F', unverified flag)).
     keep (a dict): receives keep["map"] = canonical_map(...) of the last attempt."""
     L = _L()
-    n_active, nX, nY, nZ, nT = (int(v) for v in sizes)
-    V = nX + nY + nZ
+    V, nT = int(verts.shape[0]), int(faces_i32.shape[0])
     Zs, Hs, Ws = sign_dims
     dev = verts.device
-    sizes_d = torch.tensor([n_active, nX, nY, nZ, nT, V], dtype=torch.int64, device=dev)
     vout = torch.empty((V, 3), dtype=torch.float32, device=dev)
     fout = torch.empty((nT, 3), dtype=torch.int64, device=dev)
     counts = torch.zeros(4, dtype=torch.int64, device=dev)
-    cap_z, cap_g0 = max(nZ, 1), 0
+    cap_z, cap_g0 = max(n_z, 1), 0
     for _attempt in range(2):
         ws = torch.zeros(int(L.t3d_canonicalize_structured_workspace_bytes(V, nT, cap_z, cap_g0, Zs)) // 8 + 1, dtype=torch.int64, device=dev)
         check(L.t3d_mesh_canonicalize_structured_dev(
-            _p(verts), _p(vkeys), V, _p(sizes_d), _p(sizes_d[5:]), Zs, Hs, Ws, _p(chunkbase), _p(aw_base), int(aw_stride), int(z_offset),
-            int(unpad_shift), _p(cum_d), _p(adj_d), int(n_cum), int(zkey_bits_), cap_z, cap_g0, _p(faces_i32), nT, _p(sizes_d[4:]),
+            _p(verts), _p(vkeys), V, _p(sizes), None, Zs, Hs, Ws, _p(chunkbase), _p(aw_base), int(aw_stride), int(z_offset),
+            int(unpad_shift), _p(cum_d), _p(adj_d), int(n_cum), int(zkey_bits_), cap_z, cap_g0, _p(faces_i32), nT, None,
             _p(vout), _p(fout), None, _p(counts), _p(counts[3:]), _p(ws), 3, _stream()), "t3d_mesh_canonicalize_structured_dev")
         if keep is not None:
             keep["map"] = canonical_map(ws, 2, V, nT, cap_z, cap_g0, Zs)
@@ -979,21 +968,13 @@ def mesh_measure_async(verts: torch.Tensor, faces: torch.Tensor) -> torch.Tensor
     out = torch.empty(2, dtype=torch.float64, device=dev)
     verts = verts.contiguous()
     faces = faces.contiguous()
-    check(L.t3d_mesh_measure(_p(verts), int(verts.shape[0]), _p(faces), int(faces.shape[0]),
-                             1 if faces.dtype == torch.int64 else 0, _p(out), _p(ws), _stream()), "t3d_mesh_measure")
+    check(L.t3d_mesh_measure_dev(_p(verts), _p(faces), int(faces.shape[0]), None, 1 if faces.dtype == torch.int64 else 0, _p(out),
+                                 _p(ws), _stream()), "t3d_mesh_measure_dev")
     return out
 
 
 def mesh_measure(verts: torch.Tensor, faces: torch.Tensor) -> Tuple[float, float]:
-    L = _L()
-    dev = verts.device
-    ws = torch.empty(int(L.t3d_mesh_measure_workspace_bytes()) // 8, dtype=torch.float64, device=dev)
-    out = torch.empty(2, dtype=torch.float64, device=dev)
-    verts = verts.contiguous()
-    faces = faces.contiguous()
-    check(L.t3d_mesh_measure(_p(verts), int(verts.shape[0]), _p(faces), int(faces.shape[0]),
-                             1 if faces.dtype == torch.int64 else 0, _p(out), _p(ws), _stream()), "t3d_mesh_measure")
-    v, a = out.cpu().tolist()
+    v, a = mesh_measure_async(verts, faces).cpu().tolist()
     return float(v), float(a)
 
 
