@@ -336,6 +336,41 @@ int t3d_reconstruct_normals(int Z, int H, int W, int n_stages, unsigned erode_ma
                             uint32_t cap_verts, uint32_t cap_faces, uint32_t cap_zverts, uint32_t cap_g0, const void* results_u64,
                             void* workspace, void* normals_out_f32, void* stream);
 
+/* ---- connected components (additive) --------------------------------------------------------------------- */
+
+/* Connected components of an occupancy volume, labelled over x-runs (maximal stretches of set bits in one row;
+ * csrc/t3d_label.cu).  connectivity 6 = scipy.ndimage.generate_binary_structure(3, 1), 26 = np.ones((3, 3, 3)).
+ *   t3d_cc_count   -> row_base_u32[Z*H + 1]: index of each row's first run, [Z*H] = R; n_runs_u64 (device) = R.
+ *   (caller reads R and allocates)
+ *   t3d_cc_label   -> runs_i32 = three int32 arrays of R back to back: x_begin | x_end (inclusive) | row (z*H + y), raster
+ *                     order; run_label_i32[R] = the label of each run, n_components_u64 (device) = K.  Labels are those of
+ *                     scipy.ndimage.label(occ, structure): components numbered 1..K in raster (z, y, x) order of their first
+ *                     voxel, independent of the order the device merges in.  R must fit int32 (returns 2 naming R
+ *                     otherwise, nothing is truncated); K <= R.
+ *   t3d_cc_stats   -> counts_i64[K] = np.bincount(labels.ravel())[1:]; bbox_i32 (K, 6) = {zmin, zmax, ymin, ymax, xmin, xmax}
+ *                     inclusive = scipy.ndimage.find_objects with stop - 1.
+ *   t3d_cc_volumes -> volumes_f64[K]: volume_calculator.py:23-35 applied to each component alone (labels == c):
+ *                     sum over z ascending, z < n_slices, of count[c, z] * slice_volumes_f64[z] in float64 without FMA
+ *                     contraction; slice_volumes_f64[z] = mm_x * mm_y * slice_depths[z] as the reference forms it (caller);
+ *                     bbox_i32 as t3d_cc_stats left it.  Workspace: t3d_cc_volumes_workspace_bytes(R, K).
+ *   t3d_cc_expand  -> labels_i32 (Z, H, W) dense: the scipy.ndimage.label array itself.
+ *   t3d_cc_select  -> out_bits (Z, H, wpr) packed: the voxels whose component has keep_u8[label] != 0 (keep_u8: K + 1 bytes,
+ *                     [0] ignored), padding words written zero. */
+int64_t t3d_cc_count_workspace_bytes(int Z, int H);
+int t3d_cc_count(const void* bits, int Z, int H, int W, void* row_base_u32, void* n_runs_u64, void* workspace, void* stream);
+int64_t t3d_cc_label_workspace_bytes(int64_t n_runs);
+int t3d_cc_label(const void* bits, int Z, int H, int W, int connectivity, const void* row_base_u32, int64_t n_runs, void* runs_i32,
+                 void* run_label_i32, void* n_components_u64, void* workspace, void* stream);
+int t3d_cc_stats(const void* runs_i32, const void* run_label_i32, int64_t n_runs, int H, int64_t n_components, void* counts_i64,
+                 void* bbox_i32, void* stream);
+int64_t t3d_cc_volumes_workspace_bytes(int64_t n_runs, int64_t n_components);
+int t3d_cc_volumes(const void* runs_i32, const void* run_label_i32, int64_t n_runs, int H, int64_t n_components, const void* bbox_i32,
+                   const void* slice_volumes_f64, int n_slices, void* volumes_f64, void* workspace, void* stream);
+int t3d_cc_expand(const void* bits, int Z, int H, int W, const void* row_base_u32, const void* run_label_i32, void* labels_i32,
+                  void* stream);
+int t3d_cc_select(const void* bits, int Z, int H, int W, const void* row_base_u32, const void* run_label_i32, const void* keep_u8,
+                  void* out_bits, void* stream);
+
 /* ---- device-side mesh consumers: the step right after the path (SURVEY.md 8f-3) ----------------------------- */
 
 /* glb_exporter.py:52-91 create_layer_colors: rgba_u8 (V,4) = grey (200,200,200,255); red where first_start <= z <=

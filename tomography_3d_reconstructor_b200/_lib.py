@@ -95,6 +95,15 @@ SIGNATURES = {
     "t3d_canonical_map_offsets": (_i, [_i, _i64, _i64, _u32, _u32, _i, _vp]),
     "t3d_reconstruct_normals": (_i, [_i, _i, _i, _i, _c.c_uint, _i, _vp, _vp, _i, _dbl, _dbl, _u32, _u32, _u32, _u32, _u32, _vp, _vp,
                                      _vp, _vp]),
+    "t3d_cc_count_workspace_bytes": (_i64, [_i, _i]),
+    "t3d_cc_count": (_i, [_vp, _i, _i, _i, _vp, _vp, _vp, _vp]),
+    "t3d_cc_label_workspace_bytes": (_i64, [_i64]),
+    "t3d_cc_label": (_i, [_vp, _i, _i, _i, _i, _vp, _i64, _vp, _vp, _vp, _vp, _vp]),
+    "t3d_cc_stats": (_i, [_vp, _vp, _i64, _i, _i64, _vp, _vp, _vp]),
+    "t3d_cc_volumes_workspace_bytes": (_i64, [_i64, _i64]),
+    "t3d_cc_volumes": (_i, [_vp, _vp, _i64, _i, _i64, _vp, _vp, _i, _vp, _vp, _vp]),
+    "t3d_cc_expand": (_i, [_vp, _i, _i, _i, _vp, _vp, _vp, _vp]),
+    "t3d_cc_select": (_i, [_vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp]),
 }
 
 

@@ -1019,3 +1019,123 @@ def point_cloud(dv: DeviceVolume, mm_per_pixel_x, mm_per_pixel_y, slice_depths, 
                                      float(mm_per_pixel_y), float(mm_per_pixel_x), _p(out), _stream()),
               "t3d_point_cloud_emit")
     return out.cpu().numpy()
+
+
+# ----------------------------------------------------------------------------------------------------------
+# connected components (additive; oracle scipy.ndimage.label)
+# ----------------------------------------------------------------------------------------------------------
+class Components:
+    """Connected components of a DeviceVolume (label_components), kept on the device as a run table: row bases, runs
+    (x_begin | x_end | row), one label per run.  `n` = K; counts / boxes are computed once, with the labelling."""
+
+    __slots__ = ("dv", "connectivity", "n_runs", "row_base", "runs", "run_label", "n", "_counts", "_bbox")
+
+    def __init__(self, dv, connectivity, n_runs, row_base, runs, run_label, n, counts, bbox):
+        self.dv, self.connectivity = dv, connectivity
+        self.n_runs, self.row_base, self.runs, self.run_label, self.n = n_runs, row_base, runs, run_label, n
+        self._counts, self._bbox = counts, bbox
+
+    def counts(self) -> np.ndarray:
+        """int64 (K,) voxels per component = np.bincount(labels.ravel())[1:]."""
+        if isinstance(self._counts, torch.Tensor):
+            self._counts = download(self._counts)
+        return self._counts
+
+    def bbox_index(self) -> np.ndarray:
+        """int32 (K, 6) [zmin, zmax, ymin, ymax, xmin, xmax], inclusive (scipy.ndimage.find_objects, stop - 1)."""
+        if isinstance(self._bbox, torch.Tensor):
+            self._bbox = download(self._bbox)
+        return self._bbox
+
+    def labels(self) -> torch.Tensor:
+        """Device int32 (Z, H, W) label volume, equal to scipy.ndimage.label(grid, structure)[0]."""
+        Z, H, W = self.dv.shape
+        out = torch.empty((Z, H, W), dtype=torch.int32, device=self.dv.bits.device)
+        check(_L().t3d_cc_expand(_p(self.dv.bits), Z, H, W, _p(self.row_base), _p(self.run_label), _p(out), _stream()),
+              "t3d_cc_expand")
+        return out
+
+    def volumes_mm3(self, mm_per_pixel_x, mm_per_pixel_y, slice_depths) -> np.ndarray:
+        """float64 (K,): calculate_voxel_volume_variable_depth (volume_calculator.py:23-35) of each component alone, bit for
+        bit.  The per-component volumes need not add up bit-exactly to the volume of the whole grid: the float64 sums run
+        per component."""
+        K = self.n
+        if K == 0 or len(slice_depths) == 0:
+            return np.zeros(K, dtype=np.float64)
+        n_sv = min(self.dv.Z, len(slice_depths))
+        # the reference's own expression per slice (slice_volume = mm_x * mm_y * slice_depths[z]), evaluated on the host
+        sv = np.array([mm_per_pixel_x * mm_per_pixel_y * slice_depths[z] for z in range(n_sv)], dtype=np.float64)
+        dev = self.dv.bits.device
+        sv_d = torch.from_numpy(sv).to(dev)
+        out = torch.empty(K, dtype=torch.float64, device=dev)
+        L = _L()
+        ws = torch.empty(int(L.t3d_cc_volumes_workspace_bytes(self.n_runs, K)) // 8 + 1, dtype=torch.int64, device=dev)
+        check(L.t3d_cc_volumes(_p(self.runs), _p(self.run_label), self.n_runs, self.dv.H, K, _p(self._bbox_dev()), _p(sv_d), n_sv,
+                               _p(out), _p(ws), _stream()), "t3d_cc_volumes")
+        return download(out)
+
+    def _bbox_dev(self) -> torch.Tensor:
+        b = self._bbox
+        return b if isinstance(b, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(b)).to(self.dv.bits.device)
+
+    def select(self, keep) -> DeviceVolume:
+        """Device volume (the package's bit-packed format) of the voxels whose label is in `keep` (labels 1..K)."""
+        Z, H, W = self.dv.shape
+        dev = self.dv.bits.device
+        mask = np.zeros(self.n + 1, dtype=np.uint8)
+        mask[np.asarray(keep, dtype=np.int64)] = 1
+        mask[0] = 0
+        out = torch.empty_like(self.dv.bits)
+        check(_L().t3d_cc_select(_p(self.dv.bits), Z, H, W, _p(self.row_base), _p(self.run_label), _p(torch.from_numpy(mask).to(dev)),
+                                 _p(out), _stream()), "t3d_cc_select")
+        return DeviceVolume(out, Z, H, W)
+
+
+def label_components(dv: DeviceVolume, connectivity: int = 6) -> Components:
+    """scipy.ndimage.label of the volume with the 6- (scipy's default structure) or 26-connected structure, on the device.
+    Memoised on the volume: labelling, statistics and filtering of the same array label once."""
+    if connectivity not in (6, 26) or isinstance(connectivity, bool):
+        raise ValueError("connectivity must be 6 or 26, got %r" % (connectivity,))
+    key = ("components", int(connectivity))
+    hit = dv.memo.get(key)
+    if hit is not None:
+        return hit
+    L = _L()
+    Z, H, W = dv.shape
+    dev = dv.bits.device
+    rows = Z * H
+    row_base = torch.empty(rows + 1, dtype=torch.int32, device=dev)
+    n_runs_d = torch.empty(1, dtype=torch.int64, device=dev)
+    ws = torch.empty(int(L.t3d_cc_count_workspace_bytes(Z, H)) // 8 + 1, dtype=torch.int64, device=dev)
+    check(L.t3d_cc_count(_p(dv.bits), Z, H, W, _p(row_base), _p(n_runs_d), _p(ws), _stream()), "t3d_cc_count")
+    R = int(n_runs_d.cpu().item())
+    n_alloc = R if R < 2 ** 31 else 0              # beyond int32 t3d_cc_label refuses (status 2) before touching memory
+    runs = torch.empty(3 * n_alloc, dtype=torch.int32, device=dev)
+    run_label = torch.empty(n_alloc, dtype=torch.int32, device=dev)
+    n_comp = torch.empty(1, dtype=torch.int64, device=dev)
+    ws = torch.empty(int(L.t3d_cc_label_workspace_bytes(n_alloc)) // 8 + 1, dtype=torch.int64, device=dev)
+    check(L.t3d_cc_label(_p(dv.bits), Z, H, W, int(connectivity), _p(row_base), R, _p(runs), _p(run_label), _p(n_comp), _p(ws),
+                         _stream()), "t3d_cc_label")
+    del ws
+    K = int(n_comp.cpu().item())
+    counts = torch.empty(K, dtype=torch.int64, device=dev)
+    bbox = torch.empty((K, 6), dtype=torch.int32, device=dev)
+    check(L.t3d_cc_stats(_p(runs), _p(run_label), R, H, K, _p(counts), _p(bbox), _stream()), "t3d_cc_stats")
+    comps = Components(dv, int(connectivity), R, row_base, runs, run_label, K, counts, bbox)
+    dv.memo[key] = comps
+    return comps
+
+
+def component_keep(counts: np.ndarray, min_voxels: int = 1, max_components: Optional[int] = None) -> np.ndarray:
+    """Labels (ascending) of the components a filter keeps: those with at least min_voxels voxels and, if max_components is
+    given, only the max_components largest of them, ties going to the lower label (earlier in raster order).  Host logic."""
+    if min_voxels < 1:
+        raise ValueError("min_voxels must be >= 1, got %r" % (min_voxels,))
+    if max_components is not None and max_components < 1:
+        raise ValueError("max_components must be >= 1 or None, got %r" % (max_components,))
+    counts = np.asarray(counts, dtype=np.int64)
+    cand = np.flatnonzero(counts >= min_voxels)
+    if max_components is not None and len(cand) > max_components:
+        order = np.lexsort((cand, -counts[cand]))      # size descending, then label ascending
+        cand = np.sort(cand[order[:max_components]])
+    return cand + 1

@@ -127,3 +127,44 @@ class VolumeCalculator:
             'surface_area_mm2': surface_area,
             'density': density
         }
+
+    # ------------------------------------------------------------------------------------------------
+    # additive API (no reference counterpart)
+    def analyze_components(self, voxel_data: np.ndarray, mm_per_pixel_x: float, mm_per_pixel_y: float,
+                           slice_depths: np.ndarray, connectivity: int = 6) -> dict:
+        """Per connected component (scipy.ndimage.label numbering, 6- or 26-connected), as arrays over the K components:
+          n_components   K
+          voxel_counts   int64 (K,)
+          volume_mm3     float64 (K,): calculate_voxel_volume_variable_depth(labels == c, ...) bit for bit.  The float64 sums
+                         run per component, so they need not add up bit-exactly to the volume of the whole grid.
+          bbox_index     int32 (K, 6) [zmin, zmax, ymin, ymax, xmin, xmax], inclusive
+          bbox_mm        float64 (K, 6) [z0, z1, y0, y1, x0, x1] and
+          dimensions_mm  float64 (K, 3) [x, y, z] (the order of the reference's 'dimensions'): the values of
+                         calculate_bounding_box_variable_depth(labels == c, ...), bit for bit; all zero when slice_depths is
+                         empty.  Where that function would raise IndexError (a component whose first slice lies beyond
+                         index len(slice_depths)), the z bounds and the z dimension are NaN.
+        Prints nothing."""
+        comps = engine.label_components(self._dv(voxel_data), connectivity)
+        K = comps.n
+        b = comps.bbox_index()
+        bbox_mm = np.zeros((K, 6), dtype=np.float64)
+        dims = np.zeros((K, 3), dtype=np.float64)
+        if K and len(slice_depths):
+            bi = b.astype(np.int64)
+            bbox_mm[:, 4], bbox_mm[:, 5] = bi[:, 4] * mm_per_pixel_x, bi[:, 5] * mm_per_pixel_x
+            bbox_mm[:, 2], bbox_mm[:, 3] = bi[:, 2] * mm_per_pixel_y, bi[:, 3] * mm_per_pixel_y
+            cum = np.cumsum(np.concatenate([[0], slice_depths]))
+            ok = bi[:, 0] < len(cum)
+            bbox_mm[:, 0] = np.where(ok, cum[np.minimum(bi[:, 0], len(cum) - 1)], np.nan)
+            bbox_mm[:, 1] = np.where(ok, cum[np.minimum(bi[:, 1] + 1, len(cum) - 1)], np.nan)
+            dims[:, 0] = bbox_mm[:, 5] - bbox_mm[:, 4]
+            dims[:, 1] = bbox_mm[:, 3] - bbox_mm[:, 2]
+            dims[:, 2] = bbox_mm[:, 1] - bbox_mm[:, 0]
+        return {
+            'n_components': K,
+            'voxel_counts': comps.counts(),
+            'volume_mm3': comps.volumes_mm3(mm_per_pixel_x, mm_per_pixel_y, slice_depths),
+            'bbox_index': b,
+            'bbox_mm': bbox_mm,
+            'dimensions_mm': dims,
+        }

@@ -119,3 +119,20 @@ class VoxelProcessor:
         from . import edt
         dv = engine.volume_from_host(voxel_data)
         return edt.signed_distance(dv, sampling).cpu().numpy()
+
+    def label_components(self, voxel_data: np.ndarray, connectivity: int = 6):
+        """Connected components, as scipy.ndimage.label returns them: (int32 (Z,H,W) labels, number of components).
+        connectivity 6 is scipy's default structure, 26 the full 3x3x3 one; labels are numbered in raster order of each
+        component's first voxel, bit-identical to scipy."""
+        comps = engine.label_components(engine.volume_from_host(voxel_data), connectivity)
+        return engine.download(comps.labels()), comps.n
+
+    def filter_components(self, voxel_data: np.ndarray, min_voxels: int = 1, max_components=None,
+                          connectivity: int = 6) -> np.ndarray:
+        """The voxels of the components with at least min_voxels voxels; with max_components, only that many of the largest
+        of them (ties: the component that comes first in raster order).  Equals np.isin(labels, kept).  The result is a
+        voxel array like smooth_voxel_data's: smoothing, extraction and volumes on it reuse the device copy."""
+        dv = engine.volume_from_host(voxel_data)
+        comps = engine.label_components(dv, connectivity)
+        keep = engine.component_keep(comps.counts(), min_voxels, max_components)
+        return self._publish(comps.select(keep))
