@@ -371,6 +371,41 @@ int t3d_cc_expand(const void* bits, int Z, int H, int W, const void* row_base_u3
 int t3d_cc_select(const void* bits, int Z, int H, int W, const void* row_base_u32, const void* run_label_i32, const void* keep_u8,
                   void* out_bits, void* stream);
 
+/* ---- mesh bodies (additive) ------------------------------------------------------------------------------ */
+
+/* Connected bodies of a triangle mesh: verts_f32 (V, 3), faces (F, 3) int32 or int64 (faces_are_i64).  A body is a connected
+ * component of the graph with the edges f0-f1 and f0-f2 of every face (csrc/t3d_label.cu).  V and the body count B must fit
+ * int32 and F must be at most 2^31 - 1 (status 2 naming the size otherwise, before any memory is touched).
+ *   t3d_mesh_bodies_workspace_bytes(V, F, B): enough for any of the calls below; before B is known pass B = 0 (labelling).
+ *   t3d_mesh_bodies_label     -> vertex_body_i32[V] = scipy.sparse.csgraph.connected_components(G, directed=False)[1]: bodies
+ *                                numbered 0..B-1 by their smallest vertex, independent of the order the device merges in; a
+ *                                vertex used by no face is a body of its own.  n_bodies_u64: two device uint64, [0] = B,
+ *                                [1] = faces with an index outside [0, V) (skipped; the other calls need it to be 0).
+ *   (caller reads B and allocates)
+ *   t3d_mesh_bodies_stats     -> per body: vertex_counts_i64, face_counts_i64 (faces whose f0 is in the body),
+ *                                first_vertex_i64 (its smallest vertex), bbox_f32 (B, 6) {zmin, zmax, ymin, ymax, xmin, xmax} of
+ *                                its vertex columns (a zero bound is +0.0), and volumes_f64 / areas_f64: the sum over its faces of
+ *                                the terms of t3d_mesh_measure_dev (float64, left to right, no FMA contraction), each rounded
+ *                                half-to-even to a multiple of 2^-64 and added exactly in 128-bit fixed point, the sum rounded
+ *                                once to float64.  Bit-identical in any launch order.  Reads one word back at its end: if a
+ *                                |term| >= 2^62 or F * max|term| >= 2^63 (the sums could leave 128 bits) it returns 2 naming the
+ *                                bound, and the sums are not valid.
+ *   t3d_mesh_bodies_face_body -> face_body_i32[F] = vertex_body[faces[f, 0]].
+ *   t3d_mesh_bodies_select    -> the vertices (and normal rows, if normals_f32 is not NULL) of the bodies with keep_u8[b] != 0
+ *                                and their faces, each in input order; faces (input dtype) renumbered to the kept vertices.
+ *                                The caller sizes the outputs from the counts of t3d_mesh_bodies_stats. */
+int64_t t3d_mesh_bodies_workspace_bytes(int64_t V, int64_t F, int64_t B);
+int t3d_mesh_bodies_label(const void* faces, int64_t F, int faces_are_i64, int64_t V, void* vertex_body_i32, void* n_bodies_u64,
+                          void* workspace, void* stream);
+int t3d_mesh_bodies_stats(const void* verts_f32, const void* faces, int64_t F, int faces_are_i64, int64_t V, const void* vertex_body_i32,
+                          int64_t B, void* vertex_counts_i64, void* face_counts_i64, void* first_vertex_i64, void* bbox_f32,
+                          void* volumes_f64, void* areas_f64, void* workspace, void* stream);
+int t3d_mesh_bodies_face_body(const void* faces, int64_t F, int faces_are_i64, const void* vertex_body_i32, void* face_body_i32,
+                              void* stream);
+int t3d_mesh_bodies_select(const void* verts_f32, const void* normals_f32, const void* faces, int64_t F, int faces_are_i64, int64_t V,
+                           const void* vertex_body_i32, int64_t B, const void* keep_u8, void* verts_out_f32, void* normals_out_f32,
+                           void* faces_out, void* workspace, void* stream);
+
 /* ---- device-side mesh consumers: the step right after the path (SURVEY.md 8f-3) ----------------------------- */
 
 /* glb_exporter.py:52-91 create_layer_colors: rgba_u8 (V,4) = grey (200,200,200,255); red where first_start <= z <=

@@ -104,6 +104,11 @@ SIGNATURES = {
     "t3d_cc_volumes": (_i, [_vp, _vp, _i64, _i, _i64, _vp, _vp, _i, _vp, _vp, _vp]),
     "t3d_cc_expand": (_i, [_vp, _i, _i, _i, _vp, _vp, _vp, _vp]),
     "t3d_cc_select": (_i, [_vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp]),
+    "t3d_mesh_bodies_workspace_bytes": (_i64, [_i64, _i64, _i64]),
+    "t3d_mesh_bodies_label": (_i, [_vp, _i64, _i, _i64, _vp, _vp, _vp, _vp]),
+    "t3d_mesh_bodies_stats": (_i, [_vp, _vp, _i64, _i, _i64, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "t3d_mesh_bodies_face_body": (_i, [_vp, _i64, _i, _vp, _vp, _vp]),
+    "t3d_mesh_bodies_select": (_i, [_vp, _vp, _vp, _i64, _i, _i64, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp]),
 }
 
 

@@ -18,6 +18,7 @@
 //   expand / select: warp per row, the run of a set bit is the row's base + (run starts at or before it) - 1
 #include <limits.h>
 #include <stdint.h>
+#include <string.h>
 
 #include "t3d.h"
 #include "t3d_common.cuh"
@@ -158,13 +159,15 @@ __global__ void __launch_bounds__(CC_THREADS) k_cc_flatten(int32_t* P, int64_t R
     if (lane_id() == 0 && i < R) root_mask[i >> 5] = m;
 }
 
+// label = first_label + roots before the element's root (1: scipy.ndimage.label's numbering, 0: csgraph's)
 __global__ void __launch_bounds__(CC_THREADS) k_cc_number(const int32_t* __restrict__ P, int64_t R, const uint32_t* __restrict__ root_mask,
-                                                          const uint32_t* __restrict__ word_base, int32_t* __restrict__ run_label)
+                                                          const uint32_t* __restrict__ word_base, int32_t first_label,
+                                                          int32_t* __restrict__ run_label)
 {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= R) return;
     const int r = P[i];
-    run_label[i] = 1 + (int32_t)word_base[r >> 5] + __popc(root_mask[r >> 5] & ((1u << (r & 31)) - 1u));
+    run_label[i] = first_label + (int32_t)word_base[r >> 5] + __popc(root_mask[r >> 5] & ((1u << (r & 31)) - 1u));
 }
 
 // extents are accumulated as {INT_MAX - zmin, zmax + 1, INT_MAX - ymin, ymax + 1, INT_MAX - xmin, xmax + 1} with atomicMax
@@ -392,7 +395,7 @@ extern "C" int t3d_cc_label(const void* bits, int Z, int H, int W, int connectiv
     t3d_count_launches(3);
     if (int rc = t3d_exclusive_scan_u32_dev(root_mask, word_base, nw, nw, 1, 0, 1, nullptr, n_components_u64, scan_ws, stream))
         return rc;
-    k_cc_number<<<cc_blocks(R), CC_THREADS, 0, st>>>(parent, R, root_mask, word_base, (int32_t*)run_label_i32);
+    k_cc_number<<<cc_blocks(R), CC_THREADS, 0, st>>>(parent, R, root_mask, word_base, 1, (int32_t*)run_label_i32);
     T3D_CHECK_LAUNCH("t3d_cc_label number");
     t3d_count_launches(1);
     return 0;
@@ -484,6 +487,530 @@ extern "C" int t3d_cc_select(const void* bits, int Z, int H, int W, const void* 
         (const uint32_t*)bits, rows, t3d_wpr(W), t3d_wvalid(W), (const uint32_t*)row_base_u32, (const int32_t*)run_label_i32,
         (const uint8_t*)keep_u8, (uint32_t*)out_bits);
     T3D_CHECK_LAUNCH("t3d_cc_select");
+    t3d_count_launches(1);
+    return 0;
+}
+
+// ------------------------------------------------------------------------------------------------
+// Mesh bodies: connected components of a triangle mesh's vertex graph (oracle: scipy.sparse.csgraph.connected_components
+// of the edges f0-f1 and f0-f2 of every face), with the voxel labeller's union-find over vertices instead of runs.
+//   label   k_mb_init: parent[v] = v; k_mb_merge: unite(f0, f1), unite(f0, f2) per face (faces with an index outside
+//           [0, V) are counted and skipped); k_cc_flatten / scan / k_cc_number with first label 0: the root of a body is
+//           its smallest vertex, so bodies are numbered by their smallest vertex, as csgraph numbers them
+//   stats   k_mb_vstats per vertex (count, first vertex, box) and k_mb_fstats per face (count, signed volume and area as
+//           128-bit fixed point in four 32-bit limbs, each summed in a 64-bit integer); a block or warp whose elements share
+//           a body sends one set of atomics; k_mb_final normalises the limbs and rounds each sum once to float64
+//   select  keep bitmasks of vertices and faces, scans of their popcounts, then the compaction with remapped face ids
+// ------------------------------------------------------------------------------------------------
+#define MB_WARPS (CC_THREADS / 32)
+
+__global__ void __launch_bounds__(CC_THREADS) k_mb_init(int32_t* __restrict__ P, int64_t V)
+{
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < V) P[i] = (int32_t)i;
+}
+
+template <typename IdxT>
+__global__ void __launch_bounds__(CC_THREADS) k_mb_merge(const IdxT* __restrict__ faces, int64_t F, int64_t V, int32_t* P,
+                                                         unsigned long long* __restrict__ n_bad)
+{
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= F) return;
+    const int64_t a = (int64_t)faces[3 * i], b = (int64_t)faces[3 * i + 1], c = (int64_t)faces[3 * i + 2];
+    if (a < 0 || a >= V || b < 0 || b >= V || c < 0 || c >= V) {
+        atomicAdd(n_bad, 1ull);
+        return;
+    }
+    cc_unite(P, (int)a, (int)b);
+    cc_unite(P, (int)a, (int)c);
+}
+
+// per-body accumulators of one pass: NS summed and NX max-reduced 64-bit values, NM max-reduced 32-bit values
+template <int NS, int NX, int NM>
+struct MbVals {
+    unsigned long long s[NS > 0 ? NS : 1];
+    unsigned long long x[NX > 0 ? NX : 1];
+    uint32_t m[NM > 0 ? NM : 1];
+};
+
+template <int NS, int NX, int NM>
+__device__ __forceinline__ void mb_warp_reduce(MbVals<NS, NX, NM>& v)
+{
+#pragma unroll
+    for (int k = 0; k < NS; ++k) v.s[k] = warp_sum(v.s[k]);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+#pragma unroll
+        for (int k = 0; k < NX; ++k) v.x[k] = max(v.x[k], (unsigned long long)__shfl_xor_sync(0xffffffffu, v.x[k], o));
+#pragma unroll
+        for (int k = 0; k < NM; ++k) v.m[k] = max(v.m[k], __shfl_xor_sync(0xffffffffu, v.m[k], o));
+    }
+}
+
+template <int NS, int NX, int NM>
+__device__ __forceinline__ void mb_atomics(int b, const MbVals<NS, NX, NM>& v, unsigned long long* S, unsigned long long* X, uint32_t* M)
+{
+#pragma unroll
+    for (int k = 0; k < NS; ++k) if (v.s[k]) atomicAdd(S + (int64_t)NS * b + k, v.s[k]);
+#pragma unroll
+    for (int k = 0; k < NX; ++k) atomicMax(X + (int64_t)NX * b + k, v.x[k]);
+#pragma unroll
+    for (int k = 0; k < NM; ++k) atomicMax(M + (int64_t)NM * b + k, v.m[k]);
+}
+
+// Adds the values of every thread of the block (body b, or -1 for none) into the per-body accumulators.  All threads of the
+// block call it.  A block whose threads all hold one body sends one set of atomics, a warp that does sends one, any other
+// thread its own: the integer sums and maxima are the same whichever way they are grouped.
+template <int NS, int NX, int NM>
+__device__ __forceinline__ void mb_commit(int b, MbVals<NS, NX, NM> v, unsigned long long* S, unsigned long long* X, uint32_t* M)
+{
+    __shared__ int sb[MB_WARPS];
+    __shared__ MbVals<NS, NX, NM> sv[MB_WARPS];
+    const int w = threadIdx.x >> 5;
+    const int b0 = __shfl_sync(0xffffffffu, b, 0);
+    const bool wuni = __all_sync(0xffffffffu, b == b0);
+    if (lane_id() == 0) sb[w] = wuni ? b0 : -1;
+    __syncthreads();
+    bool buni = sb[0] >= 0;
+#pragma unroll
+    for (int k = 1; k < MB_WARPS; ++k) buni = buni && sb[k] == sb[0];
+    if (wuni) {
+        mb_warp_reduce(v);
+        if (!buni && lane_id() == 0 && b0 >= 0) mb_atomics(b0, v, S, X, M);
+    } else if (b >= 0) {
+        mb_atomics(b, v, S, X, M);
+    }
+    if (!buni) return;                          // the same for the whole block
+    if (lane_id() == 0) sv[w] = v;
+    __syncthreads();
+    if (threadIdx.x != 0) return;
+    MbVals<NS, NX, NM> t = sv[0];
+    for (int k = 1; k < MB_WARPS; ++k) {
+#pragma unroll
+        for (int j = 0; j < NS; ++j) t.s[j] += sv[k].s[j];
+#pragma unroll
+        for (int j = 0; j < NX; ++j) t.x[j] = max(t.x[j], sv[k].x[j]);
+#pragma unroll
+        for (int j = 0; j < NM; ++j) t.m[j] = max(t.m[j], sv[k].m[j]);
+    }
+    mb_atomics(b0, t, S, X, M);
+}
+
+// float -> uint32 key in the float order; -0.0 is taken as +0.0, so a zero bound comes out as +0.0
+__device__ __forceinline__ uint32_t mb_key(float f)
+{
+    uint32_t u = __float_as_uint(f);
+    if (u == 0x80000000u) u = 0u;
+    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+__device__ __forceinline__ float mb_unkey(uint32_t k) { return __uint_as_float((k & 0x80000000u) ? (k & 0x7fffffffu) : ~k); }
+
+// per vertex: count, first vertex (max of ~v), box {~key(min), key(max)} per column
+__global__ void __launch_bounds__(CC_THREADS) k_mb_vstats(const float* __restrict__ verts, int64_t V, const int32_t* __restrict__ vb,
+                                                          unsigned long long* __restrict__ vcount, unsigned long long* __restrict__ first_inv,
+                                                          uint32_t* __restrict__ box_key)
+{
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    MbVals<1, 1, 6> v = {};
+    int b = -1;
+    if (i < V) {
+        b = vb[i];
+        v.s[0] = 1;
+        v.x[0] = ~(unsigned long long)i;
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+            const uint32_t k = mb_key(verts[3 * i + c]);
+            v.m[2 * c] = ~k;
+            v.m[2 * c + 1] = k;
+        }
+    }
+    mb_commit(b, v, vcount, first_inv, box_key);
+}
+
+// k_mesh_measure's two terms (t3d_surface.cu), left to right without FMA contraction
+__device__ __forceinline__ void mb_terms(const float* a, const float* b, const float* c, double& vol, double& area)
+{
+    const double ax = a[0], ay = a[1], az = a[2], bx = b[0], by = b[1], bz = b[2], cx = c[0], cy = c[1], cz = c[2];
+    const double nx = __dsub_rn(__dmul_rn(by, cz), __dmul_rn(bz, cy));
+    const double ny = __dsub_rn(__dmul_rn(bz, cx), __dmul_rn(bx, cz));
+    const double nz = __dsub_rn(__dmul_rn(bx, cy), __dmul_rn(by, cx));
+    vol = __ddiv_rn(__dadd_rn(__dadd_rn(__dmul_rn(ax, nx), __dmul_rn(ay, ny)), __dmul_rn(az, nz)), 6.0);
+    const double ux = __dsub_rn(bx, ax), uy = __dsub_rn(by, ay), uz = __dsub_rn(bz, az);
+    const double vx = __dsub_rn(cx, ax), vy = __dsub_rn(cy, ay), vz = __dsub_rn(cz, az);
+    const double px = __dsub_rn(__dmul_rn(uy, vz), __dmul_rn(uz, vy));
+    const double py = __dsub_rn(__dmul_rn(uz, vx), __dmul_rn(ux, vz));
+    const double pz = __dsub_rn(__dmul_rn(ux, vy), __dmul_rn(uy, vx));
+    area = __dmul_rn(0.5, __dsqrt_rn(__dadd_rn(__dadd_rn(__dmul_rn(px, px), __dmul_rn(py, py)), __dmul_rn(pz, pz))));
+}
+
+// t rounded half-to-even to a multiple of 2^-64, as a 128-bit two's complement integer in four 32-bit limbs (in 64-bit
+// slots).  |t| < 2^62 makes t * 2^64 exact and below 2^126; anything else (never accepted, see t3d_mesh_bodies_stats) is 0.
+__device__ __forceinline__ void mb_fixed(double t, unsigned long long* L)
+{
+    L[0] = L[1] = L[2] = L[3] = 0;
+    if (!(fabs(t) < 0x1p62)) return;
+    const double r = rint(__dmul_rn(t, 0x1p64));
+    const unsigned long long u = (unsigned long long)__double_as_longlong(r);
+    const int e = (int)((u >> 52) & 0x7ff);
+    if (e == 0) return;                         // r == 0
+    const unsigned long long m = (u & ((1ull << 52) - 1)) | (1ull << 52);
+    const int sh = e - 1075;                    // |r| = m * 2^sh, -52 <= sh <= 73 (r is an integer below 2^126)
+    unsigned long long lo, hi;
+    if (sh <= 0) { lo = m >> -sh; hi = 0; }
+    else if (sh < 64) { lo = m << sh; hi = m >> (64 - sh); }
+    else { lo = 0; hi = m << (sh - 64); }
+    if (r < 0) { lo = ~lo + 1; hi = ~hi + (lo == 0 ? 1 : 0); }
+    L[0] = lo & 0xffffffffull; L[1] = lo >> 32; L[2] = hi & 0xffffffffull; L[3] = hi >> 32;
+}
+
+// per face: acc[9 b] = {count, 4 volume limbs, 4 area limbs}, tmax[b] = max over the body's faces of |term| (float64 bits)
+template <typename IdxT>
+__global__ void __launch_bounds__(CC_THREADS) k_mb_fstats(const float* __restrict__ verts, const IdxT* __restrict__ faces, int64_t F,
+                                                          const int32_t* __restrict__ vb, unsigned long long* __restrict__ acc,
+                                                          unsigned long long* __restrict__ tmax)
+{
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    MbVals<9, 1, 0> v = {};
+    int b = -1;
+    if (i < F) {
+        const int64_t f0 = (int64_t)faces[3 * i];
+        b = vb[f0];
+        double tv, ta;
+        mb_terms(verts + 3 * f0, verts + 3 * (int64_t)faces[3 * i + 1], verts + 3 * (int64_t)faces[3 * i + 2], tv, ta);
+        v.s[0] = 1;
+        mb_fixed(tv, v.s + 1);
+        mb_fixed(ta, v.s + 5);
+        const unsigned long long mv = (unsigned long long)__double_as_longlong(fabs(tv));
+        const unsigned long long ma = (unsigned long long)__double_as_longlong(fabs(ta));   // NaN sorts above every number
+        v.x[0] = max(mv, ma);
+    }
+    mb_commit(b, v, acc, tmax, (uint32_t*)nullptr);
+}
+
+// the 128-bit sum of four limb sums c[k] (value sum_k c[k] 2^(32k) mod 2^128, read as signed) times 2^-64, rounded once
+__device__ __forceinline__ double mb_to_double(const unsigned long long* c)
+{
+    unsigned long long w[4], carry = 0;
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+        const unsigned long long t = c[k] + carry;
+        w[k] = t & 0xffffffffull;
+        carry = t >> 32;
+    }
+    unsigned long long lo = w[0] | (w[1] << 32), hi = w[2] | (w[3] << 32);
+    const bool neg = (hi >> 63) != 0;
+    if (neg) { lo = ~lo + 1; hi = ~hi + (lo == 0 ? 1 : 0); }
+    double d;
+    int scale;
+    if (hi == 0) {
+        d = __ull2double_rn(lo);
+        scale = -64;
+    } else {
+        // keep the top 64 bits and fold the rest into a sticky bit: the 64 -> 53-bit rounding then equals the 128 -> 53-bit one
+        const int p = 63 - __clzll((long long)hi);             // leading bit of hi
+        const int s = p + 1;                                    // bits shifted out of lo, 1..64
+        const unsigned long long top = s == 64 ? hi : (hi << (64 - s)) | (lo >> s);
+        const unsigned long long sticky = s == 64 ? (lo != 0) : ((lo << (64 - s)) != 0);
+        d = __ull2double_rn(top | sticky);
+        scale = s - 64;
+    }
+    d = __dmul_rn(d, __longlong_as_double((long long)(1023 + scale) << 52));   // exact: a power of two in the normal range
+    return neg ? -d : d;
+}
+
+__global__ void __launch_bounds__(CC_THREADS) k_mb_final(int64_t B, const unsigned long long* __restrict__ acc,
+                                                         const unsigned long long* __restrict__ tmax,
+                                                         const unsigned long long* __restrict__ first_inv,
+                                                         const uint32_t* __restrict__ box_key, long long* __restrict__ fcount,
+                                                         long long* __restrict__ first, float* __restrict__ bbox,
+                                                         double* __restrict__ vol, double* __restrict__ area,
+                                                         unsigned long long* __restrict__ tmax_all)
+{
+    const int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= B) return;
+    const unsigned long long* a = acc + 9 * b;
+    fcount[b] = (long long)a[0];
+    first[b] = (long long)~first_inv[b];
+#pragma unroll
+    for (int k = 0; k < 6; ++k) {
+        const uint32_t key = box_key[6 * b + k];
+        bbox[6 * b + k] = mb_unkey((k & 1) ? key : ~key);
+    }
+    vol[b] = mb_to_double(a + 1);
+    area[b] = mb_to_double(a + 5);
+    if (a[0]) atomicMax(tmax_all, tmax[b]);
+}
+
+// keep bitmasks: threads [0, 32 nwv) vertices, [32 nwv, 32 (nwv + nwf)) faces; bit set iff keep[body]
+template <typename IdxT>
+__global__ void __launch_bounds__(CC_THREADS) k_mb_keep(const IdxT* __restrict__ faces, int64_t F, int64_t V, const int32_t* __restrict__ vb,
+                                                        const uint8_t* __restrict__ keep, int64_t nwv, int64_t nwf,
+                                                        uint32_t* __restrict__ vmask, uint32_t* __restrict__ fmask)
+{
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const bool is_v = t < 32 * nwv;
+    const int64_t i = is_v ? t : t - 32 * nwv;
+    bool k = false;
+    if (is_v) { if (i < V) k = keep[vb[i]] != 0; }
+    else if (i < F) k = keep[vb[faces[3 * i]]] != 0;
+    const uint32_t m = __ballot_sync(0xffffffffu, k);
+    if (lane_id() == 0 && (i >> 5) < (is_v ? nwv : nwf)) (is_v ? vmask : fmask)[i >> 5] = m;
+}
+
+__device__ __forceinline__ int64_t mb_rank(const uint32_t* mask, const uint32_t* base, int64_t i)
+{
+    return (int64_t)base[i >> 5] + __popc(mask[i >> 5] & ((1u << (i & 31)) - 1u));
+}
+
+__global__ void __launch_bounds__(CC_THREADS) k_mb_compact_verts(const float* __restrict__ verts, const float* __restrict__ normals,
+                                                                 int64_t V, const uint32_t* __restrict__ vmask, const uint32_t* __restrict__ vbase,
+                                                                 float* __restrict__ verts_out, float* __restrict__ normals_out)
+{
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= V || !((vmask[i >> 5] >> (i & 31)) & 1u)) return;
+    const int64_t o = mb_rank(vmask, vbase, i);
+#pragma unroll
+    for (int c = 0; c < 3; ++c) verts_out[3 * o + c] = verts[3 * i + c];
+    if (normals) {
+#pragma unroll
+        for (int c = 0; c < 3; ++c) normals_out[3 * o + c] = normals[3 * i + c];
+    }
+}
+
+template <typename IdxT>
+__global__ void __launch_bounds__(CC_THREADS) k_mb_compact_faces(const IdxT* __restrict__ faces, int64_t F, const uint32_t* __restrict__ vmask,
+                                                                 const uint32_t* __restrict__ vbase, const uint32_t* __restrict__ fmask,
+                                                                 const uint32_t* __restrict__ fbase, IdxT* __restrict__ faces_out)
+{
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= F || !((fmask[i >> 5] >> (i & 31)) & 1u)) return;
+    const int64_t o = mb_rank(fmask, fbase, i);
+#pragma unroll
+    for (int c = 0; c < 3; ++c) faces_out[3 * o + c] = (IdxT)mb_rank(vmask, vbase, (int64_t)faces[3 * i + c]);
+}
+
+template <typename IdxT>
+__global__ void __launch_bounds__(CC_THREADS) k_mb_face_body(const IdxT* __restrict__ faces, int64_t F, const int32_t* __restrict__ vb,
+                                                             int32_t* __restrict__ fb)
+{
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < F) fb[i] = vb[faces[3 * i]];
+}
+
+// ---- mesh bodies: C ABI --------------------------------------------------------------------------
+static int mb_sizes_ok(const char* who, int64_t F, int64_t V, int64_t B)
+{
+    if (V < 0 || V > INT_MAX) {
+        t3d_set_error("%s: %lld vertices, more than the int32 body labels allow (%d)", who, (long long)V, INT_MAX);
+        return 2;
+    }
+    if (B < 0 || B > V) {
+        t3d_set_error("%s: %lld bodies for %lld vertices", who, (long long)B, (long long)V);
+        return 2;
+    }
+    if (F < 0 || F > INT_MAX) {
+        t3d_set_error("%s: %lld faces; the per-body sums are exact up to %d faces", who, (long long)F, INT_MAX);
+        return 2;
+    }
+    return 0;
+}
+
+struct MbLabelWs { int32_t* parent; uint32_t* root_mask; uint32_t* word_base; void* scan; };
+struct MbStatsWs { unsigned long long* acc; unsigned long long* tmax; unsigned long long* first_inv; uint32_t* box_key;
+                   unsigned long long* tmax_all; int64_t zero_bytes; };
+struct MbSelectWs { uint32_t* vmask; uint32_t* vbase; uint32_t* fmask; uint32_t* fbase; unsigned long long* totals; void* scan; };
+
+static int64_t mb_label_ws(int64_t V, char* ws, MbLabelWs* o)
+{
+    const int64_t nw = (V + 31) / 32;
+    int64_t off = 0;
+    if (o) o->parent = (int32_t*)(ws + off);
+    off += cc_align(4 * V);
+    if (o) o->root_mask = (uint32_t*)(ws + off);
+    off += cc_align(4 * nw);
+    if (o) o->word_base = (uint32_t*)(ws + off);
+    off += cc_align(4 * nw);
+    if (o) o->scan = ws + off;
+    return off + cc_align(t3d_scan_workspace_bytes(nw, 1));
+}
+
+static int64_t mb_stats_ws(int64_t B, char* ws, MbStatsWs* o)
+{
+    // everything the passes accumulate into lies in one range zeroed by one memset
+    int64_t off = 0;
+    if (o) o->acc = (unsigned long long*)(ws + off);
+    off += cc_align(72 * B);
+    if (o) o->tmax = (unsigned long long*)(ws + off);
+    off += cc_align(8 * B);
+    if (o) o->first_inv = (unsigned long long*)(ws + off);
+    off += cc_align(8 * B);
+    if (o) o->box_key = (uint32_t*)(ws + off);
+    off += cc_align(24 * B);
+    if (o) o->tmax_all = (unsigned long long*)(ws + off);
+    off += 256;
+    if (o) o->zero_bytes = off;
+    return off;
+}
+
+static int64_t mb_select_ws(int64_t V, int64_t F, char* ws, MbSelectWs* o)
+{
+    const int64_t nwv = (V + 31) / 32, nwf = (F + 31) / 32;
+    int64_t off = 0;
+    if (o) o->vmask = (uint32_t*)(ws + off);
+    off += cc_align(4 * nwv);
+    if (o) o->vbase = (uint32_t*)(ws + off);
+    off += cc_align(4 * nwv);
+    if (o) o->fmask = (uint32_t*)(ws + off);
+    off += cc_align(4 * nwf);
+    if (o) o->fbase = (uint32_t*)(ws + off);
+    off += cc_align(4 * nwf);
+    if (o) o->totals = (unsigned long long*)(ws + off);
+    off += 256;
+    if (o) o->scan = ws + off;
+    const int64_t sv = t3d_scan_workspace_bytes(nwv, 1), sf = t3d_scan_workspace_bytes(nwf, 1);
+    return off + cc_align(sv > sf ? sv : sf);
+}
+
+extern "C" int64_t t3d_mesh_bodies_workspace_bytes(int64_t V, int64_t F, int64_t B)
+{
+    int64_t n = mb_label_ws(V, nullptr, nullptr);
+    const int64_t s = mb_stats_ws(B, nullptr, nullptr), c = mb_select_ws(V, F, nullptr, nullptr);
+    if (s > n) n = s;
+    if (c > n) n = c;
+    return n;
+}
+
+extern "C" int t3d_mesh_bodies_label(const void* faces, int64_t F, int faces_are_i64, int64_t V, void* vertex_body_i32,
+                                     void* n_bodies_u64, void* workspace, void* stream)
+{
+    if (V < 0 || V > INT_MAX) {
+        t3d_set_error("t3d_mesh_bodies_label: %lld vertices, more than the int32 body labels allow (%d)", (long long)V, INT_MAX);
+        return 2;
+    }
+    if (F < 0) {
+        t3d_set_error("t3d_mesh_bodies_label: bad face count %lld", (long long)F);
+        return 2;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    if (t3d_zero_async(n_bodies_u64, 16, st)) return 1;
+    MbLabelWs w;
+    mb_label_ws(V, (char*)workspace, &w);
+    unsigned long long* n_bad = (unsigned long long*)n_bodies_u64 + 1;
+    if (V > 0) {
+        k_mb_init<<<cc_blocks(V), CC_THREADS, 0, st>>>(w.parent, V);
+        t3d_count_launches(1);
+    }
+    if (F > 0) {
+        if (faces_are_i64)
+            k_mb_merge<long long><<<cc_blocks(F), CC_THREADS, 0, st>>>((const long long*)faces, F, V, w.parent, n_bad);
+        else
+            k_mb_merge<int32_t><<<cc_blocks(F), CC_THREADS, 0, st>>>((const int32_t*)faces, F, V, w.parent, n_bad);
+        t3d_count_launches(1);
+    }
+    T3D_CHECK_LAUNCH("t3d_mesh_bodies_label merge");
+    if (V == 0) return 0;
+    const int64_t nw = (V + 31) / 32;
+    k_cc_flatten<<<cc_blocks(V), CC_THREADS, 0, st>>>(w.parent, V, w.root_mask);
+    T3D_CHECK_LAUNCH("t3d_mesh_bodies_label flatten");
+    t3d_count_launches(1);
+    if (int rc = t3d_exclusive_scan_u32_dev(w.root_mask, w.word_base, nw, nw, 1, 0, 1, nullptr, n_bodies_u64, w.scan, stream)) return rc;
+    k_cc_number<<<cc_blocks(V), CC_THREADS, 0, st>>>(w.parent, V, w.root_mask, w.word_base, 0, (int32_t*)vertex_body_i32);
+    T3D_CHECK_LAUNCH("t3d_mesh_bodies_label number");
+    t3d_count_launches(1);
+    return 0;
+}
+
+extern "C" int t3d_mesh_bodies_stats(const void* verts_f32, const void* faces, int64_t F, int faces_are_i64, int64_t V,
+                                     const void* vertex_body_i32, int64_t B, void* vertex_counts_i64, void* face_counts_i64,
+                                     void* first_vertex_i64, void* bbox_f32, void* volumes_f64, void* areas_f64, void* workspace,
+                                     void* stream)
+{
+    if (int rc = mb_sizes_ok("t3d_mesh_bodies_stats", F, V, B)) return rc;
+    if (B == 0) return 0;
+    cudaStream_t st = (cudaStream_t)stream;
+    MbStatsWs w;
+    mb_stats_ws(B, (char*)workspace, &w);
+    if (t3d_zero_async(w.acc, w.zero_bytes, st) || t3d_zero_async(vertex_counts_i64, 8 * B, st)) return 1;
+    const int32_t* vb = (const int32_t*)vertex_body_i32;
+    k_mb_vstats<<<cc_blocks(V), CC_THREADS, 0, st>>>((const float*)verts_f32, V, vb, (unsigned long long*)vertex_counts_i64, w.first_inv,
+                                                     w.box_key);
+    T3D_CHECK_LAUNCH("t3d_mesh_bodies_stats vertices");
+    if (F > 0) {
+        if (faces_are_i64)
+            k_mb_fstats<long long><<<cc_blocks(F), CC_THREADS, 0, st>>>((const float*)verts_f32, (const long long*)faces, F, vb, w.acc, w.tmax);
+        else
+            k_mb_fstats<int32_t><<<cc_blocks(F), CC_THREADS, 0, st>>>((const float*)verts_f32, (const int32_t*)faces, F, vb, w.acc, w.tmax);
+        T3D_CHECK_LAUNCH("t3d_mesh_bodies_stats faces");
+    }
+    k_mb_final<<<cc_blocks(B), CC_THREADS, 0, st>>>(B, w.acc, w.tmax, w.first_inv, w.box_key, (long long*)face_counts_i64,
+                                                    (long long*)first_vertex_i64, (float*)bbox_f32, (double*)volumes_f64,
+                                                    (double*)areas_f64, w.tmax_all);
+    T3D_CHECK_LAUNCH("t3d_mesh_bodies_stats final");
+    t3d_count_launches(F > 0 ? 3 : 2);
+    // the sums are exact only while no limb carries out of 128 bits: read the largest |term| back and refuse beyond it
+    unsigned long long tm = 0;
+    T3D_CUDA(cudaMemcpyAsync(&tm, w.tmax_all, 8, cudaMemcpyDeviceToHost, st));
+    T3D_CUDA(cudaStreamSynchronize(st));
+    double m;
+    memcpy(&m, &tm, 8);
+    if (!(m < 0x1p62) || (double)F * m >= 0x1p63) {
+        t3d_set_error("t3d_mesh_bodies_stats: a face term of magnitude %g mm^3 over %lld faces: the 128-bit fixed-point sums are "
+                      "exact only for |term| < 2^62 and F * max|term| < 2^63", m, (long long)F);
+        return 2;
+    }
+    return 0;
+}
+
+extern "C" int t3d_mesh_bodies_face_body(const void* faces, int64_t F, int faces_are_i64, const void* vertex_body_i32, void* face_body_i32,
+                                         void* stream)
+{
+    if (F < 0 || F > INT_MAX) {
+        t3d_set_error("t3d_mesh_bodies_face_body: bad face count %lld", (long long)F);
+        return 2;
+    }
+    if (F == 0) return 0;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (faces_are_i64)
+        k_mb_face_body<long long><<<cc_blocks(F), CC_THREADS, 0, st>>>((const long long*)faces, F, (const int32_t*)vertex_body_i32, (int32_t*)face_body_i32);
+    else
+        k_mb_face_body<int32_t><<<cc_blocks(F), CC_THREADS, 0, st>>>((const int32_t*)faces, F, (const int32_t*)vertex_body_i32, (int32_t*)face_body_i32);
+    T3D_CHECK_LAUNCH("t3d_mesh_bodies_face_body");
+    t3d_count_launches(1);
+    return 0;
+}
+
+extern "C" int t3d_mesh_bodies_select(const void* verts_f32, const void* normals_f32, const void* faces, int64_t F, int faces_are_i64,
+                                      int64_t V, const void* vertex_body_i32, int64_t B, const void* keep_u8, void* verts_out_f32,
+                                      void* normals_out_f32, void* faces_out, void* workspace, void* stream)
+{
+    if (int rc = mb_sizes_ok("t3d_mesh_bodies_select", F, V, B)) return rc;
+    if (V == 0) return 0;
+    cudaStream_t st = (cudaStream_t)stream;
+    MbSelectWs w;
+    mb_select_ws(V, F, (char*)workspace, &w);
+    const int64_t nwv = (V + 31) / 32, nwf = (F + 31) / 32;
+    const int32_t* vb = (const int32_t*)vertex_body_i32;
+    const uint8_t* keep = (const uint8_t*)keep_u8;
+    if (faces_are_i64)
+        k_mb_keep<long long><<<cc_blocks(32 * (nwv + nwf)), CC_THREADS, 0, st>>>((const long long*)faces, F, V, vb, keep, nwv, nwf, w.vmask, w.fmask);
+    else
+        k_mb_keep<int32_t><<<cc_blocks(32 * (nwv + nwf)), CC_THREADS, 0, st>>>((const int32_t*)faces, F, V, vb, keep, nwv, nwf, w.vmask, w.fmask);
+    T3D_CHECK_LAUNCH("t3d_mesh_bodies_select keep");
+    t3d_count_launches(1);
+    if (int rc = t3d_exclusive_scan_u32_dev(w.vmask, w.vbase, nwv, nwv, 1, 0, 1, nullptr, w.totals, w.scan, stream)) return rc;
+    k_mb_compact_verts<<<cc_blocks(V), CC_THREADS, 0, st>>>((const float*)verts_f32, (const float*)normals_f32, V, w.vmask, w.vbase,
+                                                            (float*)verts_out_f32, (float*)normals_out_f32);
+    T3D_CHECK_LAUNCH("t3d_mesh_bodies_select vertices");
+    t3d_count_launches(1);
+    if (F == 0) return 0;
+    if (int rc = t3d_exclusive_scan_u32_dev(w.fmask, w.fbase, nwf, nwf, 1, 0, 1, nullptr, w.totals + 1, w.scan, stream)) return rc;
+    if (faces_are_i64)
+        k_mb_compact_faces<long long><<<cc_blocks(F), CC_THREADS, 0, st>>>((const long long*)faces, F, w.vmask, w.vbase, w.fmask, w.fbase,
+                                                                          (long long*)faces_out);
+    else
+        k_mb_compact_faces<int32_t><<<cc_blocks(F), CC_THREADS, 0, st>>>((const int32_t*)faces, F, w.vmask, w.vbase, w.fmask, w.fbase,
+                                                                        (int32_t*)faces_out);
+    T3D_CHECK_LAUNCH("t3d_mesh_bodies_select faces");
     t3d_count_launches(1);
     return 0;
 }

@@ -154,7 +154,7 @@ class DeviceMesh:
     live in `counts_dev` until resolve() (one D2H copy) or set_sizes() trims them."""
 
     __slots__ = ("_verts", "_faces", "counts_dev", "n_ambiguous", "n_exact", "_measures", "raw", "n_active", "n_raw", "n_z",
-                 "normal_src", "canon_map", "_normals", "__weakref__")
+                 "normal_src", "canon_map", "_normals", "_bodies", "__weakref__")
 
     def __init__(self, verts: torch.Tensor, faces: torch.Tensor, n_ambiguous: int = 0, n_exact: int = 0,
                  counts_dev: Optional[torch.Tensor] = None):
@@ -170,6 +170,7 @@ class DeviceMesh:
         self.normal_src = None
         self.canon_map = None
         self._normals = None
+        self._bodies = None      # mesh_bodies(self), once computed
 
     def set_sizes(self, n_verts: int, n_faces: int, unverified: int = 0) -> None:
         """Trim the capacity-sized arrays.  unverified != 0: the fast ordering failed its device-side check, redo the
@@ -1139,3 +1140,140 @@ def component_keep(counts: np.ndarray, min_voxels: int = 1, max_components: Opti
         order = np.lexsort((cand, -counts[cand]))      # size descending, then label ascending
         cand = np.sort(cand[order[:max_components]])
     return cand + 1
+
+
+# ----------------------------------------------------------------------------------------------------------
+# mesh bodies (additive; oracle scipy.sparse.csgraph.connected_components of the mesh's vertex graph)
+# ----------------------------------------------------------------------------------------------------------
+class Bodies:
+    """Connected bodies of a DeviceMesh (mesh_bodies): a body is a connected component of the graph with the edges f0-f1 and
+    f0-f2 of every face; bodies are numbered 0..n-1 by their smallest vertex, as scipy.sparse.csgraph numbers them.  The
+    per-body arrays are computed once, with the labelling, and downloaded on first access."""
+
+    __slots__ = ("mesh", "n", "_vertex_body", "_face_body", "_stats")
+
+    _NAMES = ("vertex_counts", "face_counts", "first_vertex", "bbox_mm", "signed_volumes", "areas")
+
+    def __init__(self, mesh: DeviceMesh, n: int, vertex_body: torch.Tensor, stats: dict):
+        self.mesh, self.n, self._vertex_body, self._stats = mesh, n, vertex_body, stats
+        self._face_body = None
+
+    def vertex_body(self) -> torch.Tensor:
+        """Device int32 (V,): the body of each vertex."""
+        return self._vertex_body
+
+    def face_body(self) -> torch.Tensor:
+        """Device int32 (F,): the body of each face (that of its first vertex)."""
+        if self._face_body is None:
+            faces = self.mesh.faces.contiguous()
+            F = int(faces.shape[0])
+            out = torch.empty(F, dtype=torch.int32, device=faces.device)
+            check(_L().t3d_mesh_bodies_face_body(_p(faces), F, 1 if faces.dtype == torch.int64 else 0, _p(self._vertex_body), _p(out),
+                                                 _stream()), "t3d_mesh_bodies_face_body")
+            self._face_body = out
+        return self._face_body
+
+    def _host(self, name: str) -> np.ndarray:
+        a = self._stats[name]
+        if isinstance(a, torch.Tensor):
+            a = self._stats[name] = download(a)
+        return a
+
+    def vertex_counts(self) -> np.ndarray:
+        """int64 (n,): vertices per body."""
+        return self._host("vertex_counts")
+
+    def face_counts(self) -> np.ndarray:
+        """int64 (n,): faces per body (0 for a vertex no face uses)."""
+        return self._host("face_counts")
+
+    def first_vertex(self) -> np.ndarray:
+        """int64 (n,): the smallest vertex index of each body (ascending)."""
+        return self._host("first_vertex")
+
+    def bbox_mm(self) -> np.ndarray:
+        """float32 (n, 6) [zmin, zmax, ymin, ymax, xmin, xmax]: min / max of the body's vertex columns (a zero bound is +0.0)."""
+        return self._host("bbox_mm")
+
+    def signed_volumes(self) -> np.ndarray:
+        """float64 (n,): the divergence-theorem volume of each body, with the sign the whole-mesh measure gives (a cavity's
+        shell has the opposite sign of the outer one).  The float64 terms of DeviceMesh.measures() are rounded to multiples of
+        2^-64 and added exactly, then the sum is rounded once: bit-identical on every run, but the bodies' volumes need not
+        add up bit for bit to the whole mesh's, whose float64 sum rounds as it goes (DESIGN.md §2)."""
+        return self._host("signed_volumes")
+
+    def areas(self) -> np.ndarray:
+        """float64 (n,): surface area of each body, summed like signed_volumes()."""
+        return self._host("areas")
+
+    def select(self, keep, normals: Optional[torch.Tensor] = None) -> DeviceMesh:
+        """The mesh of the bodies in `keep` (body ids 0..n-1): their vertices and faces in the original order, faces (same
+        dtype) renumbered to the kept vertices.  Normal rows go along: `normals` (device float32 (V, 3)) if given, else the
+        mesh's own field-gradient normals if it has them."""
+        mesh = self.mesh
+        verts, faces = mesh.verts.contiguous(), mesh.faces.contiguous()
+        if normals is None and (mesh._normals is not None or mesh.normal_src is not None):
+            normals = mesh.normals
+        V, F, B = int(verts.shape[0]), int(faces.shape[0]), self.n
+        dev = verts.device
+        mask = np.zeros(max(B, 1), dtype=np.uint8)
+        kept = np.asarray(keep, dtype=np.int64).reshape(-1)
+        if len(kept) and (kept.min() < 0 or kept.max() >= B):
+            raise ValueError("body ids must lie in [0, %d)" % B)
+        mask[kept] = 1
+        V2 = int(self.vertex_counts()[mask[:B] != 0].sum())
+        F2 = int(self.face_counts()[mask[:B] != 0].sum())
+        v_out = torch.empty((V2, 3), dtype=torch.float32, device=dev)
+        f_out = torch.empty((F2, 3), dtype=faces.dtype, device=dev)
+        n_out = None
+        if normals is not None:
+            normals = normals.to(device=dev, dtype=torch.float32).contiguous()
+            if tuple(normals.shape) != (V, 3):
+                raise ValueError("normals must be (V, 3)")
+            n_out = torch.empty((V2, 3), dtype=torch.float32, device=dev)
+        if V2:
+            L = _L()
+            ws = torch.empty(int(L.t3d_mesh_bodies_workspace_bytes(V, F, 0)) // 8 + 1, dtype=torch.int64, device=dev)
+            check(L.t3d_mesh_bodies_select(_p(verts), _p(normals), _p(faces), F, 1 if faces.dtype == torch.int64 else 0, V,
+                                           _p(self._vertex_body), B, _p(torch.from_numpy(mask).to(dev)), _p(v_out), _p(n_out), _p(f_out),
+                                           _p(ws), _stream()), "t3d_mesh_bodies_select")
+        out = DeviceMesh(v_out, f_out)
+        out._normals = n_out
+        return out
+
+
+def mesh_bodies(mesh: DeviceMesh) -> Bodies:
+    """Split a mesh into its connected bodies on the device: labels equal to scipy.sparse.csgraph.connected_components of the
+    edges f0-f1 and f0-f2 of every face, per-body counts, first vertex, box, signed volume and area.  Memoised on the mesh.
+    Raises ValueError for a face index outside [0, V), T3DError (status 2) where an int32 label or the exact 128-bit sums
+    would not hold."""
+    if mesh._bodies is not None:
+        return mesh._bodies
+    L = _L()
+    verts, faces = mesh.verts.contiguous(), mesh.faces.contiguous()
+    if faces.dtype not in (torch.int32, torch.int64) or faces.dim() != 2 or faces.shape[1] != 3:
+        raise ValueError("faces must be (F, 3) int32 or int64")
+    V, F = int(verts.shape[0]), int(faces.shape[0])
+    dev = verts.device
+    i64 = 1 if faces.dtype == torch.int64 else 0
+    V_alloc = V if V < 2 ** 31 else 0              # beyond int32 the label call refuses (status 2) before touching memory
+    vertex_body = torch.empty(V_alloc, dtype=torch.int32, device=dev)
+    nb = torch.empty(2, dtype=torch.int64, device=dev)
+    ws = torch.empty(int(L.t3d_mesh_bodies_workspace_bytes(V_alloc, F, 0)) // 8 + 1, dtype=torch.int64, device=dev)
+    check(L.t3d_mesh_bodies_label(_p(faces), F, i64, V, _p(vertex_body), _p(nb), _p(ws), _stream()), "t3d_mesh_bodies_label")
+    B, n_bad = (int(v) for v in nb.cpu().tolist())
+    if n_bad:
+        raise ValueError("%d faces index a vertex outside [0, %d)" % (n_bad, V))
+    st = {"vertex_counts": torch.empty(B, dtype=torch.int64, device=dev),
+          "face_counts": torch.empty(B, dtype=torch.int64, device=dev),
+          "first_vertex": torch.empty(B, dtype=torch.int64, device=dev),
+          "bbox_mm": torch.empty((B, 6), dtype=torch.float32, device=dev),
+          "signed_volumes": torch.empty(B, dtype=torch.float64, device=dev),
+          "areas": torch.empty(B, dtype=torch.float64, device=dev)}
+    need = int(L.t3d_mesh_bodies_workspace_bytes(V, F, B)) // 8 + 1
+    if need > ws.numel():
+        ws = torch.empty(need, dtype=torch.int64, device=dev)
+    check(L.t3d_mesh_bodies_stats(_p(verts), _p(faces), F, i64, V, _p(vertex_body), B, *(_p(st[k]) for k in Bodies._NAMES), _p(ws),
+                                  _stream()), "t3d_mesh_bodies_stats")
+    mesh._bodies = Bodies(mesh, B, vertex_body, st)
+    return mesh._bodies

@@ -133,6 +133,47 @@ class SurfaceExtractor:
                 raise
             return None
 
+    def split_surface(self, vertices: np.ndarray, faces: np.ndarray) -> Tuple[np.ndarray, int]:
+        """The connected bodies of a mesh, as scipy.sparse.csgraph.connected_components returns them for the graph with the
+        edges f0-f1 and f0-f2 of every face: (int32 (V,) body of each vertex, number of bodies).  Bodies are numbered by their
+        smallest vertex; a vertex no face uses is a body of its own."""
+        bodies = engine.mesh_bodies(engine.mesh_from_host(vertices, faces))
+        return engine.download(bodies.vertex_body()), bodies.n
+
+    def analyze_surface_bodies(self, vertices: np.ndarray, faces: np.ndarray) -> dict:
+        """Per-body arrays of a mesh (bodies as split_surface numbers them): n_bodies, vertex_counts, face_counts, first_vertex
+        (int64), signed_volume_mm3, volume_mm3 (its absolute value) and surface_area_mm2 (float64, each an exactly summed
+        divergence-theorem / area sum rounded once, DESIGN.md §2), bbox_mm (float32 (n, 6) [zmin, zmax, ymin, ymax, xmin,
+        xmax]).  A hollow object gives two bodies whose signed volumes have opposite signs."""
+        b = engine.mesh_bodies(engine.mesh_from_host(vertices, faces))
+        sv = b.signed_volumes()
+        return {"n_bodies": b.n, "vertex_counts": b.vertex_counts(), "face_counts": b.face_counts(), "first_vertex": b.first_vertex(),
+                "signed_volume_mm3": sv, "volume_mm3": np.abs(sv), "surface_area_mm2": b.areas(), "bbox_mm": b.bbox_mm()}
+
+    def filter_surface_bodies(self, vertices: np.ndarray, faces: np.ndarray, min_faces: int = 1, max_bodies=None,
+                              vertex_normals: Optional[np.ndarray] = None):
+        """The mesh of the bodies with at least min_faces faces; with max_bodies, only that many of the largest by face count
+        (ties: the body with the smaller first vertex).  Vertices and faces keep their order and the faces their dtype, renumbered
+        to the kept vertices.  Returns (vertices, faces), or (vertices, faces, normals) with the rows of vertex_normals that go
+        with the kept vertices.  The arrays are read-only and, like extract_manifold_surface's, recognised by volume, area and
+        the exporters without another upload."""
+        mesh = engine.mesh_from_host(vertices, faces)
+        bodies = engine.mesh_bodies(mesh)
+        keep = engine.component_keep(bodies.face_counts(), min_faces, max_bodies) - 1
+        normals = None
+        if vertex_normals is not None:
+            if engine.meshes.lookup(vertex_normals) is mesh and mesh.normals is not None:
+                normals = mesh.normals
+            else:
+                import torch
+                normals = torch.from_numpy(np.ascontiguousarray(vertex_normals, dtype=np.float32)).to(mesh.verts.device)
+        out = bodies.select(keep, normals)
+        v = engine.publish(engine.meshes, engine.download(out.verts), out)
+        f = engine.publish(engine.meshes, engine.download(out.faces), out)
+        if normals is None:
+            return v, f
+        return v, f, engine.publish(engine.meshes, engine.download(out.normals), out)
+
     def vertex_normals(self, vertices: np.ndarray, faces: np.ndarray) -> np.ndarray:
         """Area-weighted unit vertex normals, float32 (V,3) [z,y,x]."""
         from . import normals
