@@ -406,6 +406,33 @@ int t3d_mesh_bodies_select(const void* verts_f32, const void* normals_f32, const
                            const void* vertex_body_i32, int64_t B, const void* keep_u8, void* verts_out_f32, void* normals_out_f32,
                            void* faces_out, void* workspace, void* stream);
 
+/* ---- mesh smoothing (additive) --------------------------------------------------------------------------- */
+
+/* Vertex adjacency and Taubin smoothing of a triangle mesh: verts_f32 (V, 3), faces (F, 3) int32 or int64 (faces_are_i64)
+ * (csrc/t3d_smooth.cu).  V must fit int32 (the neighbour ids) and F must be at most (2^32 - 1) / 6 = 715 827 882 (the raw
+ * entries, up to 6 per face, are counted in 32 bits); otherwise status 2 naming the size, before any memory is touched.
+ *   t3d_mesh_adjacency_workspace_bytes(V, F): the workspace of both adjacency calls; emit reads what count left in it.
+ *   t3d_mesh_adjacency_count -> offsets_i64[V + 1]: CSR row offsets of the neighbours, [V] = N; n_u64: two device uint64,
+ *                               [0] = N, [1] = faces with an index outside [0, V) (skipped; the result needs it to be 0).
+ *                               The neighbours of i are the distinct j != i that share a face edge with i (each face
+ *                               (a, b, c) gives the edges {a,b}, {b,c}, {c,a}), in ascending order.
+ *   (caller reads N and allocates)
+ *   t3d_mesh_adjacency_emit  -> neighbours_i32[N].
+ *   t3d_mesh_taubin          -> verts_out_f32 (V, 3): `iterations` steps of trimesh.smoothing.filter_taubin with equal
+ *                               weights, from the float32 input in float64: s = +0.0, s = s + w * x[j] over the neighbours
+ *                               in ascending order (w = 1.0 / degree), dd = s - x[i], x[i] + lamb * dd on even steps and
+ *                               x[i] - nu * dd on odd ones, every vertex from the previous iterate, no FMA contraction; a
+ *                               vertex without neighbours keeps its position; rounded once to float32 at the end.
+ *                               iterations >= 0 and finite lamb / nu (status 2 otherwise).  verts_out must not overlap verts.
+ *                               Workspace: t3d_mesh_taubin_workspace_bytes(V). */
+int64_t t3d_mesh_adjacency_workspace_bytes(int64_t V, int64_t F);
+int t3d_mesh_adjacency_count(const void* faces, int64_t F, int faces_are_i64, int64_t V, void* offsets_i64, void* n_u64,
+                             void* workspace, void* stream);
+int t3d_mesh_adjacency_emit(int64_t V, int64_t F, const void* offsets_i64, void* neighbours_i32, void* workspace, void* stream);
+int64_t t3d_mesh_taubin_workspace_bytes(int64_t V);
+int t3d_mesh_taubin(const void* verts_f32, int64_t V, const void* offsets_i64, const void* neighbours_i32, int iterations, double lamb,
+                    double nu, void* verts_out_f32, void* workspace, void* stream);
+
 /* ---- device-side mesh consumers: the step right after the path (SURVEY.md 8f-3) ----------------------------- */
 
 /* glb_exporter.py:52-91 create_layer_colors: rgba_u8 (V,4) = grey (200,200,200,255); red where first_start <= z <=

@@ -109,6 +109,11 @@ SIGNATURES = {
     "t3d_mesh_bodies_stats": (_i, [_vp, _vp, _i64, _i, _i64, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "t3d_mesh_bodies_face_body": (_i, [_vp, _i64, _i, _vp, _vp, _vp]),
     "t3d_mesh_bodies_select": (_i, [_vp, _vp, _vp, _i64, _i, _i64, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "t3d_mesh_adjacency_workspace_bytes": (_i64, [_i64, _i64]),
+    "t3d_mesh_adjacency_count": (_i, [_vp, _i64, _i, _i64, _vp, _vp, _vp, _vp]),
+    "t3d_mesh_adjacency_emit": (_i, [_i64, _i64, _vp, _vp, _vp, _vp]),
+    "t3d_mesh_taubin_workspace_bytes": (_i64, [_i64]),
+    "t3d_mesh_taubin": (_i, [_vp, _i64, _vp, _vp, _i, _dbl, _dbl, _vp, _vp, _vp]),
 }
 
 

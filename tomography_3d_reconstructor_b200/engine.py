@@ -154,7 +154,7 @@ class DeviceMesh:
     live in `counts_dev` until resolve() (one D2H copy) or set_sizes() trims them."""
 
     __slots__ = ("_verts", "_faces", "counts_dev", "n_ambiguous", "n_exact", "_measures", "raw", "n_active", "n_raw", "n_z",
-                 "normal_src", "canon_map", "_normals", "_bodies", "__weakref__")
+                 "normal_src", "canon_map", "_normals", "_bodies", "_adjacency", "__weakref__")
 
     def __init__(self, verts: torch.Tensor, faces: torch.Tensor, n_ambiguous: int = 0, n_exact: int = 0,
                  counts_dev: Optional[torch.Tensor] = None):
@@ -171,6 +171,7 @@ class DeviceMesh:
         self.canon_map = None
         self._normals = None
         self._bodies = None      # mesh_bodies(self), once computed
+        self._adjacency = None   # vertex_neighbors(self), once computed
 
     def set_sizes(self, n_verts: int, n_faces: int, unverified: int = 0) -> None:
         """Trim the capacity-sized arrays.  unverified != 0: the fast ordering failed its device-side check, redo the
@@ -1277,3 +1278,60 @@ def mesh_bodies(mesh: DeviceMesh) -> Bodies:
                                   _stream()), "t3d_mesh_bodies_stats")
     mesh._bodies = Bodies(mesh, B, vertex_body, st)
     return mesh._bodies
+
+
+# ----------------------------------------------------------------------------------------------------------
+# mesh smoothing (additive; oracle trimesh.smoothing.filter_taubin with equal weights, written out in numpy)
+# ----------------------------------------------------------------------------------------------------------
+def vertex_neighbors(mesh: DeviceMesh) -> Tuple[torch.Tensor, torch.Tensor]:
+    """The vertex adjacency of a mesh as device CSR arrays (offsets int64 (V + 1,), neighbours int32 (N,)): the neighbours of
+    vertex i are the distinct j != i that share a face edge with it, in ascending order (trimesh's vertex_neighbors, sorted).
+    Memoised on the mesh.  Raises ValueError for a face index outside [0, V), T3DError (status 2) beyond the int32 ids."""
+    if mesh._adjacency is not None:
+        return mesh._adjacency
+    L = _L()
+    faces = mesh.faces.contiguous()
+    if faces.dtype not in (torch.int32, torch.int64) or faces.dim() != 2 or faces.shape[1] != 3:
+        raise ValueError("faces must be (F, 3) int32 or int64")
+    V, F = int(mesh.verts.shape[0]), int(faces.shape[0])
+    dev = faces.device
+    V_alloc = V if V < 2 ** 31 else 0              # beyond int32 the count call refuses (status 2) before touching memory
+    offsets = torch.empty(V_alloc + 1, dtype=torch.int64, device=dev)
+    n = torch.empty(2, dtype=torch.int64, device=dev)
+    ws = torch.empty(int(L.t3d_mesh_adjacency_workspace_bytes(V_alloc, F)) // 8 + 1, dtype=torch.int64, device=dev)
+    i64 = 1 if faces.dtype == torch.int64 else 0
+    check(L.t3d_mesh_adjacency_count(_p(faces), F, i64, V, _p(offsets), _p(n), _p(ws), _stream()), "t3d_mesh_adjacency_count")
+    N, n_bad = (int(v) for v in n.cpu().tolist())
+    if n_bad:
+        raise ValueError("%d faces index a vertex outside [0, %d)" % (n_bad, V))
+    neighbours = torch.empty(N, dtype=torch.int32, device=dev)
+    check(L.t3d_mesh_adjacency_emit(V, F, _p(offsets), _p(neighbours), _p(ws), _stream()), "t3d_mesh_adjacency_emit")
+    mesh._adjacency = (offsets, neighbours)
+    return mesh._adjacency
+
+
+def smooth_mesh(mesh: DeviceMesh, iterations: int = 10, lamb: float = 0.5, nu: float = 0.5) -> DeviceMesh:
+    """Taubin smoothing (trimesh.smoothing.filter_taubin with the equal-weight Laplacian and its defaults), bit for bit against
+    the numpy definition of DESIGN.md §2: a new DeviceMesh with new float32 vertices and the same faces tensor.  It shares the
+    adjacency of `mesh` (so smoothing it again does not rebuild it) and has no field-gradient normals, which describe the
+    unsmoothed field.  A vertex no face edge reaches keeps its position.  Raises ValueError for iterations < 0 or a
+    non-finite lamb or nu."""
+    import math
+    import operator
+    iterations = operator.index(iterations)
+    lamb, nu = float(lamb), float(nu)
+    if not 0 <= iterations < 2 ** 31:
+        raise ValueError("iterations must be in [0, 2^31), got %d" % iterations)
+    if not (math.isfinite(lamb) and math.isfinite(nu)):
+        raise ValueError("lamb and nu must be finite, got %r and %r" % (lamb, nu))
+    L = _L()
+    offsets, neighbours = vertex_neighbors(mesh)
+    verts = mesh.verts.contiguous()
+    V = int(verts.shape[0])
+    out = torch.empty_like(verts)
+    ws = torch.empty(int(L.t3d_mesh_taubin_workspace_bytes(V)) // 8 + 1, dtype=torch.int64, device=verts.device)
+    check(L.t3d_mesh_taubin(_p(verts), V, _p(offsets), _p(neighbours), iterations, lamb, nu, _p(out), _p(ws), _stream()),
+          "t3d_mesh_taubin")
+    smoothed = DeviceMesh(out, mesh.faces)
+    smoothed._adjacency = mesh._adjacency
+    return smoothed
